@@ -71,7 +71,26 @@ def parse():
     ap.add_argument("--profile-step", default="", choices=["", "dense", "compact"],
                     help="run only warmup + steps of the device-resident step in that input form and exit without a JSON "
                          "line (the command profiles/ launch lists are taken with under ncu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps of `value`, write what the last of them computed -- the loss it returned, "
+                         "every parameter's gradient and every parameter after the optimiser step -- as float32 "
+                         "DIR/<name>.npy (inputs and initial parameters are seeded: equal arguments give equal inputs; "
+                         "git ignores bench_outputs/)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+def dump_outputs(out_dir, loss, model):
+    """DIR/loss.npy, DIR/grad.<parameter>.npy, DIR/param.<parameter>.npy (float32, ~70 KB at the default widths)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss}
+    for k, p in model.named_parameters():
+        arrays[f"grad.{k}"] = p.grad
+        arrays[f"param.{k}"] = p
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def workload_name(a):
@@ -836,7 +855,7 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
-    rate = lambda ms, steps=a.steps: world * graphs_per_step * steps / (ms / 1000.0)
+    rate = lambda ms: world * graphs_per_step * a.steps / (ms / 1000.0)
     t = lambda v: (torch.from_numpy(v) if isinstance(v, np.ndarray) else v).to(dev)
     dev_compact = [(ops.CompactBatch(t(c["label"]), t(c["row"]), t(c["col"]), t(c["node_ptr"]), t(c["edge_ptr"]),
                                      corpus.num_node_labels, int(np.diff(c["edge_ptr"]).max()), c["coalesced"]),
@@ -846,9 +865,11 @@ def main():
         b = dev_batches[i % len(dev_batches)]
         trainer.step(b["x"], b["edge_index"], b["node_ptr"], b["triplets"])
 
+    last_loss = [None]
+
     def step_resident(i):
         cb, nptr, trip = dev_compact[i % len(dev_compact)]
-        trainer.step(cb, None, nptr, trip)
+        last_loss[0] = trainer.step(cb, None, nptr, trip)
 
     if a.profile_step:
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
@@ -875,6 +896,9 @@ def main():
     launches = _lib.kernel_launches - k0
     clocks = sampler.finish()
     value = rate(ms)
+    if a.dump_outputs and rank == 0:
+        # before anything else runs the model: gradients and parameters are those of the last timed step
+        dump_outputs(a.dump_outputs, last_loss[0], model)
 
     # ---- the same step on the PyG wire format resident in HBM (fp32 one-hot x, int64 edge_index)
     for i in range(3):
@@ -906,9 +930,8 @@ def main():
     def run_wire(steps):
         return trainer.run_from_host((batches[i % len(batches)] for i in range(steps)), dev)
 
-    wire_steps = max(2, min(a.steps, 6))
     run_wire(2)
-    ms_e2e_wire = timed(lambda i: run_wire(wire_steps) if i == 0 else None, 1)
+    ms_e2e_wire = timed(lambda i: run_wire(a.steps) if i == 0 else None, 1)
     b0 = batches[0]
     h2d_wire = b0["x"].numel() * 4 + b0["edge_index"].numel() * 8 + b0["triplets"].numel() * 8 + 4 * 8 * (graphs_per_step + 1)
 
@@ -1049,7 +1072,7 @@ def main():
                                      "api": "TripletTrainer.run_from_host_compact: PRE-PACKED pinned host batches (labels i32, local "
                                             "edge lists i32, offsets, triplets), copy-stream double buffering; host-side batch assembly "
                                             "is outside the timed region"},
-                "e2e_fp32_wire": {"value": rate(ms_e2e_wire, wire_steps), "unit": UNIT, "ms_per_step": ms_e2e_wire / wire_steps,
+                "e2e_fp32_wire": {"value": rate(ms_e2e_wire), "unit": UNIT, "ms_per_step": ms_e2e_wire / a.steps,
                                   "h2d_bytes_per_step": int(h2d_wire), "d2h_bytes_per_step": 4,
                                   "api": "TripletTrainer.run_from_host: pre-packed pinned x[f32 N,89] / edge_index[i64 2,E] / triplets "
                                          "(the tensors PyG's Batch.to(device) moves): PCIe bound"},

@@ -8,7 +8,8 @@ tiny synthetic TU-format dataset (40 PROTEINS-shape graphs written by tsg.tu.wri
    reference's own math (sag over the oracle-backed torch_geometric), including the stage-2 code after training that
    crashes as shipped (evaluate() signature, int into os.environ, int default of a str option, np.matrix into sklearn).
 
-Needs /root/reference (this container); skipped on the GPU box.  One helper process per mode runs all cases concurrently."""
+The script cases need the original project's source tree (launcher_driver.REF) and skip without it.  One helper
+process per mode runs all cases concurrently."""
 import json
 import os
 import subprocess
@@ -17,10 +18,12 @@ import sys
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/Code/sag"), reason="reference checkout not present on this box")
 
 sys.path.insert(0, HERE)
-from launcher_driver import cases  # noqa: E402
+from launcher_driver import REF, cases  # noqa: E402
+
+needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "sag")),
+                                     reason="the original project's source tree is not present")
 
 IDS = [f"{d}-{s}" + (f"-{m}" if m else "") for d, s, m, _ in cases()]
 
@@ -43,6 +46,7 @@ def e2e(tmp_path_factory):
     return _run("e2e", tmp_path_factory.mktemp("e2e"))
 
 
+@needs_reference
 @pytest.mark.parametrize("case", IDS)
 def test_script_reaches_the_tsg_drop_ins(reach, case):
     r = reach[case]
@@ -65,6 +69,7 @@ def test_script_reaches_the_tsg_drop_ins(reach, case):
             assert r["script_classes_patched"].get("encoders.Pool.forward") is True
 
 
+@needs_reference
 @pytest.mark.parametrize("case", IDS)
 def test_compat_layer_carries_the_script_to_its_end(e2e, case):
     r = e2e[case]

@@ -139,24 +139,47 @@ def test_gat_cfg3_matches_reference():
             assert rel_err(r["a"].grad, d[f"grad/{lname}.attention_{h}.a"]) <= 1e-5, (lname, h)
 
 
+# Config 4's assignment tower: its weight gradients are ill-conditioned in fp32.  The fixture (the original project's
+# fp32 result) sits 4.9e-5 to 7.8e-5 from their float64 value, and the fp32 oracle lands up to 1.7e-4 from the fixture
+# depending on the host BLAS's summation order (one thread; 4e-6 where it sums like the machine that made the fixture).
+# Both bounds below are against the fixture: the float64 oracle must reproduce it to within its own fp32 noise (host
+# independent), the fp32 oracle to within that noise plus the host's.
+ASSIGN_TOWER = ("assign_conv_first_modules.0", "assign_conv_block_modules.0.0", "assign_conv_last_modules.0",
+                "assign_pred_modules.0")
+ASSIGN_FP64_VS_FIXTURE = 1e-4
+ASSIGN_FP32_VS_FIXTURE = 3e-4
+
+
 def test_diffpool_cfg4_matches_reference():
-    """Config 4 dims: N = 1000 -> K = 100, D = 96, Linear(164 -> 100), DD-shape graph."""
+    """Config 4 dims: N = 1000 -> K = 100, D = 96, Linear(164 -> 100), DD-shape graph.  Every weight gradient of the
+    fp32 oracle AND of its float64 evaluation against the fixture: 1e-5, the assignment tower at the bounds above."""
     from golden_util import dense_adj, padded
     d = load("dense_diffpool_cfg4.npz")
     N, Fi, H, O, L = [int(v) for v in d["dims"]]
     n = int(d["n"])
+    x, adj = padded(d["x"], N), dense_adj(d["ei"], N)
     p = _diffpool_params(d, req=True)
-    out, aux = D.soft_pool_readout(padded(d["x"], N), dense_adj(d["ei"], N), [n], p)
+    out, aux = D.soft_pool_readout(x, adj, [n], p)
     assert aux["s"].shape[-1] == 100 and out.shape[-1] == 192
     assert rel_err(aux["s"][0, :n], d["assign"]) <= PIN
     assert rel_err(out, d["readout"]) <= PIN
     (out * d["cot"]).sum().backward()
+    d64 = {k: v.double() if torch.is_tensor(v) and v.is_floating_point() else v for k, v in d.items()}
+    p64 = _diffpool_params(d64, req=True)
+    o64, _ = D.soft_pool_readout(x.double(), adj.double(), [n], p64)
+    (o64 * d64["cot"]).sum().backward()
+    grads = {"assign_pred_modules.0": (p["assign_pred.weight"].grad, p64["assign_pred.weight"].grad)}
     for key, (f, b, l) in dict(conv=("conv_first", "conv_block", "conv_last"),
                                assign_conv=("assign_conv_first_modules.0", "assign_conv_block_modules.0", "assign_conv_last_modules.0"),
                                conv_after=("conv_first_after_pool.0", "conv_block_after_pool.0", "conv_last_after_pool.0")).items():
-        for c, nm in zip(p[key], conv_names(f, b, l, L)):
-            assert rel_err(c["weight"].grad, d[f"grad/{nm}.weight"]) <= 1e-5, nm
-    assert rel_err(p["assign_pred.weight"].grad, d["grad/assign_pred_modules.0.weight"]) <= 1e-5
+        for c, c64, nm in zip(p[key], p64[key], conv_names(f, b, l, L)):
+            grads[nm] = (c["weight"].grad, c64["weight"].grad)
+    assert len(grads) == 3 * L + 1 and set(ASSIGN_TOWER) <= set(grads)
+    for nm, (g32, g64) in grads.items():
+        fixture = d[f"grad/{nm}.weight"]
+        tower = nm in ASSIGN_TOWER
+        assert rel_err(g64, fixture) <= (ASSIGN_FP64_VS_FIXTURE if tower else 1e-5), ("float64", nm)
+        assert rel_err(g32, fixture) <= (ASSIGN_FP32_VS_FIXTURE if tower else 1e-5), ("fp32", nm)
 
 
 def test_eigen_cfg5_matches_reference():

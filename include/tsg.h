@@ -568,6 +568,36 @@ int tsg_sag_step_bwd_compact(const tsg_sag_shape* shape, const tsg_sag_head* hea
                              float* const* grads, void* arena, size_t arena_bytes, void* workspace,
                              size_t workspace_bytes, void* stream);
 
+/* The supervised ("original") setting of the same model.  num_triplets / margin / eps of `head` are not used here.
+ * The head backward of K14 takes every even hidden width whose head forward fits shared memory (H = 128 with C <= 64
+ * included): where its per-CTA gradient row does not fit, per-graph deltas go to the workspace and the parameter
+ * gradients come from K3's fixed-order reductions (tsg_linear_bwd_weight / tsg_relu_bwd_colsum).
+ *   tsg_sag_nll_step_compact replaces the body of the loop of Code/sag/train.py:194: out = model(data);
+ *     F.nll_loss(out, data.y) (mean over the G graphs); loss.backward().  y int64 [G] graph labels; loss: device float;
+ *     emb_out optional [G, C] log-probabilities; gradients WRITTEN into the 18 grads as in K14.  The gradients are
+ *     bit-identical to tsg_sag_step_fwd_compact + autograd F.nll_loss + tsg_sag_step_bwd_compact.
+ *   tsg_sag_classify_compact replaces `test()` of Code/sag/train.py:19-29 on a packed batch: model.eval() forward
+ *     (tsg_sag_encoder_embed_compact, then the head with dropout off), pred int64 [G] = out.max(dim=1)[1] (first index
+ *     on ties), optional logp_out [G, C]; with y: *correct (int64) = #(pred == y) and *nll_sum (float) =
+ *     F.nll_loss(out, y, reduction='sum'), both reduced in a fixed order (y NULL: both must be NULL).
+ * A label outside [0, C) is clamped for the read and sets bit TSG_SAG_LABEL_RANGE in shape->status (or, when that is
+ * NULL, in the arena's TSG_SAG_STATUS word).  Workspace queries return 0 exactly when the call cannot run the shape. */
+#define TSG_SAG_LABEL_RANGE 8
+size_t tsg_sag_nll_step_workspace_bytes(const tsg_sag_shape* shape, const tsg_sag_head* head);
+int tsg_sag_nll_step_compact(const tsg_sag_shape* shape, const tsg_sag_head* head, const int32_t* label,
+                             const int32_t* local_row, const int32_t* local_col, const int64_t* edge_ptr,
+                             const int64_t* level_ptr, const float* const* params, const int64_t* y,
+                             const float* dropout_mask /*nullable*/, float* const* grads, float* loss,
+                             float* emb_out /*nullable*/, void* arena, size_t arena_bytes, void* workspace,
+                             size_t workspace_bytes, void* stream);
+size_t tsg_sag_classify_workspace_bytes(const tsg_sag_shape* shape, const tsg_sag_head* head);
+int tsg_sag_classify_compact(const tsg_sag_shape* shape, const tsg_sag_head* head, const int32_t* label,
+                             const int32_t* local_row, const int32_t* local_col, const int64_t* edge_ptr,
+                             const int64_t* level_ptr, const float* const* params, const int64_t* y /*nullable*/,
+                             int64_t* pred, float* logp_out /*nullable*/, int64_t* correct /*nullable*/,
+                             float* nll_sum /*nullable*/, void* arena, size_t arena_bytes, void* workspace,
+                             size_t workspace_bytes, void* stream);
+
 /* Row-softmax backward from the saved output of tsg_linear_fwd(..., TSG_LIN_SOFTMAX): dL = S * (dS - rowsum(S * dS))
  * (SoftPoolingGcnEncoder's assignment, encoders.py:369; SURVEY A.4 K7). */
 int tsg_softmax_bwd(const float* S, const float* dS, float* dL, int64_t num_rows, int64_t num_cols, void* stream);

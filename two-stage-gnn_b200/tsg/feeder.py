@@ -53,12 +53,17 @@ class DeviceCorpus:
             self.label, self.x, self.feat = t(corpus.node_label, np.int32), None, corpus.num_node_labels
         else:
             self.label, self.x, self.feat = None, t(dense_x, np.float32), int(dense_x.shape[1])
+        self.y_host = np.ascontiguousarray(corpus.y, dtype=np.int64)      # graph labels (the supervised setting)
+        self.y = torch.from_numpy(self.y_host).to(device)
+        self.labels_checked = None
 
     @classmethod
     def from_device(cls, label: torch.Tensor, row: torch.Tensor, col: torch.Tensor, node_ptr_host: np.ndarray,
-                    edge_ptr_host: np.ndarray, num_labels: int, coalesced: bool) -> "DeviceCorpus":
+                    edge_ptr_host: np.ndarray, num_labels: int, coalesced: bool,
+                    y: torch.Tensor | None = None) -> "DeviceCorpus":
         """A corpus whose arrays already live in HBM (e.g. a shard assembled on the GPU from a smaller base corpus:
-        bench.py's 1 M-graph config-5 corpus); only the two offset arrays come from the host."""
+        bench.py's 1 M-graph config-5 corpus); only the two offset arrays come from the host.  `y`: optional int64
+        [num_graphs] graph labels on the device."""
         self = cls.__new__(cls)
         self.device = label.device
         self.n = np.diff(node_ptr_host).astype(np.int64); self.e = np.diff(edge_ptr_host).astype(np.int64)
@@ -67,7 +72,25 @@ class DeviceCorpus:
         self.edge_ptr = torch.from_numpy(np.ascontiguousarray(edge_ptr_host, dtype=np.int64)).to(self.device)
         self.row, self.col, self.label, self.x, self.feat = row, col, label, None, int(num_labels)
         self.coalesced = bool(coalesced)
+        if y is not None and tuple(y.shape) != (self.num_graphs,):
+            raise ValueError(f"tsg: y has shape {tuple(y.shape)}, the corpus has {self.num_graphs} graphs")
+        self.y = None if y is None else y.to(device=self.device, dtype=torch.int64).contiguous()
+        self.y_host, self.labels_checked = None, None
         return self
+
+    def check_labels(self, num_classes: int) -> None:
+        """Raise ValueError unless every graph label lies in [0, num_classes): once per corpus and class count, on the
+        host (a device-resident `y` is read back for it once).  An out-of-range label would otherwise reach ATen's
+        nll_loss on the autograd path, which stops the process with a device assert."""
+        if self.labels_checked == num_classes:
+            return
+        if self.y is None:
+            raise ValueError("tsg: the corpus carries no graph labels (y)")
+        y = self.y_host if self.y_host is not None else self.y.cpu().numpy()
+        if y.size and (int(y.min()) < 0 or int(y.max()) >= num_classes):
+            bad = int(np.flatnonzero((y < 0) | (y >= num_classes))[0])
+            raise ValueError(f"tsg: graph {bad} has label {int(y[bad])}, outside [0, {num_classes})")
+        self.labels_checked = num_classes
 
     def offsets(self, ids_host: np.ndarray):
         """Packed offsets for a list of graph ids (host numpy; int64 [B+1] each)."""

@@ -138,8 +138,12 @@ def sag_arena_view(shape, arena: torch.Tensor, level: int, field: str) -> torch.
     return arena[off.value:off.value + nb.value].view(dt)
 
 
+LABEL_RANGE = 8           # TSG_SAG_LABEL_RANGE (include/tsg.h)
+
+
 def check_fused_status() -> None:
-    """Look at the status word the verifying kernels (K1d, K13) OR-ed their bits into since the last call -- ONE device
+    """Look at the status word the verifying kernels (K1d, K13, and the label checks of the supervised step and the
+    classification forward) OR-ed their bits into since the last call -- ONE device
     read per device, so callers do it where they synchronise anyway (loss read-back, end of a feeder loop, tests).  A non-zero word means a graph's
     edge list was not what those kernels require (endpoints in range, no self loops, sorted by (row, col), symmetric:
     the TUDataset / TU-loader form); its embedding was zeroed.  There is no silent fallback: this raises."""
@@ -150,6 +154,9 @@ def check_fused_status() -> None:
         bits |= int(_STATUS[i].item())
         _STATUS[i].zero_()
     _STATUS_DIRTY.clear()
+    if bits & LABEL_RANGE:
+        raise RuntimeError("tsg: a graph label lies outside [0, num_classes) (status bit 8, set by the supervised step or "
+                           "the classification forward); it was clamped, so the loss and the accuracy are invalid")
     if bits:
         names = [n for b, n in ((1, "edge endpoint out of range / self loop"), (2, "edge list not sorted by (row, col)"),
                                 (4, "edge list not symmetric")) if bits & b]
@@ -377,14 +384,28 @@ class PackedSAGNet(torch.nn.Module):
             self.__dict__["_flat_grad"], self.__dict__["_grad_views"] = fg, views
         return fg, views
 
+    def _head_fits(self) -> bool:
+        """The head's shape is one the native steps run (the workspace query is 0 otherwise): a pure host query, cached."""
+        from . import _lib
+        key = (self.nhid, self.num_classes)
+        hit = self.__dict__.get("_head_fits_cache")
+        if hit is None or hit[0] != key:
+            shape = _lib.SagShape(1, self.num_features, self.nhid, 0)
+            head = _lib.SagHead(self.num_classes, 1, 0.0, 0.0, 0.0, 0)
+            hit = self.__dict__["_head_fits_cache"] = (
+                key, _lib.lib.tsg_sag_triplet_step_workspace_bytes(ctypes.byref(shape), ctypes.byref(head)) != 0)
+        return hit[1]
+
     def native_step_supported(self, cb, node_ptr_host=None) -> bool:
-        """Can K14 take this batch?  (Compact input, even hidden width, label table within the kernels' range, float32
-        CUDA parameters, and -- when the offsets are given -- every graph within the executor's per-graph limits;
+        """Can K14 take this batch?  (Compact input, even hidden width, a head the native steps run, label table within
+        the kernels' range, float32 CUDA parameters, and -- when the offsets are given -- every graph within the executor's per-graph limits;
         otherwise the caller uses the autograd path, which handles anything.)"""
         from . import _lib
         if not (USE_EXECUTOR and USE_NATIVE_STEP and isinstance(cb, ops.CompactBatch)) or self.nhid % 2:
             return False
         if cb.num_labels != self.num_features or _lib.lib.tsg_embed_bwd_weight_workspace_bytes(cb.num_labels, self.nhid) == 0:
+            return False
+        if not self._head_fits():
             return False
         if node_ptr_host is not None:
             plan, _ = self._level_plan(node_ptr_host, cb.label.device)
@@ -392,7 +413,10 @@ class PackedSAGNet(torch.nn.Module):
                 return False
         return all(p.is_cuda and p.dtype == torch.float32 and p.is_contiguous() for p in self._step_params())
 
-    def _native_setup(self, cb, node_ptr_host, num_triplets, margin, eps, dropout_mask):
+    _WS_QUERY = {"triplet": "tsg_sag_triplet_step_workspace_bytes", "nll": "tsg_sag_nll_step_workspace_bytes",
+                 "classify": "tsg_sag_classify_workspace_bytes"}
+
+    def _native_setup(self, cb, node_ptr_host, num_triplets, margin, eps, dropout_mask, entry="triplet"):
         from . import _lib
         dev = cb.label.device
         plan, ptrs = self._level_plan(node_ptr_host, dev)
@@ -402,14 +426,17 @@ class PackedSAGNet(torch.nn.Module):
         shape.max_graph_edges = int(cb.max_graph_edges)
         shape.pooling_ratio = float(self.pooling_ratio)
         shape.flags = 1 if cb.coalesced else 0
-        if cb.coalesced:
+        if cb.coalesced or entry != "triplet":      # the label checks report through the persistent word as well
             shape.status = _status_word(dev).data_ptr()
-        count = self.__dict__["_native_steps"] = self.__dict__.get("_native_steps", 0) + 1
-        p_drop = float(self.dropout_ratio) if (self.training and dropout_mask is None) else 0.0
+        if entry == "classify":                     # evaluation: dropout off, and no draw from the step counter
+            count, p_drop = 0, 0.0
+        else:
+            count = self.__dict__["_native_steps"] = self.__dict__.get("_native_steps", 0) + 1
+            p_drop = float(self.dropout_ratio) if (self.training and dropout_mask is None) else 0.0
         head = _lib.SagHead(self.num_classes, max(int(num_triplets), 1), float(margin), float(eps), p_drop,
                             (torch.initial_seed() * 0x9E3779B1 + count) & 0xFFFFFFFFFFFFFFFF)
         arena_bytes = _lib.lib.tsg_sag_arena_bytes(ctypes.byref(shape))
-        ws_bytes = _lib.lib.tsg_sag_triplet_step_workspace_bytes(ctypes.byref(shape), ctypes.byref(head))
+        ws_bytes = getattr(_lib.lib, self._WS_QUERY[entry])(ctypes.byref(shape), ctypes.byref(head))
         if arena_bytes == 0 or ws_bytes == 0:
             raise RuntimeError("tsg: bad shape for the native training step")
         arena = torch.empty(arena_bytes, dtype=torch.uint8, device=dev)
@@ -440,6 +467,58 @@ class PackedSAGNet(torch.nn.Module):
             global LAST_ARENA
             LAST_ARENA = (shape, arena)
         return (loss.view(()), emb) if return_emb else loss.view(())
+
+    def native_nll_step(self, cb, node_ptr_host, y: torch.Tensor, dropout_mask: Optional[torch.Tensor] = None,
+                        return_emb: bool = False):
+        """The supervised step of Code/sag/train.py:194 -- forward, F.nll_loss(out, y) (mean over the batch's graphs) and
+        backward -- through tsg_sag_nll_step_compact.  `y` int64 [G] graph labels on the device.  Same contract as
+        native_step: returns the loss (device scalar, a view into the flat gradient buffer) and WRITES every parameter's
+        .grad; dropout follows self.training, `dropout_mask` [G, nhid] injects the keep multipliers.  A label outside
+        [0, num_classes) raises at the next check_fused_status()."""
+        from . import _lib
+        dev = cb.label.device
+        G = int(np.asarray(node_ptr_host).shape[0]) - 1
+        if tuple(y.shape) != (G,):
+            raise ValueError(f"tsg: y has shape {tuple(y.shape)}, the batch has {G} graphs")
+        shape, head, ptrs, arena, arena_bytes, ws, ws_bytes, parr = self._native_setup(
+            cb, node_ptr_host, 1, 0.0, 0.0, dropout_mask, entry="nll")
+        flat, views = self._flat_grads()
+        emb = torch.empty(G, self.num_classes, dtype=torch.float32, device=dev) if return_emb else None
+        garr = (ctypes.c_void_p * 18)(*[v.data_ptr() for v in views])
+        loss = flat[-2:-1]
+        _lib.call("tsg_sag_nll_step_compact", ctypes.byref(shape), ctypes.byref(head), _lib.ptr(cb.label), _lib.ptr(cb.row),
+                  _lib.ptr(cb.col), _lib.ptr(cb.edge_ptr), _lib.ptr(ptrs), parr, _lib.ptr(y.to(torch.int64).contiguous()),
+                  _lib.ptr(dropout_mask.contiguous()) if dropout_mask is not None else None, garr, loss.data_ptr(),
+                  _lib.ptr(emb), _lib.ptr(arena), arena_bytes, _lib.ptr(ws), ws_bytes, _lib.stream_ptr())
+        if KEEP_ARENA:
+            global LAST_ARENA
+            LAST_ARENA = (shape, arena)
+        return (loss.view(()), emb) if return_emb else loss.view(())
+
+    def native_classify(self, cb, node_ptr_host, y: Optional[torch.Tensor] = None):
+        """`test()` of Code/sag/train.py:19-29 on one packed batch through tsg_sag_classify_compact: the model.eval()
+        forward (dropout off whatever self.training says), pred = out.max(dim=1)[1] and, with labels `y` (int64 [G] on
+        the device), the batch's correct count and summed NLL, reduced on the device.  Returns
+        (pred int64 [G], log-probabilities [G, C], correct int64 [1] or None, nll_sum float32 [1] or None)."""
+        from . import _lib
+        dev = cb.label.device
+        G = int(np.asarray(node_ptr_host).shape[0]) - 1
+        if y is not None and tuple(y.shape) != (G,):
+            raise ValueError(f"tsg: y has shape {tuple(y.shape)}, the batch has {G} graphs")
+        shape, head, ptrs, arena, arena_bytes, ws, ws_bytes, parr = self._native_setup(
+            cb, node_ptr_host, 1, 0.0, 0.0, None, entry="classify")
+        pred = torch.empty(G, dtype=torch.int64, device=dev)
+        logp = torch.empty(G, self.num_classes, dtype=torch.float32, device=dev)
+        correct = nll_sum = None
+        if y is not None:
+            y = y.to(torch.int64).contiguous()
+            correct = torch.empty(1, dtype=torch.int64, device=dev)
+            nll_sum = torch.empty(1, dtype=torch.float32, device=dev)
+        _lib.call("tsg_sag_classify_compact", ctypes.byref(shape), ctypes.byref(head), _lib.ptr(cb.label), _lib.ptr(cb.row),
+                  _lib.ptr(cb.col), _lib.ptr(cb.edge_ptr), _lib.ptr(ptrs), parr, _lib.ptr(y), _lib.ptr(pred), _lib.ptr(logp),
+                  _lib.ptr(correct), _lib.ptr(nll_sum), _lib.ptr(arena), arena_bytes, _lib.ptr(ws), ws_bytes,
+                  _lib.stream_ptr())
+        return pred, logp, correct, nll_sum
 
     def native_forward(self, cb, node_ptr_host, dropout_mask: Optional[torch.Tensor] = None):
         """First half of the native step: embeddings [G, C] (no autograd graph) + the context native_backward needs."""

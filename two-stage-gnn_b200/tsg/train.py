@@ -1,4 +1,5 @@
-"""2stg training step over packed batches: the public call a user of this framework makes.
+"""2stg training step over packed batches: the public call a user of this framework makes (ClassifierTrainer, at the
+end, is the supervised "original" setting of Code/sag/train.py).
 
 Mirrors the loop of Code/sag/train_triplet.py:198-214 (TNet forward -> MarginRankingLoss ->
 backward -> Adam step) with two differences that are the point of this framework: the step runs
@@ -15,6 +16,7 @@ from typing import Optional
 import numpy as np
 import torch
 import torch.distributed as dist
+import torch.nn.functional as F
 
 from . import ops
 
@@ -115,6 +117,18 @@ def _check_status():
     _nn.check_fused_status()
 
 
+def _all_reduce_native_flat(model, num_local: int, group) -> None:
+    """The native step's ONE collective: the model's flat buffer [grads | loss | weight] becomes
+    [n_r * grads, n_r * loss, n_r], is summed over the ranks and divided by sum_r n_r -- the global batch's mean loss and
+    its gradient, in place (n_r = this rank's triplets or graphs)."""
+    flat, _ = model._flat_grads()
+    flat[-1:].fill_(1.0)           # (NOT flat[-1] = 1.0: a Python scalar store is a blocking H2D copy -- measured
+                                   # 1.2 ms of host stall per step, 1.43 -> 1.87 ms at any N > 1: profiles/tools/scale_probe2.py)
+    flat.mul_(float(num_local))
+    dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
+    flat.div_(flat[-1].clone())
+
+
 class TripletTrainer:
     """model: tsg.nn.PackedSAGNet (or any module with the same forward signature)."""
 
@@ -139,12 +153,7 @@ class TripletTrainer:
             # K14: forward, loss and backward are ONE C-ABI call; gradients land in views of one flat buffer
             loss = self.model.native_step(x, node_ptr_host, triplets, self.margin)
             if world > 1:
-                flat, _ = self.model._flat_grads()
-                flat[-1:].fill_(1.0)           # (NOT flat[-1] = 1.0: a Python scalar store is a blocking H2D copy -- measured
-                                               # 1.2 ms of host stall per step, 1.43 -> 1.87 ms at any N > 1: profiles/tools/scale_probe2.py)
-                flat.mul_(float(triplets.size(0)))                       # [T_r * grads, T_r * loss, T_r]
-                dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=self.group)
-                flat.div_(flat[-1].clone())
+                _all_reduce_native_flat(self.model, int(triplets.size(0)), self.group)     # [T_r * grads, T_r * loss, T_r]
             loss = loss.clone()                                           # the buffer is rewritten by the next step
             self.opt.step()
             return loss
@@ -382,3 +391,109 @@ class TripletTrainer:
         loss = float(self.step(x, ei, nptr, tr).item())
         _check_status()
         return loss
+
+
+class ClassifierTrainer:
+    """The "original" setting of Code/sag/train.py: the classifier trained end to end with F.nll_loss on its own
+    log-softmax output (the baseline 2stg is compared with).  model: tsg.nn.PackedSAGNet, or any module with the same
+    forward signature that returns log-probabilities [G, C] and has `num_classes`."""
+
+    def __init__(self, model: torch.nn.Module, lr: float = 5e-4, weight_decay: float = 1e-4, group=None):
+        self.model, self.group = model, group
+        # Code/sag/train.py's torch.optim.Adam(lr, weight_decay); fused on the GPU as in TripletTrainer
+        params = list(model.parameters())
+        fused = bool(params) and all(p.is_cuda for p in params)
+        self.opt = torch.optim.Adam(params, lr=lr, weight_decay=weight_decay, fused=fused)
+
+    def _world(self) -> int:
+        return dist.get_world_size(self.group) if dist.is_initialized() else 1
+
+    def _native(self, x, edge_index, node_ptr_host) -> bool:
+        return (edge_index is None and getattr(self.model, "native_step_supported", None) is not None
+                and self.model.native_step_supported(x, node_ptr_host))
+
+    def step(self, x, edge_index, node_ptr_host: np.ndarray, y: torch.Tensor) -> torch.Tensor:
+        """One step of Code/sag/train.py:190-197 on a packed batch: F.nll_loss(model(data), data.y), backward, Adam.
+        x / edge_index (or an ops.CompactBatch and None) and y (int64 [G]) on the device.  Native (one C-ABI call for
+        forward, loss and backward) when the model supports the batch, else through autograd; TSG_NATIVE_STEP=0 forces
+        the latter.  With world > 1 the returned loss is the mean over the GLOBAL batch and the parameters receive its
+        gradient: one all-reduce of [G_r * grads, G_r * loss, G_r]."""
+        self.model.train()
+        world = self._world()
+        G = int(y.shape[0])
+        if self._native(x, edge_index, node_ptr_host):
+            loss = self.model.native_nll_step(x, node_ptr_host, y)
+            if world > 1:
+                _all_reduce_native_flat(self.model, G, self.group)
+            loss = loss.clone()                                           # the buffer is rewritten by the next step
+            self.opt.step()
+            return loss
+        out = self.model(x, edge_index, node_ptr_host)
+        loss = F.nll_loss(out, y)                                         # mean over THIS rank's graphs
+        self.opt.zero_grad(set_to_none=True)
+        loss.backward()
+        if world > 1:
+            loss = all_reduce_grads_and_loss(list(self.model.parameters()), loss, G, self.group)
+        self.opt.step()
+        return loss.detach()
+
+    def _batch(self, corpus, ids_host):
+        """ids -> (x, edge_index, node_ptr_host, y): the batch assembled on the GPU from the resident corpus (one small
+        upload of ids + offsets), its labels gathered on the device from the same staged ids."""
+        meta, B, nptr, eptr = corpus._stage(ids_host)
+        y = corpus.y.index_select(0, meta[:B])
+        if corpus.label is not None and getattr(self.model, "accepts_compact", False):
+            (x, _), ei = corpus.pack_compact_staged(meta, B, nptr, eptr), None
+        else:
+            x, ei, _ = corpus.pack_staged(meta, B, nptr, eptr)
+        return x, ei, nptr, y
+
+    def run_from_ids(self, corpus, id_batches) -> list:
+        """Training loop against an HBM-resident corpus (tsg.feeder.DeviceCorpus with labels): the host provides only
+        each step's graph ids (int64 numpy [B]); batch and labels are assembled on the GPU, and every step's loss is read
+        back into pinned memory without stalling the enqueue thread.  Returns the per-step losses."""
+        corpus.check_labels(self.model.num_classes)
+        host_losses = []
+        for ids in id_batches:
+            loss = self.step(*self._batch(corpus, ids))
+            h = torch.empty((), dtype=torch.float32, pin_memory=True)
+            h.copy_(loss, non_blocking=True)
+            host_losses.append(h)
+        torch.cuda.current_stream(corpus.device).synchronize()
+        _check_status()
+        return [float(h) for h in host_losses]
+
+    def evaluate(self, corpus, ids, batch_graphs: int = 4096):
+        """`test()` of Code/sag/train.py:19-29 over the graphs `ids` of the corpus in packed batches of `batch_graphs`:
+        (accuracy, mean NLL) of the model in eval mode, pred = out.max(dim=1)[1].  Per-batch totals stay on the device
+        and are read back once at the end, then summed in float64; under a process group every rank passes its own ids
+        and [correct, loss_sum, count] is all-reduced."""
+        corpus.check_labels(self.model.num_classes)
+        ids = np.asarray(ids, dtype=np.int64)
+        was_training = self.model.training
+        self.model.eval()
+        totals = []
+        try:
+            with torch.no_grad():
+                for s in range(0, ids.shape[0], batch_graphs):
+                    x, ei, nptr, y = self._batch(corpus, ids[s:s + batch_graphs])
+                    if self._native(x, ei, nptr):
+                        _, _, correct, nll_sum = self.model.native_classify(x, nptr, y)
+                    else:
+                        if ei is None and not getattr(self.model, "accepts_compact", False):
+                            x, ei = x.expand()
+                        out = self.model(x, ei, nptr)
+                        correct = (out.max(dim=1)[1] == y).sum().view(1)
+                        nll_sum = F.nll_loss(out, y, reduction="sum").view(1)
+                    totals.append(torch.cat([correct.double(), nll_sum.double()]))
+        finally:
+            self.model.train(was_training)
+        t = torch.stack(totals).cpu().numpy() if totals else np.zeros((0, 2))
+        _check_status()
+        acc = np.array([t[:, 0].sum(), t[:, 1].sum(), float(ids.shape[0])], dtype=np.float64)
+        if self._world() > 1:
+            red = torch.from_numpy(acc).to(corpus.device)
+            dist.all_reduce(red, op=dist.ReduceOp.SUM, group=self.group)
+            acc = red.cpu().numpy()
+        n = max(acc[2], 1.0)
+        return float(acc[0] / n), float(acc[1] / n)

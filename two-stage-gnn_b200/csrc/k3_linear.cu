@@ -43,23 +43,23 @@ __device__ __forceinline__ void cp_async16(float* smem_dst, const float* gsrc) {
 // as ONE contiguous 16-byte stream; K % 4 == 0 pads by 4 floats so every row stays 16-byte aligned.
 __host__ __device__ __forceinline__ int lin_pitch(int K) { return (K & 1) ? K : ((K & 3) == 0 ? K + 4 : K + 1); }
 
-// asynchronously stage rows [r0, r0+R) of X[N,K] into Xs[R][pitch] (rows past N are zero filled)
+// asynchronously stage rows [r0, r0+R) of X[N,K] (row stride ldx) into Xs[R][pitch] (rows past N are zero filled)
 __device__ __forceinline__ void stage_rows_async(float* Xs, const float* __restrict__ X, int r0, int R,
-                                                 int N, int K, int pitch) {
+                                                 int N, int K, int pitch, int ldx) {
   const int rows = min(R, N - r0);
-  const bool base16 = ((((size_t)(X + (size_t)r0 * K)) & 15) == 0);
-  if (pitch == K && base16) {                    // contiguous tile: 16-byte stream + scalar tail
+  const bool base16 = ((((size_t)(X + (size_t)r0 * ldx)) & 15) == 0);
+  if (pitch == K && ldx == K && base16) {        // contiguous tile: 16-byte stream + scalar tail
     const float* src = X + (size_t)r0 * K;
     const int total = rows * K, total4 = total & ~3;
     for (int i = threadIdx.x * 4; i < total4; i += LIN_THREADS * 4) cp_async16(Xs + i, src + i);
     for (int i = total4 + threadIdx.x; i < total; i += LIN_THREADS) cp_async4(Xs + i, src + i);
     for (int i = total + threadIdx.x; i < R * K; i += LIN_THREADS) Xs[i] = 0.f;
-  } else if ((K & 3) == 0 && base16) {           // 16-byte aligned rows, padded pitch
+  } else if ((K & 3) == 0 && (ldx & 3) == 0 && base16) {     // 16-byte aligned rows, padded pitch
     const int K4 = K >> 2;
     for (int i = threadIdx.x; i < R * K4; i += LIN_THREADS) {
       const int r = i / K4, k = (i - r * K4) * 4;
       float* dst = Xs + r * pitch + k;
-      if (r < rows) cp_async16(dst, X + (size_t)(r0 + r) * K + k);
+      if (r < rows) cp_async16(dst, X + (size_t)(r0 + r) * ldx + k);
       else { dst[0] = 0.f; dst[1] = 0.f; dst[2] = 0.f; dst[3] = 0.f; }
     }
   } else {
@@ -67,7 +67,7 @@ __device__ __forceinline__ void stage_rows_async(float* Xs, const float* __restr
     for (int r = w; r < R; r += LIN_THREADS / 32) {
       float* dst = Xs + r * pitch;
       if (r < rows) {
-        const float* src = X + (size_t)(r0 + r) * K;
+        const float* src = X + (size_t)(r0 + r) * ldx;
         for (int k = lane; k < K; k += 32) cp_async4(dst + k, src + k);
       } else {
         for (int k = lane; k < K; k += 32) dst[k] = 0.f;
@@ -137,10 +137,15 @@ __device__ __forceinline__ void row_epilogue(float (&u)[4], const bool (&ok)[4],
 
 // Y[N,M] = epilogue(X[N,K] . Wop + bias), Wop = W[K,M] or W[M,K]^T.  Persistent CTAs: W staged in
 // shared memory once, then a grid-stride loop over tiles of R = (256/CG)*2 rows.
+// A K too long for W's slab runs as consecutive launches over blocks of K (X row stride ldx): LIN_KACC_IN starts every
+// accumulator from Y, LIN_KPARTIAL stores it without bias and epilogue -- one k-ascending FMA chain per output, as in a
+// single pass.
+constexpr int LIN_KACC_IN = 1, LIN_KPARTIAL = 2;
 template <int CG>
 __global__ void __launch_bounds__(LIN_THREADS)
 k_linear_fwd(const float* __restrict__ X, const float* __restrict__ W, const float* __restrict__ bias,
-             float* __restrict__ Y, int N, int K, int M, int ldw, int ldy, int w_transposed, int flags) {
+             float* __restrict__ Y, int N, int K, int M, int ldw, int ldy, int w_transposed, int flags, int ldx,
+             int kmode) {
   extern __shared__ __align__(16) float smem[];
   constexpr int RS = LIN_THREADS / CG;
   constexpr int R = RS * LIN_RPT;
@@ -165,14 +170,14 @@ k_linear_fwd(const float* __restrict__ X, const float* __restrict__ W, const flo
   }
   const int num_tiles = (N + R - 1) / R;
   int buf = 0;
-  if ((int)blockIdx.x < num_tiles) stage_rows_async(Xs, X, blockIdx.x * R, R, N, K, pitch);
+  if ((int)blockIdx.x < num_tiles) stage_rows_async(Xs, X, blockIdx.x * R, R, N, K, pitch, ldx);
   for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
     const int r0 = tile * R;
     const int rows = min(R, N - r0);
     const int next = tile + gridDim.x;
     float* Xcur = Xs + (size_t)buf * R * pitch;
     if (next < num_tiles) {                      // prefetch the next tile into the other buffer
-      stage_rows_async(Xs + (size_t)(buf ^ 1) * R * pitch, X, next * R, R, N, K, pitch);
+      stage_rows_async(Xs + (size_t)(buf ^ 1) * R * pitch, X, next * R, R, N, K, pitch, ldx);
       cp_async_wait<1>();
     } else {
       cp_async_wait<0>();
@@ -182,7 +187,8 @@ k_linear_fwd(const float* __restrict__ X, const float* __restrict__ W, const flo
 #pragma unroll
     for (int j = 0; j < LIN_RPT; ++j)
 #pragma unroll
-      for (int c = 0; c < 4; ++c) acc[j][c] = 0.f;
+      for (int c = 0; c < 4; ++c)
+        acc[j][c] = (kmode & LIN_KACC_IN) && rs + j * RS < rows && ok[c] ? Y[(size_t)(r0 + rs + j * RS) * ldy + cg * 4 + c] : 0.f;
     const float* x0 = Xcur + (rs)*pitch;
     const float* x1 = Xcur + (rs + RS) * pitch;
     for (int k = 0; k < K; ++k) {
@@ -197,9 +203,11 @@ k_linear_fwd(const float* __restrict__ X, const float* __restrict__ W, const flo
 #pragma unroll
     for (int j = 0; j < LIN_RPT; ++j) {
       const int r = rs + j * RS;
+      if (!(kmode & LIN_KPARTIAL)) {
 #pragma unroll
-      for (int c = 0; c < 4; ++c) acc[j][c] += b4[c];
-      if (flags) row_epilogue<CG>(acc[j], ok, M, flags, gmask);
+        for (int c = 0; c < 4; ++c) acc[j][c] += b4[c];
+        if (flags) row_epilogue<CG>(acc[j], ok, M, flags, gmask);
+      }
       if (r < rows) {
         float* dst = Y + (size_t)(r0 + r) * ldy + cg * 4;
         if ((M & 3) == 0 && (ldy & 3) == 0) {
@@ -247,14 +255,14 @@ k_linear_fwd_dense(const float* __restrict__ X, const float* __restrict__ W, con
   }
   const int num_tiles = (N + R - 1) / R;
   int buf = 0;
-  if ((int)blockIdx.x < num_tiles) stage_rows_async(Xs, X, blockIdx.x * R, R, N, K, pitch);
+  if ((int)blockIdx.x < num_tiles) stage_rows_async(Xs, X, blockIdx.x * R, R, N, K, pitch, K);
   for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
     const int r0 = tile * R;
     const int rows = min(R, N - r0);
     const int next = tile + gridDim.x;
     const float* Xcur = Xs + (size_t)buf * R * pitch;
     if (next < num_tiles) {
-      stage_rows_async(Xs + (size_t)(buf ^ 1) * R * pitch, X, next * R, R, N, K, pitch);
+      stage_rows_async(Xs + (size_t)(buf ^ 1) * R * pitch, X, next * R, R, N, K, pitch, K);
       cp_async_wait<1>();
     } else {
       cp_async_wait<0>();
@@ -332,14 +340,14 @@ k_dense_epilogue_bwd(const float* __restrict__ X, const float* __restrict__ W, c
   }
   const int num_tiles = (N + R - 1) / R;
   int buf = 0;
-  if ((int)blockIdx.x < num_tiles) stage_rows_async(Xs, X, blockIdx.x * R, R, N, K, pitch);
+  if ((int)blockIdx.x < num_tiles) stage_rows_async(Xs, X, blockIdx.x * R, R, N, K, pitch, K);
   for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
     const int r0 = tile * R;
     const int rows = min(R, N - r0);
     const int next = tile + gridDim.x;
     float* Xcur = Xs + (size_t)buf * R * pitch;
     if (next < num_tiles) {                      // prefetch the next tile into the other buffer
-      stage_rows_async(Xs + (size_t)(buf ^ 1) * R * pitch, X, next * R, R, N, K, pitch);
+      stage_rows_async(Xs + (size_t)(buf ^ 1) * R * pitch, X, next * R, R, N, K, pitch, K);
       cp_async_wait<1>();
     } else {
       cp_async_wait<0>();
@@ -467,7 +475,7 @@ constexpr int LBW_GRID = TSG_NUM_SMS * 2;
 template <int NK, int U>
 __global__ void __launch_bounds__(256)
 k_linear_bwd_weight(const float* __restrict__ X, const float* __restrict__ dY, float* __restrict__ part,
-                    int N, int K, int M, int m0) {
+                    int N, int K, int M, int m0, int ldx) {
   extern __shared__ __align__(16) float smem[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
   float* acc = smem + (size_t)w * K * 32;                   // [K][32] private to this warp
@@ -493,7 +501,7 @@ k_linear_bwd_weight(const float* __restrict__ X, const float* __restrict__ dY, f
 #pragma unroll
       for (int c = 0; c < NK; ++c) {
         const int k = c * 32 + lane;
-        xv[u][c] = (rok && k < K) ? __ldg(X + (size_t)r * K + k) : 0.f;
+        xv[u][c] = (rok && k < K) ? __ldg(X + (size_t)r * ldx + k) : 0.f;
       }
     }
 #pragma unroll
@@ -711,6 +719,8 @@ static int pick_cg(int64_t M, int64_t K) {
   return c;
 }
 
+constexpr int LIN_KBLOCK = 256;       // K block of k_linear_fwd where W's whole slab does not fit
+
 static size_t lin_smem_bytes(int cg, int64_t K) {
   int R = (LIN_THREADS / cg) * LIN_RPT;
   return ((size_t)K * cg * 4 + 2 * (size_t)R * lin_pitch((int)K)) * sizeof(float);      // W + two X tiles
@@ -774,18 +784,28 @@ extern "C" int tsg_linear_fwd(const float* X, const float* W, const float* bias,
 #undef TSG_GOD
       continue;
     }
-    size_t smem = lin_smem_bytes(cg, K);
-    int R = (LIN_THREADS / cg) * LIN_RPT;
-    int tiles = (int)((N + R - 1) / R);
-    int grid = tiles < TSG_NUM_SMS * 4 ? tiles : TSG_NUM_SMS * 4;
+    // W's slab [K][4 cg] and two X tiles in shared memory; a K beyond that (the input gradient of a classifier layer
+    // with ~1,000 classes) runs in blocks of LIN_KBLOCK -- shapes that fit keep their single launch
+    const int64_t kb = lin_smem_bytes(cg, K) <= 227 * 1024 ? K : LIN_KBLOCK;
+    for (int64_t k0 = 0; k0 < K; k0 += kb) {
+      const int64_t kc = K - k0 < kb ? K - k0 : kb;
+      const int cgb = kb == K ? cg : pick_cg(mc, kc);
+      const int kmode = (k0 > 0 ? LIN_KACC_IN : 0) | (k0 + kc < K ? LIN_KPARTIAL : 0);
+      const float* Wb = w_transposed ? Wc + k0 : Wc + k0 * ldw;
+      size_t smem = lin_smem_bytes(cgb, kc);
+      int R = (LIN_THREADS / cgb) * LIN_RPT;
+      int tiles = (int)((N + R - 1) / R);
+      int grid = tiles < TSG_NUM_SMS * 4 ? tiles : TSG_NUM_SMS * 4;
 #define TSG_GO(C)                                                                                  \
-    rc = set_smem(k_linear_fwd<C>, smem, "linear_fwd"); if (rc) return rc;                          \
-    k_linear_fwd<C><<<grid, LIN_THREADS, smem, st>>>(X, Wc, bc, Yc, (int)N, (int)K, (int)mc, ldw, (int)M, w_transposed, flags)
-    switch (cg) {
-      case 1: TSG_GO(1); break; case 2: TSG_GO(2); break; case 4: TSG_GO(4); break;
-      case 8: TSG_GO(8); break; case 16: TSG_GO(16); break; default: TSG_GO(32); break;
-    }
+      rc = set_smem(k_linear_fwd<C>, smem, "linear_fwd"); if (rc) return rc;                        \
+      k_linear_fwd<C><<<grid, LIN_THREADS, smem, st>>>(X + k0, Wb, bc, Yc, (int)N, (int)kc, (int)mc, ldw, (int)M,      \
+                                                       w_transposed, flags, (int)K, kmode)
+      switch (cgb) {
+        case 1: TSG_GO(1); break; case 2: TSG_GO(2); break; case 4: TSG_GO(4); break;
+        case 8: TSG_GO(8); break; case 16: TSG_GO(16); break; default: TSG_GO(32); break;
+      }
 #undef TSG_GO
+    }
   }
   return check_launch("linear_fwd");
 }
@@ -870,24 +890,28 @@ extern "C" int tsg_linear_bwd_weight(const float* X, const float* dY, float* dW,
       return check_launch("linear_bwd_weight(dense)");
     }
   }
-  TSG_REQUIRE(K <= 256, "linear_bwd_weight: in_feat %lld > 256 not supported", (long long)K);
-  int nk = (int)((K + 31) / 32);
-  int nwarps = 8;
-  while (nwarps > 1 && (size_t)nwarps * K * 32 * 4 > 200 * 1024) --nwarps;
-  size_t smem = (size_t)nwarps * K * 32 * sizeof(float);
-  int grid = LBW_GRID;                       // fixed => the summation order never depends on the device
-  for (int m0 = 0; m0 < M; m0 += 32) {
+  // blocks of <= 256 input columns (one block up to 256; more for the 2 * nhid inputs of the head's lin1 from nhid 130),
+  // each the kernel's [kc][32] accumulators -- dW rows [k0, k0 + kc) are contiguous, and every entry keeps its order
+  const int grid = LBW_GRID;                 // fixed => the summation order never depends on the device
+  for (int64_t k0 = 0; k0 < K; k0 += 256) {
+    const int64_t kc = K - k0 < 256 ? K - k0 : 256;
+    int nk = (int)((kc + 31) / 32);
+    int nwarps = 8;
+    while (nwarps > 1 && (size_t)nwarps * kc * 32 * 4 > 200 * 1024) --nwarps;
+    size_t smem = (size_t)nwarps * kc * 32 * sizeof(float);
+    for (int m0 = 0; m0 < M; m0 += 32) {
 #define TSG_GO(NK_, U_)                                                                                    \
-    { int rc = set_smem(k_linear_bwd_weight<NK_, U_>, smem, "linear_bwd_weight"); if (rc) return rc;         \
-      k_linear_bwd_weight<NK_, U_><<<grid, nwarps * 32, smem, st>>>(X, dY, part, (int)N, (int)K, (int)M, m0); }
-    switch (nk) {
-      case 1: TSG_GO(1, 8); break; case 2: TSG_GO(2, 8); break; case 3: TSG_GO(3, 4); break;
-      case 4: TSG_GO(4, 4); break; case 5: TSG_GO(5, 2); break; case 6: TSG_GO(6, 2); break;
-      case 7: TSG_GO(7, 2); break; default: TSG_GO(8, 2); break;
-    }
+      { int rc = set_smem(k_linear_bwd_weight<NK_, U_>, smem, "linear_bwd_weight"); if (rc) return rc;       \
+        k_linear_bwd_weight<NK_, U_><<<grid, nwarps * 32, smem, st>>>(X + k0, dY, part, (int)N, (int)kc, (int)M, m0, (int)K); }
+      switch (nk) {
+        case 1: TSG_GO(1, 8); break; case 2: TSG_GO(2, 8); break; case 3: TSG_GO(3, 4); break;
+        case 4: TSG_GO(4, 4); break; case 5: TSG_GO(5, 2); break; case 6: TSG_GO(6, 2); break;
+        case 7: TSG_GO(7, 2); break; default: TSG_GO(8, 2); break;
+      }
 #undef TSG_GO
+    }
+    launch_partial_sum_final(part, dW + k0 * M, (int)(kc * M), nullptr, grid, (int)(kc * M), st);
   }
-  launch_partial_sum_final(part, dW, (int)(K * M), nullptr, grid, (int)(K * M), st);
   return check_launch("linear_bwd_weight");
 }
 

@@ -409,9 +409,17 @@ int tsg_coarsen_edges(const int64_t* row, const int64_t* col, const float* weigh
 
 /* ------------------------------------------------------------------------------------------
  * K12  stage-2 evaluation heads on graph embeddings (SURVEY 8f n4)
- *   tsg_knn_predict replaces KNeighborsClassifier(n_neighbors=3).fit(train).predict(query) of `evaluate`
+ *   tsg_knn_classify replaces KNeighborsClassifier(n_neighbors=k).fit(train).predict(query) of `evaluate`
  *     (Code/sage+gat+diffpool/train_triplet.py:80-85): Euclidean, uniform weights; distance ties -> lower
- *     train index, vote ties -> lower class id.  k <= 8, num_classes <= 16.
+ *     train index, vote ties -> lower class id.  1 <= k <= 32 (fewer than k train rows: all of them vote),
+ *     1 <= num_classes <= 1024.  pred int64 [num_query]; with query_labels, *correct (int64, device) = #(pred ==
+ *     label), an integer reduction (correct NULL: not written; with num_query > 0 correct needs query_labels).  A train or query label
+ *     outside [0, num_classes) is clamped for the read and ORs TSG_SAG_LABEL_RANGE into *status (nullable: not
+ *     reported).  tsg_knn_predict is tsg_knn_classify(query_labels = correct = status = NULL).
+ *   tsg_mlp1_predict is that MLP's forward over num_rows rows (params as for tsg_mlp1_train): pred int64 [num_rows] =
+ *     first-index argmax of the logits; logits (nullable) [num_rows, classes]; labels / correct / status as for
+ *     tsg_knn_classify.  Every unit is the trainer's own fmaf chain over its input index ascending, so the logits
+ *     equal those the trainer's forward computes for the same parameters, bit for bit.
  *   tsg_mlp1_train replaces the stage-2 classifier loop of `evaluate_mlp` (train_triplet.py:148-165):
  *     MLP dim -> hidden1 -> hidden2 -> classes with LeakyReLU(slope), Adam, ONE sample per step in the given
  *     order; all num_samples steps run inside one CTA with weights and moments in shared memory.
@@ -422,6 +430,14 @@ int tsg_coarsen_edges(const int64_t* row, const int64_t* col, const float* weigh
 int tsg_knn_predict(const float* train, const int64_t* train_labels, const float* query,
                     int64_t num_train, int64_t num_query, int64_t dim, int k, int num_classes,
                     int64_t* pred, void* stream);
+int tsg_knn_classify(const float* train, const int64_t* train_labels, const float* query,
+                     const int64_t* query_labels /*nullable*/, int64_t num_train, int64_t num_query, int64_t dim, int k,
+                     int num_classes, int64_t* pred, int64_t* correct /*nullable*/, int32_t* status /*nullable*/,
+                     void* stream);
+int tsg_mlp1_predict(const float* emb, const int64_t* labels /*nullable*/, int64_t num_rows, int64_t dim,
+                     int64_t hidden1, int64_t hidden2, int64_t num_classes, const float* params, float slope,
+                     int64_t* pred, float* logits /*nullable*/, int64_t* correct /*nullable*/,
+                     int32_t* status /*nullable*/, void* stream);
 int tsg_mlp1_train(const float* emb, const int64_t* labels, int64_t num_samples, int64_t dim,
                    int64_t hidden1, int64_t hidden2, int64_t num_classes,
                    float* params, float* adam_m, float* adam_v, int64_t step0,

@@ -78,6 +78,8 @@ _PROTOTYPES = {
     "tsg_linkpred_loss_fwd": (I, [P, P, P, P, I64, I64, ctypes.c_double, F32, P, P, SZ, P]),
     "tsg_linkpred_loss_bwd": (I, [P, P, P, P, I64, I64, ctypes.c_double, F32, P, P, P]),
     "tsg_knn_predict": (I, [P, P, P, I64, I64, I64, I, I, P, P]),
+    "tsg_knn_classify": (I, [P, P, P, P, I64, I64, I64, I, I, P, P, P, P]),
+    "tsg_mlp1_predict": (I, [P, P, I64, I64, I64, I64, I64, P, F32, P, P, P, P, P]),
     "tsg_mlp1_train": (I, [P, P, I64, I64, I64, I64, I64, P, P, P, I64, F32, F32, F32, F32, F32, P, P]),
     "tsg_tu_load": (I, [c_char_p, I, I64, P]),
     "tsg_tu_sizes": (I, [P, P]),

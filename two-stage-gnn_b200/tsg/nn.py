@@ -141,22 +141,24 @@ def sag_arena_view(shape, arena: torch.Tensor, level: int, field: str) -> torch.
 LABEL_RANGE = 8           # TSG_SAG_LABEL_RANGE (include/tsg.h)
 
 
-def check_fused_status() -> None:
-    """Look at the status word the verifying kernels (K1d, K13, and the label checks of the supervised step and the
-    classification forward) OR-ed their bits into since the last call -- ONE device
+def check_fused_status(already_read: Optional[dict] = None) -> None:
+    """Look at the status word the verifying kernels (K1d, K13, and the label checks of the supervised step, the
+    classification forward and the stage-2 heads) OR-ed their bits into since the last call -- ONE device
     read per device, so callers do it where they synchronise anyway (loss read-back, end of a feeder loop, tests).  A non-zero word means a graph's
     edge list was not what those kernels require (endpoints in range, no self loops, sorted by (row, col), symmetric:
-    the TUDataset / TU-loader form); its embedding was zeroed.  There is no silent fallback: this raises."""
+    the TUDataset / TU-loader form); its embedding was zeroed.  There is no silent fallback: this raises.
+    `already_read` {device index: word}: words the caller copied back together with its own results (no second read)."""
     if not _STATUS_DIRTY:
         return
     bits = 0
     for i in list(_STATUS_DIRTY):
-        bits |= int(_STATUS[i].item())
+        bits |= int(already_read[i]) if already_read and i in already_read else int(_STATUS[i].item())
         _STATUS[i].zero_()
     _STATUS_DIRTY.clear()
     if bits & LABEL_RANGE:
-        raise RuntimeError("tsg: a graph label lies outside [0, num_classes) (status bit 8, set by the supervised step or "
-                           "the classification forward); it was clamped, so the loss and the accuracy are invalid")
+        raise RuntimeError("tsg: a graph label lies outside [0, num_classes) (status bit 8, set by the supervised step, "
+                           "the classification forward or a stage-2 head); it was clamped, so the loss and the accuracy "
+                           "are invalid")
     if bits:
         names = [n for b, n in ((1, "edge endpoint out of range / self loop"), (2, "edge list not sorted by (row, col)"),
                                 (4, "edge list not symmetric")) if bits & b]
@@ -518,6 +520,9 @@ class PackedSAGNet(torch.nn.Module):
                   _lib.ptr(cb.col), _lib.ptr(cb.edge_ptr), _lib.ptr(ptrs), parr, _lib.ptr(y), _lib.ptr(pred), _lib.ptr(logp),
                   _lib.ptr(correct), _lib.ptr(nll_sum), _lib.ptr(arena), arena_bytes, _lib.ptr(ws), ws_bytes,
                   _lib.stream_ptr())
+        if KEEP_ARENA:
+            global LAST_ARENA
+            LAST_ARENA = (shape, arena)
         return pred, logp, correct, nll_sum
 
     def native_forward(self, cb, node_ptr_host, dropout_mask: Optional[torch.Tensor] = None):

@@ -129,6 +129,41 @@ def _all_reduce_native_flat(model, num_local: int, group) -> None:
     flat.div_(flat[-1].clone())
 
 
+def _native_ok(model, x, edge_index, node_ptr_host) -> bool:
+    """The batch runs on the model's native (K14) entries: compact input the model's shape checks accept."""
+    return (edge_index is None and getattr(model, "native_step_supported", None) is not None
+            and model.native_step_supported(x, node_ptr_host))
+
+
+def gather_score_reduce(train_emb: torch.Tensor, train_y: torch.Tensor, query_emb: torch.Tensor, query_y: torch.Tensor,
+                        score, group=None) -> torch.Tensor:
+    """Stage-2 scoring of a sharded evaluation: every rank holds its own train rows (embeddings [M_r, D], labels [M_r])
+    and its own queries.  The train rows of all ranks are all-gathered in rank order (the shard sizes first: they may
+    differ, so each shard travels padded to the largest), `score(train_emb, train_y, query_emb, query_y)` -> int64 [1]
+    correct count runs against the gathered set on every rank, and [correct, count] is all-reduced.  Returns int64 [2]
+    = [correct, count] over all ranks.  Without a process group (or at world size 1) nothing is exchanged."""
+    world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
+    if world > 1:
+        dev = train_emb.device
+        n = torch.full((1,), train_emb.size(0), dtype=torch.int64, device=dev)
+        sizes = [torch.empty_like(n) for _ in range(world)]
+        dist.all_gather(sizes, n, group=group)
+        sizes = torch.cat(sizes).tolist()
+        m = max(sizes)
+
+        def gather(t):
+            padded = torch.cat([t, t.new_zeros((m - t.size(0),) + tuple(t.shape[1:]))]) if t.size(0) < m else t.contiguous()
+            parts = [torch.empty_like(padded) for _ in range(world)]
+            dist.all_gather(parts, padded, group=group)
+            return torch.cat([p[:s] for p, s in zip(parts, sizes)])
+        train_emb, train_y = gather(train_emb), gather(train_y)
+    correct = score(train_emb, train_y, query_emb, query_y).reshape(1).to(torch.int64)
+    tot = torch.cat([correct, torch.full((1,), query_emb.size(0), dtype=torch.int64, device=correct.device)])
+    if world > 1:
+        dist.all_reduce(tot, op=dist.ReduceOp.SUM, group=group)
+    return tot
+
+
 class TripletTrainer:
     """model: tsg.nn.PackedSAGNet (or any module with the same forward signature)."""
 
@@ -392,6 +427,104 @@ class TripletTrainer:
         _check_status()
         return loss
 
+    def _pack(self, corpus, ids_host):
+        """ids -> (x or an ops.CompactBatch, edge_index or None, node_ptr_host), assembled on the GPU from the corpus."""
+        if corpus.label is not None and getattr(self.model, "accepts_compact", False):
+            (x, nptr), ei = corpus.pack_compact(ids_host), None
+        else:
+            x, ei, nptr = corpus.pack(ids_host)
+        return x, ei, nptr
+
+    def _embed(self, corpus, ids: np.ndarray, batch_graphs: int) -> torch.Tensor:
+        model = self.model
+        was_training = model.training
+        model.eval()
+        parts = []
+        try:
+            with torch.no_grad():
+                for s in range(0, ids.shape[0], batch_graphs):
+                    x, ei, nptr = self._pack(corpus, ids[s:s + batch_graphs])
+                    if _native_ok(model, x, ei, nptr):
+                        parts.append(model.native_classify(x, nptr)[1])      # the head's log-softmax output = embedding
+                    else:
+                        if ei is None and not getattr(model, "accepts_compact", False):
+                            x, ei = x.expand()
+                        parts.append(model(x, ei, nptr))
+        finally:
+            model.train(was_training)
+        if not parts:
+            return torch.empty(0, model.num_classes, dtype=torch.float32, device=corpus.device)
+        return parts[0] if len(parts) == 1 else torch.cat(parts)
+
+    def embed(self, corpus, ids, batch_graphs: int = 4096) -> torch.Tensor:
+        """Embeddings [len(ids), D] on the device of the graphs `ids` of an HBM-resident corpus (tsg.feeder.DeviceCorpus),
+        row i = graph ids[i] (duplicates allowed): what the stage-2 loops of Code/sag/train_triplet.py:36-58,86-99 feed
+        their classifiers.  The model runs in eval mode (dropout off, as in ClassifierTrainer.evaluate) in packed batches
+        of `batch_graphs`, natively (tsg_sag_classify_compact: K13 where the shape allows, then the head) where
+        native_step_supported holds, else through a torch.no_grad() forward; the caller's training flag is restored.
+        The status word is checked once, at the end."""
+        if batch_graphs < 1:
+            raise ValueError("tsg: batch_graphs must be at least 1")
+        out = self._embed(corpus, np.asarray(ids, dtype=np.int64).reshape(-1), int(batch_graphs))
+        _check_status()
+        return out
+
+    def evaluate(self, corpus, train_ids, eval_ids, head: str = "knn", k: int = 3, mlp_epochs: int = 1, seed: int = 0,
+                 num_classes: Optional[int] = None, batch_graphs: int = 4096) -> float:
+        """The 2stg accuracy: the encoder's embeddings (`embed`) of `train_ids` fit a stage-2 classifier that labels
+        `eval_ids`; labels come from `corpus.y`.
+          head="knn": KNeighborsClassifier(n_neighbors=k) on the train embeddings (Code/sage+gat+diffpool/
+            train_triplet.py:80-85) -- tsg_knn_classify, k <= 32, up to 1,024 classes.
+          head="mlp": evaluate_mlp's classifier (tsg.heads.Mlp1Classifier) trained one sample per step in the order of
+            `train_ids` for `mlp_epochs` passes, then scored with tsg_mlp1_predict.  Its initial weights are drawn from
+            `seed` under torch.random.fork_rng, so evaluating does not move the caller's RNG stream.
+        `num_classes` = the graph-class count (default: 1 + the corpus's largest label; NOT model.num_classes, which for
+        a triplet model is the embedding width); every label is checked against it on the host, once per corpus.
+        Under a process group each rank passes its own ids: train rows are all-gathered in rank order, every rank fits
+        the same classifier on them and scores its own queries, and [correct, count] is all-reduced
+        (gather_score_reduce).  One device-to-host read, at the end (plus the shard sizes under a process group)."""
+        from . import heads, nn as tnn
+        if head not in ("knn", "mlp"):
+            raise ValueError(f"tsg: head must be 'knn' or 'mlp', not {head!r}")
+        train_ids = np.asarray(train_ids, dtype=np.int64).reshape(-1)
+        eval_ids = np.asarray(eval_ids, dtype=np.int64).reshape(-1)
+        if train_ids.size == 0 or eval_ids.size == 0:
+            raise ValueError("tsg: evaluate needs at least one train id and one eval id")
+        if not 1 <= int(k) <= 32:
+            raise ValueError(f"tsg: k must be in [1, 32], not {k}")
+        if head == "mlp" and int(mlp_epochs) < 1:
+            raise ValueError("tsg: mlp_epochs must be at least 1")
+        if batch_graphs < 1:
+            raise ValueError("tsg: batch_graphs must be at least 1")
+        if corpus.y is None:
+            raise ValueError("tsg: the corpus carries no graph labels (y)")
+        if num_classes is None:
+            y_all = corpus.y_host if corpus.y_host is not None else corpus.y.cpu().numpy()
+            num_classes = int(y_all.max()) + 1 if y_all.size else 1
+        C = int(num_classes)
+        corpus.check_labels(C)
+        dev = corpus.device
+        status = tnn._status_word(dev)
+        train_emb = self._embed(corpus, train_ids, int(batch_graphs))
+        eval_emb = self._embed(corpus, eval_ids, int(batch_graphs))
+        take = lambda ids: corpus.y.index_select(0, torch.from_numpy(ids).to(dev))
+        train_y, eval_y = take(train_ids), take(eval_ids)
+        if head == "knn":
+            def score(a, ya, q, yq):
+                return heads.knn_classify(a, ya, q, yq, k=int(k), num_classes=C, status=status)[1]
+        else:
+            def score(a, ya, q, yq):
+                with torch.random.fork_rng(devices=[]):
+                    torch.manual_seed(int(seed))
+                    clf = heads.Mlp1Classifier(a.size(1), dev, num_classes=C)
+                for _ in range(int(mlp_epochs)):
+                    clf.fit(a, ya)
+                return clf.score(q, yq, status=status)
+        tot = gather_score_reduce(train_emb, train_y, eval_emb, eval_y, score, self.group)
+        host = torch.cat([tot, status.to(torch.int64)]).cpu()            # the one read: totals and the status word
+        tnn.check_fused_status({status.device.index: int(host[2])})
+        return float(host[0]) / max(float(host[1]), 1.0)
+
 
 class ClassifierTrainer:
     """The "original" setting of Code/sag/train.py: the classifier trained end to end with F.nll_loss on its own
@@ -409,8 +542,7 @@ class ClassifierTrainer:
         return dist.get_world_size(self.group) if dist.is_initialized() else 1
 
     def _native(self, x, edge_index, node_ptr_host) -> bool:
-        return (edge_index is None and getattr(self.model, "native_step_supported", None) is not None
-                and self.model.native_step_supported(x, node_ptr_host))
+        return _native_ok(self.model, x, edge_index, node_ptr_host)
 
     def step(self, x, edge_index, node_ptr_host: np.ndarray, y: torch.Tensor) -> torch.Tensor:
         """One step of Code/sag/train.py:190-197 on a packed batch: F.nll_loss(model(data), data.y), backward, Adam.

@@ -72,6 +72,26 @@ int tsg_pack_batch_compact(const int64_t* ids, const int64_t* out_node_ptr, cons
                            int64_t batch_graphs, const int64_t* corpus_node_ptr, const int64_t* corpus_edge_ptr,
                            const int32_t* corpus_row, const int32_t* corpus_col, const int32_t* corpus_label,
                            int32_t* label_out, int32_t* row_out, int32_t* col_out, void* stream);
+/* K0d: a dense-encoder batch (GraphSAGE / GAT / DiffPool) in ONE launch, for a corpus whose per-graph edge lists are
+ * coalesced and symmetric (sorted by (row, col), loop free, (r, c) <=> (c, r); graph-local int32 endpoints).
+ *   replaces: the reference's per-graph padded numpy adjacency / feature tensors and their `torch.Tensor([ndarray])`
+ *   marshaling (Code/sage+gat+diffpool/tripletnet.py:18-33, load_data.py:74-87 padding to max_nodes), with the node
+ *   features = rows of the shared feature table by node position (train_triplet.py:379-385).
+ *   Writes for graph b = corpus graph ids[b]: x_out rows out_node_ptr[b] + i = table[i] (table [max_nodes, feat] fp32),
+ *   has_pad[b] = (n_b < max_nodes), and -- when rowptr is given -- the RAW 0/1 CSR of the packed adjacency exactly as
+ *   tsg_csr_build(TSG_CSR_RAW) builds it from the expanded edge_index: rowptr [num_nodes + 1], colidx / val
+ *   [num_edges] serve BOTH orientations (symmetric), t_eid (nullable) = the src-major eid = identity, eid (nullable) =
+ *   the dst-major eid = position of the reverse edge.  Row starts come from run boundaries: no scan, no atomics.
+ *   The promise is verified per graph; violations OR TSG_FUSED_* bits (1 range / self loop, 2 order, 4 symmetry) into
+ *   *status (int32, device) and that graph's CSR is replaced by one whose indices stay in range.  rowptr == NULL:
+ *   x_out and has_pad only (callers that build the CSR with tsg_csr_build).  Sizes below 2^31 (num_nodes + num_edges);
+ *   max_nodes + 2 ints of shared memory per CTA (graphs of up to 12,286 nodes); TSG_EINVAL otherwise. */
+int tsg_pack_dense_batch(const int64_t* ids, const int64_t* out_node_ptr, const int64_t* out_edge_ptr,
+                         int64_t batch_graphs, int64_t num_nodes, int64_t num_edges, const int64_t* corpus_node_ptr,
+                         const int64_t* corpus_edge_ptr, const int32_t* corpus_row, const int32_t* corpus_col,
+                         const float* table, int64_t max_nodes, int64_t feat, float* x_out, uint8_t* has_pad,
+                         int32_t* rowptr /*nullable*/, int32_t* colidx, float* val, int32_t* eid /*nullable*/,
+                         int32_t* t_eid /*nullable*/, int32_t* status, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * K1  CSR construction + GCN normalisation

@@ -6,6 +6,8 @@ once (DD: 1,168 graphs = 14 MB) and a step ships only graph ids; `tsg_pack_batch
 batch at HBM speed."""
 from __future__ import annotations
 
+from dataclasses import dataclass
+
 import numpy as np
 import torch
 
@@ -139,6 +141,89 @@ class DeviceCorpus:
              ptr(self.row), ptr(self.col), ptr(self.label), ptr(label), ptr(rc[0]), ptr(rc[1]), stream_ptr())
         return CompactBatch(label, rc[0], rc[1], d_nptr, d_eptr, self.feat, int(np.diff(eptr).max()) if B else 0,
                             self.coalesced), nptr
+
+    def check_dense(self, ids_host, table: torch.Tensor, max_nodes: int) -> np.ndarray:
+        """The host-side checks of `pack_dense` (no device work): -> the ids as int64 numpy.  ValueError for a corpus with
+        per-node feature rows, an empty id list, an id outside the corpus, a graph larger than `max_nodes` (named: the
+        reference drops such graphs when it loads the dataset, load_data.py), a batch without any edge and a table that
+        is not [>= max_nodes, F] fp32."""
+        if self.x is not None:
+            raise ValueError("tsg: pack_dense takes its features from the position-indexed table; this corpus carries "
+                             "per-node feature rows (dense_x)")
+        ids = np.asarray(ids_host, dtype=np.int64).reshape(-1)
+        if ids.size == 0:
+            raise ValueError("tsg: pack_dense needs at least one graph id")
+        if int(ids.min()) < 0 or int(ids.max()) >= self.num_graphs:
+            raise ValueError(f"tsg: graph ids must lie in [0, {self.num_graphs})")
+        max_nodes = int(max_nodes)
+        if max_nodes < 1:
+            raise ValueError("tsg: max_nodes must be at least 1")
+        n = self.n[ids]
+        if int(n.max()) > max_nodes:
+            at = int(np.argmax(n))
+            raise ValueError(f"tsg: graph {int(ids[at])} has {int(n[at])} nodes, more than max_nodes = {max_nodes}")
+        if int(self.e[ids].sum()) == 0:
+            raise ValueError("tsg: the chosen graphs have no edges; the dense encoders' kernels need at least one edge "
+                             "per batch (pack edge-free graphs together with others)")
+        if table.dim() != 2 or table.size(0) < max_nodes:
+            raise ValueError(f"tsg: the feature table must be [max_nodes = {max_nodes}, F], not {tuple(table.shape)}")
+        if table.dtype != torch.float32:
+            raise ValueError(f"tsg: the feature table must be float32, not {table.dtype}")
+        return ids
+
+    def pack_dense(self, ids_host, table: torch.Tensor, max_nodes: int, want_eid: bool = False) -> "DenseBatch":
+        """-> DenseBatch: what the packed dense encoders (tsg.dense.PackedGcnEncoder, tsg.gat.PackedGatEncoder,
+        tsg.diffpool.PackedSoftPoolEncoder) take for the graphs `ids_host` (duplicates allowed): x = rows of `table`
+        ([>= max_nodes, F] fp32 on the device) by node position, the RAW 0/1 CSR of the packed adjacency in both
+        orientations (eids with `want_eid`: GAT's backward needs them), graph offsets and has-padded-row flags.
+        One small staged upload (ids + offsets), then one launch (K0d, tsg_pack_dense_batch), which verifies the
+        coalesced promise per graph: a violation raises at the next tsg.nn.check_fused_status().  A corpus that is not
+        coalesced takes the general path with the same result: K0 tsg_pack_batch + K1 build_csr(CSR_RAW)."""
+        ids = self.check_dense(ids_host, table, max_nodes)
+        return self.pack_dense_staged(*self._stage(ids), table, max_nodes, want_eid)
+
+    def pack_dense_staged(self, meta: torch.Tensor, B: int, nptr: np.ndarray, eptr: np.ndarray, table: torch.Tensor,
+                          max_nodes: int, want_eid: bool = False) -> "DenseBatch":
+        """`pack_dense` when ids + offsets are already on the device (`meta` = [ids | nptr | eptr], int64) and the ids
+        passed `check_dense`."""
+        from . import nn as tnn, ops
+        d_ids, d_nptr, d_eptr = meta[:B], meta[B:2 * B + 1], meta[2 * B + 1:]
+        N, E, F = int(nptr[-1]), int(eptr[-1]), int(table.size(1))
+        dev = self.device
+        table = table.contiguous()
+        x = torch.empty(N, F, dtype=torch.float32, device=dev)
+        has_pad = torch.empty(B, dtype=torch.bool, device=dev)
+        i32 = dict(dtype=torch.int32, device=dev)
+        if self.coalesced:
+            rowptr, colidx = torch.empty(N + 1, **i32), torch.empty(E, **i32)
+            val = torch.empty(E, dtype=torch.float32, device=dev)
+            eid, t_eid = (torch.empty(E, **i32), torch.empty(E, **i32)) if want_eid else (None, None)
+            status = tnn._status_word(dev)
+            call("tsg_pack_dense_batch", ptr(d_ids), ptr(d_nptr), ptr(d_eptr), B, N, E, ptr(self.node_ptr),
+                 ptr(self.edge_ptr), ptr(self.row), ptr(self.col), ptr(table), int(max_nodes), F, ptr(x), ptr(has_pad),
+                 ptr(rowptr), ptr(colidx), ptr(val), ptr(eid), ptr(t_eid), ptr(status), stream_ptr())
+            # symmetric lists: the src-major orientation is the same arrays; only the eids differ
+            csr = ops.CSR(rowptr, colidx, val, eid, rowptr, colidx, val, t_eid, N)
+        else:
+            _, ei, _ = self.pack_staged(meta, B, nptr, eptr)
+            csr = ops.build_csr(ops.EdgeList.from_edge_index(ei), N, mode=ops.CSR_RAW, want_eid=want_eid)
+            call("tsg_pack_dense_batch", ptr(d_ids), ptr(d_nptr), ptr(d_eptr), B, N, E, ptr(self.node_ptr),
+                 ptr(self.edge_ptr), None, None, ptr(table), int(max_nodes), F, ptr(x), ptr(has_pad),
+                 None, None, None, None, None, None, stream_ptr())
+        return DenseBatch(x, csr, d_nptr, has_pad, nptr, int(max_nodes))
+
+
+@dataclass
+class DenseBatch:
+    """A packed batch in the form the dense encoders take (DeviceCorpus.pack_dense).  `csr` is what
+    ops.build_csr(CSR_RAW) returns for the expanded edge list (tile_ptr / tma_ok unset); `graph_ptr` int64 [B+1] and
+    `has_pad` bool [B] (n_b < max_nodes) live on the device, `node_ptr_host` is the same offsets in host memory."""
+    x: torch.Tensor
+    csr: "ops.CSR"
+    graph_ptr: torch.Tensor
+    has_pad: torch.Tensor
+    node_ptr_host: np.ndarray
+    max_nodes: int
 
 
 class DeviceRagged:

@@ -164,6 +164,55 @@ def gather_score_reduce(train_emb: torch.Tensor, train_y: torch.Tensor, query_em
     return tot
 
 
+def _stage2_args(corpus, train_ids, eval_ids, head, k, mlp_epochs, num_classes, batch_graphs):
+    """The host-side validation of a 2stg evaluation (before any device work): -> (train ids, eval ids, class count)."""
+    if head not in ("knn", "mlp"):
+        raise ValueError(f"tsg: head must be 'knn' or 'mlp', not {head!r}")
+    train_ids = np.asarray(train_ids, dtype=np.int64).reshape(-1)
+    eval_ids = np.asarray(eval_ids, dtype=np.int64).reshape(-1)
+    if train_ids.size == 0 or eval_ids.size == 0:
+        raise ValueError("tsg: evaluate needs at least one train id and one eval id")
+    if not 1 <= int(k) <= 32:
+        raise ValueError(f"tsg: k must be in [1, 32], not {k}")
+    if head == "mlp" and int(mlp_epochs) < 1:
+        raise ValueError("tsg: mlp_epochs must be at least 1")
+    if batch_graphs < 1:
+        raise ValueError("tsg: batch_graphs must be at least 1")
+    if corpus.y is None:
+        raise ValueError("tsg: the corpus carries no graph labels (y)")
+    if num_classes is None:
+        y_all = corpus.y_host if corpus.y_host is not None else corpus.y.cpu().numpy()
+        num_classes = int(y_all.max()) + 1 if y_all.size else 1
+    C = int(num_classes)
+    corpus.check_labels(C)
+    return train_ids, eval_ids, C
+
+
+def _stage2_accuracy(corpus, status, train_emb, eval_emb, train_ids, eval_ids, head, k, mlp_epochs, seed, C, group):
+    """The scoring half of a 2stg evaluation on embeddings already computed: labels gathered from `corpus.y`, the kNN or
+    MLP head (K12), gather_score_reduce under a process group, and ONE device-to-host read of the totals together with
+    the status word (`status`, which the embedding passes may also have written)."""
+    from . import heads, nn as tnn
+    dev = corpus.device
+    take = lambda ids: corpus.y.index_select(0, torch.from_numpy(ids).to(dev))
+    train_y, eval_y = take(train_ids), take(eval_ids)
+    if head == "knn":
+        def score(a, ya, q, yq):
+            return heads.knn_classify(a, ya, q, yq, k=int(k), num_classes=C, status=status)[1]
+    else:
+        def score(a, ya, q, yq):
+            with torch.random.fork_rng(devices=[]):
+                torch.manual_seed(int(seed))
+                clf = heads.Mlp1Classifier(a.size(1), dev, num_classes=C)
+            for _ in range(int(mlp_epochs)):
+                clf.fit(a, ya)
+            return clf.score(q, yq, status=status)
+    tot = gather_score_reduce(train_emb, train_y, eval_emb, eval_y, score, group)
+    host = torch.cat([tot, status.to(torch.int64)]).cpu()            # the one read: totals and the status word
+    tnn.check_fused_status({status.device.index: int(host[2])})
+    return float(host[0]) / max(float(host[1]), 1.0)
+
+
 class TripletTrainer:
     """model: tsg.nn.PackedSAGNet (or any module with the same forward signature)."""
 
@@ -483,47 +532,13 @@ class TripletTrainer:
         Under a process group each rank passes its own ids: train rows are all-gathered in rank order, every rank fits
         the same classifier on them and scores its own queries, and [correct, count] is all-reduced
         (gather_score_reduce).  One device-to-host read, at the end (plus the shard sizes under a process group)."""
-        from . import heads, nn as tnn
-        if head not in ("knn", "mlp"):
-            raise ValueError(f"tsg: head must be 'knn' or 'mlp', not {head!r}")
-        train_ids = np.asarray(train_ids, dtype=np.int64).reshape(-1)
-        eval_ids = np.asarray(eval_ids, dtype=np.int64).reshape(-1)
-        if train_ids.size == 0 or eval_ids.size == 0:
-            raise ValueError("tsg: evaluate needs at least one train id and one eval id")
-        if not 1 <= int(k) <= 32:
-            raise ValueError(f"tsg: k must be in [1, 32], not {k}")
-        if head == "mlp" and int(mlp_epochs) < 1:
-            raise ValueError("tsg: mlp_epochs must be at least 1")
-        if batch_graphs < 1:
-            raise ValueError("tsg: batch_graphs must be at least 1")
-        if corpus.y is None:
-            raise ValueError("tsg: the corpus carries no graph labels (y)")
-        if num_classes is None:
-            y_all = corpus.y_host if corpus.y_host is not None else corpus.y.cpu().numpy()
-            num_classes = int(y_all.max()) + 1 if y_all.size else 1
-        C = int(num_classes)
-        corpus.check_labels(C)
-        dev = corpus.device
-        status = tnn._status_word(dev)
+        from . import nn as tnn
+        train_ids, eval_ids, C = _stage2_args(corpus, train_ids, eval_ids, head, k, mlp_epochs, num_classes, batch_graphs)
+        status = tnn._status_word(corpus.device)
         train_emb = self._embed(corpus, train_ids, int(batch_graphs))
         eval_emb = self._embed(corpus, eval_ids, int(batch_graphs))
-        take = lambda ids: corpus.y.index_select(0, torch.from_numpy(ids).to(dev))
-        train_y, eval_y = take(train_ids), take(eval_ids)
-        if head == "knn":
-            def score(a, ya, q, yq):
-                return heads.knn_classify(a, ya, q, yq, k=int(k), num_classes=C, status=status)[1]
-        else:
-            def score(a, ya, q, yq):
-                with torch.random.fork_rng(devices=[]):
-                    torch.manual_seed(int(seed))
-                    clf = heads.Mlp1Classifier(a.size(1), dev, num_classes=C)
-                for _ in range(int(mlp_epochs)):
-                    clf.fit(a, ya)
-                return clf.score(q, yq, status=status)
-        tot = gather_score_reduce(train_emb, train_y, eval_emb, eval_y, score, self.group)
-        host = torch.cat([tot, status.to(torch.int64)]).cpu()            # the one read: totals and the status word
-        tnn.check_fused_status({status.device.index: int(host[2])})
-        return float(host[0]) / max(float(host[1]), 1.0)
+        return _stage2_accuracy(corpus, status, train_emb, eval_emb, train_ids, eval_ids, head, k, mlp_epochs, seed, C,
+                                self.group)
 
 
 class ClassifierTrainer:
@@ -629,3 +644,153 @@ class ClassifierTrainer:
             acc = red.cpu().numpy()
         n = max(acc[2], 1.0)
         return float(acc[0] / n), float(acc[1] / n)
+
+
+class DenseTripletTrainer:
+    """2stg stage-1 training and scoring of the dense encoders of Code/sage+gat+diffpool against an HBM-resident corpus
+    (tsg.feeder.DeviceCorpus): tsg.dense.PackedGcnEncoder ("base" / GraphSAGE), tsg.gat.PackedGatEncoder and
+    tsg.diffpool.PackedSoftPoolEncoder.  Every batch is assembled on the GPU by DeviceCorpus.pack_dense: node features are
+    the rows of `table` ([>= max_nodes, F], the shared N(0, 2^2) table indexed by node position,
+    train_triplet.py:379-385), the adjacency is the RAW 0/1 CSR.  The embedding is element [1] of the model's output, the
+    one the triplet loss sees (tripletnet.py:36-38).
+
+    The step is the reference's dense stage-1 setting: MarginRankingLoss(margin) on the embedding distances, Adam(lr)
+    (train_triplet.py:216) and clip_grad_norm(clip_norm) (:286); clip_norm=None skips the clip.  Documented deviation:
+    the reference's dense triplet loss also adds L1 / L2 norms of the embeddings (SURVEY section 3b); their coefficients
+    are not recorded, so this trainer leaves those terms out rather than guess them.
+
+    `max_nodes` is the reference's padding size: a graph with fewer nodes has zero-padded rows (has_pad, or GAT's
+    max_nodes argument), one with more is refused.  A DiffPool model's `max_num_nodes` must equal it."""
+
+    def __init__(self, model: torch.nn.Module, table: torch.Tensor, max_nodes: int = 1000, lr: float = 1e-3,
+                 margin: float = 1.5, clip_norm: Optional[float] = 2.0, group=None):
+        from . import dense, diffpool, gat
+        if isinstance(model, gat.PackedGatEncoder):
+            self.kind, in_dim = "gat", model.conv_first.heads()[0].input_dim
+        elif isinstance(model, diffpool.PackedSoftPoolEncoder):
+            self.kind, in_dim = "diffpool", model.conv_first.input_dim
+            if int(model.max_num_nodes) != int(max_nodes):
+                raise ValueError(f"tsg: the DiffPool model was built for max_num_nodes = {model.max_num_nodes}, the trainer "
+                                 f"pads to max_nodes = {max_nodes}")
+        elif isinstance(model, dense.PackedGcnEncoder):
+            self.kind, in_dim = "base", model.conv_first.input_dim
+        else:
+            raise TypeError("tsg: DenseTripletTrainer takes a PackedGcnEncoder, PackedGatEncoder or PackedSoftPoolEncoder")
+        if int(max_nodes) < 1:
+            raise ValueError("tsg: max_nodes must be at least 1")
+        if table.dim() != 2 or table.size(0) < int(max_nodes):
+            raise ValueError(f"tsg: the feature table must be [max_nodes = {max_nodes}, F], not {tuple(table.shape)}")
+        if table.size(1) != in_dim:
+            raise ValueError(f"tsg: the feature table has {table.size(1)} columns, the model takes {in_dim}")
+        params = list(model.parameters())
+        dev = params[0].device if params else table.device
+        self.model, self.margin, self.group = model, margin, group
+        self.max_nodes, self.clip_norm = int(max_nodes), clip_norm
+        self.table = table.to(device=dev, dtype=torch.float32).contiguous()
+        self.want_eid = self.kind == "gat"                 # GAT's backward walks both orientations by edge id
+        self.opt = torch.optim.Adam(params, lr=lr)          # train_triplet.py:216
+
+    def _forward(self, batch):
+        if self.kind == "gat":
+            return self.model(batch.x, batch.csr, batch.graph_ptr, batch.max_nodes)
+        return self.model(batch.x, batch.csr, batch.graph_ptr, batch.has_pad)
+
+    def _readout(self, batch):
+        """The model's forward up to its graph readout (the input of the head that makes element [1])."""
+        if self.kind == "gat":
+            return self.model.readout(batch.x, batch.csr, batch.graph_ptr, batch.max_nodes)
+        return self.model.readout(batch.x, batch.csr, batch.graph_ptr, batch.has_pad)
+
+    def _head(self, r):
+        """Element [1] of the model's forward from its readout `r` (encoders.py:207-217, encoders_GAT.py:191-198)."""
+        m = self.model
+        if self.kind == "gat":
+            return (m.pred_model if m.final_dim != "output_dim" else m.map_model)(r)
+        if m.final_dim not in ("pretrain", "output_dim"):
+            return m.pred_model(m.pre_pred_model(r))
+        return m.map_model(r)
+
+    def pack(self, corpus, ids_host):
+        """ids -> tsg.feeder.DenseBatch for this trainer's model (eids for GAT), assembled on the GPU."""
+        return corpus.pack_dense(ids_host, self.table, self.max_nodes, want_eid=self.want_eid)
+
+    def step(self, batch, triplets: torch.Tensor) -> torch.Tensor:
+        """One stage-1 step on a DenseBatch: embeddings, the triplet loss over `triplets` [T, 3] (rows of this batch),
+        backward, the optional clip, Adam.  With world > 1 one all-reduce of [T_r * grads, T_r * loss, T_r] makes the loss
+        and gradient those of the global batch (triplets are rank-local); the clip then applies to that gradient."""
+        self.model.train()
+        emb = self._forward(batch)[1]
+        loss, _, _ = ops.triplet_loss(emb, triplets, self.margin)
+        self.opt.zero_grad(set_to_none=True)
+        loss.backward()
+        params = list(self.model.parameters())
+        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
+        if world > 1:
+            loss = all_reduce_grads_and_loss(params, loss, int(triplets.size(0)), self.group)
+        if self.clip_norm is not None:
+            torch.nn.utils.clip_grad_norm_(params, self.clip_norm)
+        self.opt.step()
+        return loss.detach()
+
+    def run_from_ids(self, corpus, id_batches) -> list:
+        """Training loop against an HBM-resident corpus, with TripletTrainer.run_from_ids's contract: per step the host
+        provides (graph_ids int64 numpy [B], triplets int64 pinned tensor [T, 3] into graph_ids).  Inside the loop the ids
+        and offsets go up in one small staged upload, pack_dense assembles the batch in one launch, the step runs and its
+        loss is read back into pinned memory without stalling the enqueue thread.  The status word is checked once, at
+        the end.  Returns the per-step losses."""
+        dev = corpus.device
+        host_losses = []
+        for ids_host, trip_host in id_batches:
+            ids = corpus.check_dense(ids_host, self.table, self.max_nodes)
+            batch = corpus.pack_dense_staged(*corpus._stage(ids), self.table, self.max_nodes, self.want_eid)
+            loss = self.step(batch, trip_host.to(dev, non_blocking=True))
+            h = torch.empty((), dtype=torch.float32, pin_memory=True)
+            h.copy_(loss, non_blocking=True)
+            host_losses.append(h)
+        torch.cuda.current_stream(dev).synchronize()
+        _check_status()
+        return [float(h) for h in host_losses]
+
+    def _embed(self, corpus, ids: np.ndarray, batch_graphs: int) -> torch.Tensor:
+        model = self.model
+        was_training = model.training
+        model.eval()
+        parts = []
+        try:
+            with torch.no_grad():
+                for s in range(0, ids.shape[0], batch_graphs):
+                    parts.append(self._readout(self.pack(corpus, ids[s:s + batch_graphs])))
+                # the head runs ONCE over all rows: the ATen GEMM picks its algorithm by row count, so one call per
+                # packed batch would make a row's last bits depend on batch_graphs
+                return self._head(parts[0] if len(parts) == 1 else torch.cat(parts))
+        finally:
+            model.train(was_training)
+
+    def embed(self, corpus, ids, batch_graphs: int = 4096) -> torch.Tensor:
+        """Embeddings [len(ids), D] on the device, row i = graph ids[i] (duplicates allowed): the model in eval mode under
+        torch.no_grad(): readouts in packed batches of `batch_graphs`, then the model's head over all of them in one call, so
+        the result does not depend on `batch_graphs`; the caller's training flag is restored.  The status word is checked
+        once, at the end."""
+        if batch_graphs < 1:
+            raise ValueError("tsg: batch_graphs must be at least 1")
+        ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+        corpus.check_dense(ids, self.table, self.max_nodes)
+        out = self._embed(corpus, ids, int(batch_graphs))
+        _check_status()
+        return out
+
+    def evaluate(self, corpus, train_ids, eval_ids, head: str = "knn", k: int = 3, mlp_epochs: int = 1, seed: int = 0,
+                 num_classes: Optional[int] = None, batch_graphs: int = 4096) -> float:
+        """The 2stg accuracy of the encoder (Code/sage+gat+diffpool/train_triplet.py:80-85 kNN, evaluate_mlp's MLP):
+        TripletTrainer.evaluate's contract, validation and scoring (K12 heads, the MLP's initial weights drawn from `seed`
+        under fork_rng, gather_score_reduce under a process group, one device-to-host read) on this trainer's
+        embeddings."""
+        from . import nn as tnn
+        train_ids, eval_ids, C = _stage2_args(corpus, train_ids, eval_ids, head, k, mlp_epochs, num_classes, batch_graphs)
+        corpus.check_dense(train_ids, self.table, self.max_nodes)
+        corpus.check_dense(eval_ids, self.table, self.max_nodes)
+        status = tnn._status_word(corpus.device)
+        train_emb = self._embed(corpus, train_ids, int(batch_graphs))
+        eval_emb = self._embed(corpus, eval_ids, int(batch_graphs))
+        return _stage2_accuracy(corpus, status, train_emb, eval_emb, train_ids, eval_ids, head, k, mlp_epochs, seed, C,
+                                self.group)

@@ -92,6 +92,42 @@ int tsg_pack_dense_batch(const int64_t* ids, const int64_t* out_node_ptr, const 
                          const float* table, int64_t max_nodes, int64_t feat, float* x_out, uint8_t* has_pad,
                          int32_t* rowptr /*nullable*/, int32_t* colidx, float* val, int32_t* eid /*nullable*/,
                          int32_t* t_eid /*nullable*/, int32_t* status, void* stream);
+/* K0e: an EigenGCN batch (WavePoolingGcnEncoder + Pool, Code/eigengcn) in ONE launch, from the corpus (coalesced,
+ * symmetric graph-local lists as for K0d; int32 node labels, F classes) and its resident EigenPooling operands:
+ * cluster_of [sum n] graph-local cluster ids, pool_w [J, pool_stride] (P_j[node, cluster_of[node]]), c_cluster_ptr /
+ * c_coarse_ptr [G+1], coarse_row / coarse_col graph-local cluster ids with coarse_w (the coarsened adjacency, coalesced
+ * and symmetric in position and weight, no self loops), final_w [Jf, final_stride] (one weight per cluster).
+ *   replaces: the reference's per-graph spectral pooling operands padded to max_nodes and marshaled per graph
+ *   (Code/eigengcn/tripletnet.py:19-56, coarsen_pooling_with_last_eigen_padding.py:121-182), and bench.Config5's
+ *   K0 + K1 + gathers + repeat_interleave + build_rect_csr + K11 (tsg_eigpool_build is not needed: pool_w is resident).
+ *   Writes for graph b = ids[b] at the packed offsets out_*_ptr (nodes, edges, clusters, coarse entries):
+ *   x_out [N, F] one-hot; has_pad [3, B] = (n_b < max_nodes, nc_b < max_nodes, 1 < max_nodes); when rowptr is given the
+ *   RAW 0/1 adjacency CSR (rowptr [N+1], colidx / val [E], one orientation = its own transpose; NULL: built elsewhere);
+ *   P_j^T: member_ptr [NC+1] / member [N] (cluster rows, members in ascending node order) / pool_val [J, N] and its
+ *   transpose node_iota [N+1] (= arange) / node_cluster [N] (batch-global cluster) / pool_val_nodes [J, N];
+ *   the coarsened adjacency coarse_rowptr [NC+1] / coarse_colidx / coarse_val [EC] (RAW, its own transpose);
+ *   when Jf > 0 the final pooling final_rowptr [B+1] / cluster_iota [NC+1] (its [:NC] = colidx, all of it = the
+ *   transposed rowptr) / cluster_graph [NC] / final_val [Jf, NC]; graph_iota [B+1] int64 = arange (the final level's
+ *   row offsets).  Violations OR into *status: TSG_FUSED_* 1 / 2 / 4 for the adjacency as in K0d, 16 for the operands
+ *   (cluster id outside [0, nc_b), nc_b > max_nodes, no cluster for a graph with nodes, a coarse list out of range,
+ *   unsorted, with a self loop or asymmetric); indices stay in range either way.  TSG_EINVAL: sizes of 2^31 or more,
+ *   null pointers (an array with nothing to read or write may be NULL: node arrays when N = 0, coarse-entry arrays
+ *   when EC = 0, adjacency arrays when E = 0), J = 0, N > 0 with NC = 0, or max_nodes above the shared-memory budget
+ *   (3 max_nodes + 2 ints per CTA: 19,370 nodes). */
+int tsg_pack_eigen_batch(const int64_t* ids, const int64_t* out_node_ptr, const int64_t* out_edge_ptr,
+                         const int64_t* out_cluster_ptr, const int64_t* out_coarse_ptr, int64_t batch_graphs,
+                         int64_t num_nodes, int64_t num_edges, int64_t num_clusters, int64_t num_coarse,
+                         const int64_t* corpus_node_ptr, const int64_t* corpus_edge_ptr, const int32_t* corpus_label,
+                         const int32_t* corpus_row, const int32_t* corpus_col, int64_t feat,
+                         const int64_t* corpus_cluster_ptr, const int64_t* corpus_coarse_ptr, const int32_t* cluster_of,
+                         const float* pool_w, int64_t pool_stride, int64_t num_pool, const int32_t* coarse_row,
+                         const int32_t* coarse_col, const float* coarse_w, const float* final_w /*nullable if Jf = 0*/,
+                         int64_t final_stride, int64_t num_final, int64_t max_nodes, float* x_out, uint8_t* has_pad,
+                         int32_t* rowptr /*nullable*/, int32_t* colidx, float* val, int32_t* member_ptr,
+                         int32_t* member, float* pool_val, int32_t* node_iota, int32_t* node_cluster,
+                         float* pool_val_nodes, int32_t* coarse_rowptr, int32_t* coarse_colidx, float* coarse_val,
+                         int32_t* final_rowptr, int32_t* cluster_iota, int32_t* cluster_graph, float* final_val,
+                         int64_t* graph_iota, int32_t* status, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * K1  CSR construction + GCN normalisation

@@ -18,8 +18,7 @@
 // Replaces bench.py's host path for these configs (synth.select + synth.pack on the CPU, an int64 edge_index H2D copy,
 // K1 tsg_csr_build(CSR_RAW): three passes with global atomics) and the reference's per-graph padded numpy tensors
 // (Code/sage+gat+diffpool/tripletnet.py:18-33).
-#include "common.cuh"
-#include "sag_fused.cuh"
+#include "pack_csr.cuh"
 
 namespace tsg {
 
@@ -63,19 +62,7 @@ k_pack_dense(const int64_t* __restrict__ ids, const int64_t* __restrict__ out_no
     if (tid == 0) s_bad = n > nmax ? TSG_FUSED_BAD_EDGE : 0;
     __syncthreads();
     int bad = 0;
-    if (n <= nmax) {
-      for (int p = tid; p <= e; p += PDENSE_THREADS) {
-        const int r = p < e ? lrow[ce + p] : n;
-        const int r0 = p > 0 ? lrow[ce + p - 1] : -1;
-        if (p < e) {
-          const int q = lcol[ce + p];
-          if ((unsigned)r >= (unsigned)n || (unsigned)q >= (unsigned)n || r == q) { bad |= TSG_FUSED_BAD_EDGE; continue; }
-          if (p > 0 && !(r0 < r || (r0 == r && lcol[ce + p - 1] < q))) { bad |= TSG_FUSED_UNSORTED; continue; }
-        }
-        if (r0 != -1 && (unsigned)r0 >= (unsigned)n) continue;
-        for (int rr = r0 + 1; rr <= r; ++rr) rs[rr] = p;      // rows r0+1 .. r start here (empty rows included)
-      }
-    }
+    if (n <= nmax) bad = coalesced_row_starts(lrow + ce, lcol + ce, n, e, rs, tid, PDENSE_THREADS);
     if (bad) atomicOr(&s_bad, bad);
     __syncthreads();
     const int sb = s_bad;
@@ -103,13 +90,7 @@ k_pack_dense(const int64_t* __restrict__ ids, const int64_t* __restrict__ out_no
       val[o] = 1.0f;
       if (t_eid) t_eid[o] = (int32_t)o;                        // src-major: slot o holds edge o itself
       // dst-major: slot o is row r's entry q, i.e. the edge (q -> r); its position is r's place in row q
-      int lo = rs[q], hi = rs[q + 1], at = -1;
-      while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        const int v = lcol[ce + mid];
-        if (v == r) { at = mid; break; }
-        if (v < r) lo = mid + 1; else hi = mid;
-      }
+      int at = coalesced_find(lcol + ce, rs, q, r);
       if (at < 0) { bad |= TSG_FUSED_ASYMMETRIC; at = p; }
       if (eid) eid[o] = (int32_t)(ob + at);
     }

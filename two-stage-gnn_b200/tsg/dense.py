@@ -278,22 +278,34 @@ class PackedWaveEncoder(nn.Module):
         width = D * (len(self.pool_sizes) + 1) + (D * num_pool_final_matrix if num_pool_final_matrix > 0 else 0)
         self.pred_model = _pred_layers(width, pred_hidden_dims, label_dim)      # eigengcn/encoders.py:294-296
 
-    def forward(self, x, csr_adj: CSR, graph_ptr, pool_csrs: List[List[CSR]], csr_pooled: List[CSR],
-                pooled_ptrs: List[torch.Tensor], final_ptr: Optional[torch.Tensor] = None):
-        """x packed [sum n, F]; pool_csrs[i] = the P_j^T CSRs of level i (level len(pool_sizes) = final);
-        csr_pooled[i] / pooled_ptrs[i] = coarsened adjacency / cluster offsets of level i.  Every graph
-        is assumed to have n < N (padded rows exist), as in the reference's max_nodes padding."""
+    def readout(self, x, csr_adj: CSR, graph_ptr, pool_csrs: List[List[CSR]], csr_pooled: List[CSR],
+                pooled_ptrs: List[torch.Tensor], final_ptr: Optional[torch.Tensor] = None,
+                has_pad: Optional[Sequence[torch.Tensor]] = None) -> torch.Tensor:
+        """The concatenated max-readouts (`output`, eigengcn/encoders.py:323-370): the input of pred_model.
+        has_pad: per readout (level 0, every pooled level, then the final pooling if any) bool [graphs] -- whether the
+        reference's max_nodes padding leaves a zero row there, so its max is taken against 0.  None: every graph is
+        padded at every level (n < max_nodes, as bench config 5 assumes)."""
         outs = []
+        ones = torch.ones(graph_ptr.numel() - 1, dtype=torch.bool, device=x.device) if has_pad is None else None
+        pad = (lambda k: ones) if has_pad is None else (lambda k: has_pad[k])
         convs = [self.conv_first] + list(self.conv_block) + [self.conv_last]
         z = gcn_forward(x, csr_adj, convs, self.bn)
-        ones = torch.ones(graph_ptr.numel() - 1, dtype=torch.bool, device=x.device)
-        outs.append(_readout_max(z, graph_ptr, 0.0, ones))
+        outs.append(_readout_max(z, graph_ptr, 0.0, pad(0)))
         for i in range(len(self.pool_sizes)):
             z = eigen_pool(z, pool_csrs[i][:self.num_pool_matrix])
             convs = [self.conv_first_after_pool[i]] + list(self.conv_block_after_pool[i]) + [self.conv_last_after_pool[i]]
             z = gcn_forward(z, csr_pooled[i], convs, self.bn)
-            outs.append(_readout_max(z, pooled_ptrs[i], 0.0, ones))
+            outs.append(_readout_max(z, pooled_ptrs[i], 0.0, pad(i + 1)))
         if self.num_pool_final_matrix > 0:
             z = eigen_pool(z, pool_csrs[len(self.pool_sizes)][:self.num_pool_final_matrix])
-            outs.append(_readout_max(z, final_ptr, 0.0, ones))
-        return self.pred_model(torch.cat(outs, dim=1))
+            outs.append(_readout_max(z, final_ptr, 0.0, pad(len(self.pool_sizes) + 1)))
+        return torch.cat(outs, dim=1)
+
+    def forward(self, x, csr_adj: CSR, graph_ptr, pool_csrs: List[List[CSR]], csr_pooled: List[CSR],
+                pooled_ptrs: List[torch.Tensor], final_ptr: Optional[torch.Tensor] = None,
+                has_pad: Optional[Sequence[torch.Tensor]] = None):
+        """x packed [sum n, F]; pool_csrs[i] = the P_j^T CSRs of level i (level len(pool_sizes) = final);
+        csr_pooled[i] / pooled_ptrs[i] = coarsened adjacency / cluster offsets of level i; has_pad: see readout (None =
+        every graph has n < N, padded rows exist, as in the reference's max_nodes padding)."""
+        return self.pred_model(self.readout(x, csr_adj, graph_ptr, pool_csrs, csr_pooled, pooled_ptrs, final_ptr,
+                                            has_pad))

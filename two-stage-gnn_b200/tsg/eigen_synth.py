@@ -58,11 +58,39 @@ def _eigvecs(adj: np.ndarray, num: int) -> np.ndarray:
     return out
 
 
-def make_operands(c: Corpus, pool_size: int = 10, num_pool_matrix: int = 1, num_pool_final_matrix: int = 1
-                  ) -> EigenOperands:
+def bfs_clusters(c: Corpus, pool_size: int = 10):
+    """The synthetic clustering: contiguous chunks of `pool_size` nodes in BFS order from node 0.  Returns
+    (cluster_of int64 [sum n], order int64 [sum n]): graph-local cluster ids and every graph's BFS node order."""
+    cluster_of = np.zeros(int(c.node_ptr[-1]), np.int64)
+    order_all = np.zeros(int(c.node_ptr[-1]), np.int64)
+    for g in range(c.num_graphs):
+        n0, n1 = int(c.node_ptr[g]), int(c.node_ptr[g + 1])
+        e0, e1 = int(c.edge_ptr[g]), int(c.edge_ptr[g + 1])
+        n = n1 - n0
+        order = _bfs_order(n, c.row[e0:e1], c.col[e0:e1])
+        pos = np.empty(n, np.int64); pos[order] = np.arange(n)
+        cluster_of[n0:n1] = pos // pool_size
+        order_all[n0:n1] = order
+    return cluster_of, order_all
+
+
+def operands_from_clusters(c: Corpus, cluster_of, num_pool_matrix: int = 1, num_pool_final_matrix: int = 1,
+                           member_order=None) -> EigenOperands:
+    """EigenPooling operands of a corpus for a given clustering (e.g. the reference's SpectralClustering labels,
+    coarsen_pooling_with_last_eigen_padding.py:36-60): `cluster_of` [sum n] graph-local cluster ids in [0, nc_g), every
+    graph's clusters numbered from 0.  Per cluster, P_j[:, c] = the j-th eigenvector of its unnormalised Laplacian over
+    its members listed in ascending node order, or in the order of `member_order` ([sum n], a per-graph permutation of
+    the local node ids) when given; the coarsened adjacency and the final pooling follow (module docstring)."""
+    cluster_of = np.asarray(cluster_of).reshape(-1)
+    if cluster_of.shape[0] != int(c.node_ptr[-1]):
+        raise ValueError(f"tsg: cluster_of has {cluster_of.shape[0]} entries, the corpus has {int(c.node_ptr[-1])} nodes")
+    if cluster_of.size and not np.issubdtype(cluster_of.dtype, np.integer):
+        raise ValueError("tsg: cluster_of must hold integer cluster ids")
+    cluster_of = cluster_of.astype(np.int64)
+    if cluster_of.size and int(cluster_of.min()) < 0:
+        raise ValueError("tsg: cluster ids must be non-negative")
     G = c.num_graphs
     cluster_ptr = np.zeros(G + 1, np.int64)
-    cluster_of = np.zeros(int(c.node_ptr[-1]), np.int64)
     pool_w = [np.zeros(int(c.node_ptr[-1]), np.float32) for _ in range(num_pool_matrix)]
     c_rows, c_cols, c_ws, coarse_ptr = [], [], [], np.zeros(G + 1, np.int64)
     final_parts = [[] for _ in range(num_pool_final_matrix)]
@@ -71,15 +99,17 @@ def make_operands(c: Corpus, pool_size: int = 10, num_pool_matrix: int = 1, num_
         e0, e1 = int(c.edge_ptr[g]), int(c.edge_ptr[g + 1])
         n = n1 - n0
         row, col = c.row[e0:e1], c.col[e0:e1]
-        order = _bfs_order(n, row, col)
-        pos = np.empty(n, np.int64); pos[order] = np.arange(n)
-        cl = pos // pool_size
-        nc = int(cl.max()) + 1
-        cluster_of[n0:n1] = cl
+        cl = cluster_of[n0:n1]
+        nc = int(cl.max()) + 1 if n else 0
         cluster_ptr[g + 1] = cluster_ptr[g] + nc
+        order = np.arange(n, dtype=np.int64) if member_order is None else np.asarray(member_order[n0:n1], np.int64)
+        members = order[np.argsort(cl[order], kind="stable")]           # by cluster, `order` within a cluster
+        starts = np.searchsorted(cl[members], np.arange(nc + 1))
         adj = np.zeros((n, n), np.float32); adj[row, col] = 1.0
         for k in range(nc):
-            nodes = order[k * pool_size:(k + 1) * pool_size]
+            nodes = members[starts[k]:starts[k + 1]]
+            if nodes.size == 0:
+                continue
             ev = _eigvecs(adj[np.ix_(nodes, nodes)], num_pool_matrix)
             for j in range(num_pool_matrix):
                 pool_w[j][n0 + nodes] = ev[:, j].astype(np.float32)
@@ -89,13 +119,20 @@ def make_operands(c: Corpus, pool_size: int = 10, num_pool_matrix: int = 1, num_
         rr, cc = np.nonzero(coarse)
         c_rows.append(rr.astype(np.int64)); c_cols.append(cc.astype(np.int64)); c_ws.append(coarse[rr, cc].astype(np.float32))
         coarse_ptr[g + 1] = coarse_ptr[g] + rr.shape[0]
-        if num_pool_final_matrix > 0:
+        if num_pool_final_matrix > 0 and nc > 0:
             ev = _eigvecs((coarse > 0).astype(np.float32), num_pool_final_matrix)
             for j in range(num_pool_final_matrix):
                 final_parts[j].append(ev[:, j].astype(np.float32))
     cat = lambda parts, dt: np.concatenate(parts).astype(dt) if parts else np.zeros(0, dt)
-    return EigenOperands(cluster_ptr, cluster_of, pool_w, coarse_ptr, cat(c_rows, np.int64), cat(c_cols, np.int64),
-                         cat(c_ws, np.float32), [cat(p, np.float32) for p in final_parts])
+    return EigenOperands(cluster_ptr, cluster_of.copy(), pool_w, coarse_ptr, cat(c_rows, np.int64),
+                         cat(c_cols, np.int64), cat(c_ws, np.float32), [cat(p, np.float32) for p in final_parts])
+
+
+def make_operands(c: Corpus, pool_size: int = 10, num_pool_matrix: int = 1, num_pool_final_matrix: int = 1
+                  ) -> EigenOperands:
+    """Synthetic operands: bfs_clusters, members listed in BFS order (operands_from_clusters)."""
+    cluster_of, order = bfs_clusters(c, pool_size)
+    return operands_from_clusters(c, cluster_of, num_pool_matrix, num_pool_final_matrix, member_order=order)
 
 
 def pack_operands(c: Corpus, op: EigenOperands, graph_ids) -> dict:

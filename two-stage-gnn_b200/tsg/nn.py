@@ -139,10 +139,11 @@ def sag_arena_view(shape, arena: torch.Tensor, level: int, field: str) -> torch.
 
 
 LABEL_RANGE = 8           # TSG_SAG_LABEL_RANGE (include/tsg.h)
+EIGEN_OPERANDS = 16       # K0e tsg_pack_eigen_batch: the EigenPooling operands of a graph are not what it relies on
 
 
 def check_fused_status(already_read: Optional[dict] = None) -> None:
-    """Look at the status word the verifying kernels (K1d, K13, and the label checks of the supervised step, the
+    """Look at the status word the verifying kernels (K1d, K13, K0d / K0e, and the label checks of the supervised step, the
     classification forward and the stage-2 heads) OR-ed their bits into since the last call -- ONE device
     read per device, so callers do it where they synchronise anyway (loss read-back, end of a feeder loop, tests).  A non-zero word means a graph's
     edge list was not what those kernels require (endpoints in range, no self loops, sorted by (row, col), symmetric:
@@ -159,6 +160,12 @@ def check_fused_status(already_read: Optional[dict] = None) -> None:
         raise RuntimeError("tsg: a graph label lies outside [0, num_classes) (status bit 8, set by the supervised step, "
                            "the classification forward or a stage-2 head); it was clamped, so the loss and the accuracy "
                            "are invalid")
+    if bits & EIGEN_OPERANDS:
+        raise RuntimeError("tsg: a graph's EigenPooling operands are invalid (status bit 16, set by pack_eigen): a cluster "
+                           "id outside [0, clusters of the graph), more clusters than max_nodes, or a coarsened "
+                           "adjacency list that is out of range, unsorted, has a self loop or is not symmetric in "
+                           "position and weight" + (f"; adjacency bits {bits & 7} are set too" if bits & 7 else "") +
+                           ".  Build them with tsg.eigen_synth.operands_from_clusters.")
     if bits:
         names = [n for b, n in ((1, "edge endpoint out of range / self loop"), (2, "edge list not sorted by (row, col)"),
                                 (4, "edge list not symmetric")) if bits & b]

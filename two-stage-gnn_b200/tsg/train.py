@@ -714,12 +714,24 @@ class DenseTripletTrainer:
         """ids -> tsg.feeder.DenseBatch for this trainer's model (eids for GAT), assembled on the GPU."""
         return corpus.pack_dense(ids_host, self.table, self.max_nodes, want_eid=self.want_eid)
 
+    def _check(self, corpus, ids_host) -> np.ndarray:
+        """The host-side checks of a pack (no device work): -> the ids as int64 numpy."""
+        return corpus.check_dense(ids_host, self.table, self.max_nodes)
+
+    def _pack_checked(self, corpus, ids: np.ndarray):
+        """`pack` for ids that passed `_check`: one staged upload, one launch."""
+        return corpus.pack_dense_staged(*corpus._stage(ids), self.table, self.max_nodes, self.want_eid)
+
+    def _embedding(self, batch) -> torch.Tensor:
+        """The embedding the triplet loss sees (element [1] of the model's output)."""
+        return self._forward(batch)[1]
+
     def step(self, batch, triplets: torch.Tensor) -> torch.Tensor:
         """One stage-1 step on a DenseBatch: embeddings, the triplet loss over `triplets` [T, 3] (rows of this batch),
         backward, the optional clip, Adam.  With world > 1 one all-reduce of [T_r * grads, T_r * loss, T_r] makes the loss
         and gradient those of the global batch (triplets are rank-local); the clip then applies to that gradient."""
         self.model.train()
-        emb = self._forward(batch)[1]
+        emb = self._embedding(batch)
         loss, _, _ = ops.triplet_loss(emb, triplets, self.margin)
         self.opt.zero_grad(set_to_none=True)
         loss.backward()
@@ -741,8 +753,7 @@ class DenseTripletTrainer:
         dev = corpus.device
         host_losses = []
         for ids_host, trip_host in id_batches:
-            ids = corpus.check_dense(ids_host, self.table, self.max_nodes)
-            batch = corpus.pack_dense_staged(*corpus._stage(ids), self.table, self.max_nodes, self.want_eid)
+            batch = self._pack_checked(corpus, self._check(corpus, ids_host))
             loss = self.step(batch, trip_host.to(dev, non_blocking=True))
             h = torch.empty((), dtype=torch.float32, pin_memory=True)
             h.copy_(loss, non_blocking=True)
@@ -773,8 +784,7 @@ class DenseTripletTrainer:
         once, at the end."""
         if batch_graphs < 1:
             raise ValueError("tsg: batch_graphs must be at least 1")
-        ids = np.asarray(ids, dtype=np.int64).reshape(-1)
-        corpus.check_dense(ids, self.table, self.max_nodes)
+        ids = self._check(corpus, ids)
         out = self._embed(corpus, ids, int(batch_graphs))
         _check_status()
         return out
@@ -787,10 +797,67 @@ class DenseTripletTrainer:
         embeddings."""
         from . import nn as tnn
         train_ids, eval_ids, C = _stage2_args(corpus, train_ids, eval_ids, head, k, mlp_epochs, num_classes, batch_graphs)
-        corpus.check_dense(train_ids, self.table, self.max_nodes)
-        corpus.check_dense(eval_ids, self.table, self.max_nodes)
+        self._check(corpus, train_ids)
+        self._check(corpus, eval_ids)
         status = tnn._status_word(corpus.device)
         train_emb = self._embed(corpus, train_ids, int(batch_graphs))
         eval_emb = self._embed(corpus, eval_ids, int(batch_graphs))
         return _stage2_accuracy(corpus, status, train_emb, eval_emb, train_ids, eval_ids, head, k, mlp_epochs, seed, C,
                                 self.group)
+
+
+class WaveTripletTrainer(DenseTripletTrainer):
+    """2stg stage-1 training and scoring of the EigenGCN encoder (tsg.dense.PackedWaveEncoder = Code/eigengcn's
+    WavePoolingGcnEncoder with one pooling level) against an HBM-resident corpus whose EigenPooling operands are
+    attached (DeviceCorpus.attach_eigen).  Every batch is assembled on the GPU by DeviceCorpus.pack_eigen in one launch:
+    one-hot node labels, the RAW adjacency, P_j^T, the coarsened adjacency and the final pooling, with the per-level
+    padded-row flags of `max_nodes`.  The embedding is the model's output, the one bench config 5 feeds the triplet
+    loss; DenseTripletTrainer's step / run_from_ids / embed / evaluate contract applies (embed: readouts in packed
+    batches, pred_model once over all rows).  Defaults: Adam 1e-3, margin 1.5, no clip (bench config 5's step).
+    Refused on the host: a model with more than one pooling level (the operands describe one), operands with fewer
+    pooling matrices than the model uses, and a corpus whose node-label count differs from the model's input_dim."""
+
+    def __init__(self, model: torch.nn.Module, max_nodes: int = 1000, lr: float = 1e-3, margin: float = 1.5,
+                 clip_norm: Optional[float] = None, group=None):
+        from . import dense
+        if not isinstance(model, dense.PackedWaveEncoder):
+            raise TypeError("tsg: WaveTripletTrainer takes a PackedWaveEncoder")
+        if len(model.pool_sizes) != 1:
+            raise ValueError(f"tsg: the model has {len(model.pool_sizes)} pooling levels; the EigenPooling operands "
+                             "describe one")
+        if int(max_nodes) < 1:
+            raise ValueError("tsg: max_nodes must be at least 1")
+        self.kind, self.table, self.want_eid = "wave", None, False
+        self.model, self.margin, self.group = model, margin, group
+        self.max_nodes, self.clip_norm = int(max_nodes), clip_norm
+        self.opt = torch.optim.Adam(list(model.parameters()), lr=lr)
+
+    def _check(self, corpus, ids_host) -> np.ndarray:
+        m = self.model
+        if corpus.feat != m.conv_first.input_dim:
+            raise ValueError(f"tsg: the corpus has {corpus.feat} node labels, the model takes input_dim = "
+                             f"{m.conv_first.input_dim}")
+        ids, _, _ = corpus.check_eigen(ids_host, self.max_nodes, m.num_pool_matrix, m.num_pool_final_matrix)
+        return ids
+
+    def _pack_checked(self, corpus, ids: np.ndarray):
+        return corpus.pack_eigen_checked(ids, self.max_nodes, self.model.num_pool_matrix,
+                                         self.model.num_pool_final_matrix)
+
+    def pack(self, corpus, ids_host):
+        """ids -> tsg.feeder.EigenBatch for this trainer's model, assembled on the GPU."""
+        return self._pack_checked(corpus, self._check(corpus, ids_host))
+
+    def _forward(self, batch):
+        args, kw = batch.readout_args()
+        return self.model(*args, **kw)
+
+    def _embedding(self, batch) -> torch.Tensor:
+        return self._forward(batch)
+
+    def _readout(self, batch):
+        args, kw = batch.readout_args()
+        return self.model.readout(*args, **kw)
+
+    def _head(self, r):
+        return self.model.pred_model(r)

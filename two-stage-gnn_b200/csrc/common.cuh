@@ -5,6 +5,7 @@
 #include <stdio.h>
 #include <stdarg.h>
 #include <stdlib.h>
+#include <utility>
 #include "../../include/tsg.h"
 
 #ifndef TSG_NUM_SMS
@@ -35,6 +36,41 @@ inline int check_launch(const char* what) {
 #define TSG_LAUNCH_CHECK(what)                       \
   do {                                               \
     int _rc = ::tsg::check_launch(what);             \
+    if (_rc != TSG_OK) return _rc;                   \
+  } while (0)
+
+// ------------------------------------------------------------------------------------------
+// Programmatic dependent launch (PDL).  A kernel launched by launch_pdl may be scheduled while its predecessor in
+// the stream is still draining, so the launch, the drain and the ramp-up of consecutive kernels overlap.  The rule
+// that keeps this as safe as plain stream order: every CTA of such a kernel calls pdl_wait() unconditionally, before
+// its first global load or store and before any early return, then pdl_launch_dependents().  pdl_wait() returns once
+// the predecessor grid has completed and its memory is visible; since every kernel of the chain waits, completion is
+// transitive and kernel i + 2 also sees kernel i's writes.  Launched with <<<>>> (other paths, graph capture), the
+// two instructions do nothing.  Memsets, copies and library kernels between two launches stay ordinary stream order.
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+template <typename... KArgs, typename... Args>
+static inline int launch_pdl(const char* what, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
+                             cudaStream_t st, Args&&... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+  if (e != cudaSuccess) {
+    set_error("%s: %s", what, cudaGetErrorString(e));
+    return TSG_ELAUNCH;
+  }
+  return TSG_OK;
+}
+
+#define TSG_LAUNCH_PDL(...)                          \
+  do {                                               \
+    int _rc = ::tsg::launch_pdl(__VA_ARGS__);        \
     if (_rc != TSG_OK) return _rc;                   \
   } while (0)
 
@@ -107,6 +143,8 @@ constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
 
 template <typename F>
 __global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_reduce(F f, int64_t n, int* tile_sum) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ int sm[33];
   int64_t base = (int64_t)blockIdx.x * SCAN_TILE;
   int s = 0;
@@ -122,6 +160,8 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_reduce(F f, int64_t 
 
 template <typename OutT>
 __global__ void __launch_bounds__(1024) k_scan_tile_sums(int* tile_sum, int num_tiles, OutT* out_total) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ int sm[33];
   long long carry = 0;
   for (int base = 0; base < num_tiles; base += 1024) {
@@ -137,6 +177,8 @@ __global__ void __launch_bounds__(1024) k_scan_tile_sums(int* tile_sum, int num_
 
 template <typename F, typename OutT>
 __global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_scan(F f, int64_t n, const int* tile_off, OutT* out) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ int sm[33];
   __shared__ int vals[SCAN_TILE];
   int64_t base = (int64_t)blockIdx.x * SCAN_TILE;
@@ -170,14 +212,10 @@ static inline size_t scan_ws_ints(int64_t n) { return (size_t)((n + SCAN_TILE - 
 template <typename F, typename OutT>
 int exclusive_scan(F f, int64_t n, OutT* out, int* tile_ws, cudaStream_t st) {
   int num_tiles = (int)((n + SCAN_TILE - 1) / SCAN_TILE);
-  if (num_tiles == 0) {
-    k_scan_tile_sums<OutT><<<1, 1024, 0, st>>>(tile_ws, 0, out);
-    return check_launch("scan(empty)");
-  }
-  k_scan_tile_reduce<F><<<num_tiles, SCAN_THREADS, 0, st>>>(f, n, tile_ws);
-  k_scan_tile_sums<OutT><<<1, 1024, 0, st>>>(tile_ws, num_tiles, out + n);
-  k_scan_tile_scan<F, OutT><<<num_tiles, SCAN_THREADS, 0, st>>>(f, n, tile_ws, out);
-  return check_launch("scan");
+  if (num_tiles == 0) return launch_pdl("scan(empty)", k_scan_tile_sums<OutT>, 1, 1024, 0, st, tile_ws, 0, out);
+  TSG_LAUNCH_PDL("scan(reduce)", k_scan_tile_reduce<F>, num_tiles, SCAN_THREADS, 0, st, f, n, tile_ws);
+  TSG_LAUNCH_PDL("scan(tile sums)", k_scan_tile_sums<OutT>, 1, 1024, 0, st, tile_ws, num_tiles, out + n);
+  return launch_pdl("scan", k_scan_tile_scan<F, OutT>, num_tiles, SCAN_THREADS, 0, st, f, n, (const int*)tile_ws, out);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -188,6 +226,8 @@ int exclusive_scan(F f, int64_t n, OutT* out, int* tile_ws, cudaStream_t st) {
 static __global__ void __launch_bounds__(1024)
 k_partial_sum_final(const float* __restrict__ part, float* __restrict__ out0, int n0,
                     float* __restrict__ out1, int nb, int total) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ float sm[32][33];
   const int x = threadIdx.x & 31, y = threadIdx.x >> 5;
   const int i = blockIdx.x * 32 + x;
@@ -266,9 +306,14 @@ static inline bool fused_tail_ok(int64_t nb, int64_t total) {
 
 unsigned* ticket_next();      // api.cu: a zeroed device counter from a per-device pool (nullptr if the pool cannot be made)
 
-static inline void launch_partial_sum_final(const float* part, float* out0, int n0, float* out1, int nb,
-                                            int total, cudaStream_t st) {
-  k_partial_sum_final<<<(total + 31) / 32, 1024, 0, st>>>(part, out0, n0, out1, nb, total);
+// k9_triplet.cu: tsg_triplet_fwd that also stores 1.0 to *dloss_seed (if given) from its last kernel
+int triplet_fwd(const float* emb, const int64_t* trip, int64_t T, int64_t M, int64_t D, float margin, float eps,
+                float* dpos, float* dneg, float* loss, float* dloss_seed, void* workspace, size_t workspace_bytes,
+                void* stream);
+
+static inline int launch_partial_sum_final(const float* part, float* out0, int n0, float* out1, int nb,
+                                           int total, cudaStream_t st) {
+  return launch_pdl("partial_sum_final", k_partial_sum_final, (total + 31) / 32, 1024, 0, st, part, out0, n0, out1, nb, total);
 }
 
 }  // namespace tsg

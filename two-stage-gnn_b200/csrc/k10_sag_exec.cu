@@ -102,6 +102,8 @@ static void layout(const tsg_sag_shape* sh, void* arena, SagArena* a) {
 
 __global__ void __launch_bounds__(256)
 k_add3(const float* __restrict__ a, const float* __restrict__ b, const float* __restrict__ c, float* __restrict__ o, int64_t n) {
+  pdl_wait();
+  pdl_launch_dependents();
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     o[i] = (a[i] + b[i]) + c[i];
 }
@@ -281,8 +283,8 @@ static int sag_fwd(const tsg_sag_shape* sh, const SagInput& in, const int64_t* l
     xin = b.xg;
   }
   const int64_t tot = G * 2 * H;
-  k_add3<<<grid_for(tot, 256, 8), 256, 0, st>>>(a.lv[0].out, a.lv[1].out, a.lv[2].out, z, tot);
-  return check_launch("sag_encoder_fwd");
+  return launch_pdl("sag_encoder_fwd", k_add3, grid_for(tot, 256, 8), 256, 0, st, (const float*)a.lv[0].out, (const float*)a.lv[1].out,
+                    (const float*)a.lv[2].out, z, tot);
 }
 
 extern "C" int tsg_sag_encoder_fwd(const tsg_sag_shape* sh, const float* x, const int64_t* row, const int64_t* col,

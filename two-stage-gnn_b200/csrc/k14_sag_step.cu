@@ -59,6 +59,8 @@ __global__ void __launch_bounds__(HEAD_THREADS)
 k_head_fwd(HeadPtrs P, const float* __restrict__ z, HeadDims d, float dropout_p, unsigned long long seed,
            const float* __restrict__ mask_in, float* __restrict__ a1, float* __restrict__ m, float* __restrict__ a2,
            float* __restrict__ emb) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float hsm[];
   float* prm = hsm;
   float* stage = hsm + head_param_floats(d.H, d.H2, d.C);          // per warp: 2H + H + H2 + C floats
@@ -155,6 +157,8 @@ __global__ void __launch_bounds__(HEAD_THREADS)
 k_head_bwd(HeadPtrs P, const float* __restrict__ z, HeadDims d, const float* __restrict__ a1, const float* __restrict__ m,
            const float* __restrict__ a2, const float* __restrict__ emb, const float* __restrict__ demb,
            float* __restrict__ dz, float* __restrict__ part) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float hsm[];
   float* prm = hsm;
   const int per = 2 * d.H + d.H + d.H + d.H2 + d.H2 + d.C;         // staged per graph: z, a1, da1, a2, da2, do
@@ -214,6 +218,8 @@ k_head_bwd(HeadPtrs P, const float* __restrict__ z, HeadDims d, const float* __r
 __global__ void __launch_bounds__(256)
 k_head_unpack(const float* __restrict__ packed, float* g0, float* g1, float* g2, float* g3, float* g4, float* g5,
               int n0, int n1, int n2, int n3, int n4, int n5) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   int o = i;
   if (o < n0) { g0[o] = packed[i]; return; }
@@ -231,6 +237,8 @@ __global__ void __launch_bounds__(HEAD_THREADS)
 k_head_delta(HeadPtrs P, HeadDims d, const float* __restrict__ a1, const float* __restrict__ m,
              const float* __restrict__ a2, const float* __restrict__ emb, const float* __restrict__ demb,
              float* __restrict__ dz, float* __restrict__ dO_out, float* __restrict__ da2_out, float* __restrict__ da1_out) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float hsm[];
   const int per = 2 * d.H + 2 * d.H2 + d.C;                       // staged per warp: a1, da1, a2, da2, do
   float* stage = hsm + head_param_floats(d.H, d.H2, d.C);
@@ -258,6 +266,8 @@ __device__ __forceinline__ int64_t clamp_label(int64_t y, int C) { return y < 0 
 // F.nll_loss(emb, y) (mean) backward as autograd builds it: demb = -(1/G) onehot(y); nll[g] = -emb[g, y_g]
 __global__ void k_nll_demb(const float* __restrict__ emb, const int64_t* __restrict__ y, int G, int C,
                            float* __restrict__ demb, float* __restrict__ nll, int* status) {
+  pdl_wait();
+  pdl_launch_dependents();
   const float grad = -(1.0f / (float)G);
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < (int64_t)G * C; i += (int64_t)gridDim.x * blockDim.x) {
     const int g = (int)(i / C), j = (int)(i % C);
@@ -293,6 +303,8 @@ __global__ void k_classify_rows(const float* __restrict__ emb, const int64_t* __
 constexpr int SUM_THREADS = 1024;
 __global__ void __launch_bounds__(SUM_THREADS)
 k_sum_fixed(const float* __restrict__ v, const int* __restrict__ hit, int n, float div, float* sum_out, int64_t* count_out) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ float sv[SUM_THREADS];
   __shared__ long long sc[SUM_THREADS];
   float s = 0.f;
@@ -312,8 +324,6 @@ k_sum_fixed(const float* __restrict__ v, const int* __restrict__ hit, int n, flo
     if (count_out) *count_out = sc[0];
   }
 }
-
-__global__ void k_store_one(float* p, float v) { *p = v; }
 
 static int head_ctas(int G) {
   // one batch of HEAD_WARPS graphs per CTA up to two CTAs per SM (ncu, first cut: 110 CTAs of 4 batches = 12 % warps
@@ -427,9 +437,8 @@ static int head_fwd(const tsg_sag_shape* sh, const tsg_sag_head* hd, const float
                     const float* dropout_mask, const float* z, float* a1, float* m, float* a2, float* emb, cudaStream_t st) {
   const int H = (int)sh->hidden, H2 = H / 2, C = (int)hd->num_classes, G = (int)sh->num_graphs;
   head_attr_once();
-  k_head_fwd<<<grid_for(G, HEAD_WARPS, 2), HEAD_THREADS, head_fwd_smem(H, H2, C), st>>>(
-      head_ptrs(params), z, HeadDims{G, H, H2, C}, dropout_p, (unsigned long long)hd->seed, dropout_mask, a1, m, a2, emb);
-  return check_launch("sag_step(head fwd)");
+  return launch_pdl("sag_step(head fwd)", k_head_fwd, grid_for(G, HEAD_WARPS, 2), HEAD_THREADS, head_fwd_smem(H, H2, C), st,
+                    head_ptrs(params), z, HeadDims{G, H, H2, C}, dropout_p, (unsigned long long)hd->seed, dropout_mask, a1, m, a2, emb);
 }
 
 // encoder forward (K10) + head forward -> emb [G, C]
@@ -450,9 +459,8 @@ static int step_bwd(const tsg_sag_shape* sh, const tsg_sag_head* hd, const int32
   const HeadPtrs P = head_ptrs(params);
   head_attr_once();
   if (head_wide(H, H2, C)) {
-    k_head_delta<<<grid_for(G, HEAD_WARPS, 1), HEAD_THREADS, head_delta_smem(H, H2, C), st>>>(
-        P, d, w.a1, w.m, w.a2, emb, demb, w.dz, w.dO, w.da2, w.da1);
-    TSG_LAUNCH_CHECK("sag_step(head delta)");
+    TSG_LAUNCH_PDL("sag_step(head delta)", k_head_delta, grid_for(G, HEAD_WARPS, 1), HEAD_THREADS, head_delta_smem(H, H2, C), st,
+                   P, d, (const float*)w.a1, (const float*)w.m, (const float*)w.a2, emb, demb, w.dz, w.dO, w.da2, w.da1);
     // nn.Linear's [out, in] gradient delta^T . input is K3's X^T . dY with X = the delta, dY = the layer's input
     const float* delta[3] = {w.da1, w.da2, w.dO};
     const float* input[3] = {w.z, w.a1, w.a2};
@@ -464,12 +472,11 @@ static int step_bwd(const tsg_sag_shape* sh, const tsg_sag_head* hd, const int32
   } else {
     const int ctas = head_ctas(G);
     const int NG = head_grad_floats(H, H2, C);
-    k_head_bwd<<<ctas, HEAD_THREADS, head_bwd_smem(H, H2, C), st>>>(P, w.z, d, w.a1, w.m, w.a2, emb, demb, w.dz, w.part);
-    TSG_LAUNCH_CHECK("sag_step(head bwd)");
-    launch_partial_sum_final(w.part, w.packed, NG, nullptr, ctas, NG, st);
-    k_head_unpack<<<(NG + 255) / 256, 256, 0, st>>>(w.packed, grads[12], grads[13], grads[14], grads[15], grads[16], grads[17],
-                                                     H * 2 * H, H, H2 * H, H2, C * H2, C);
-    TSG_LAUNCH_CHECK("sag_step(head grads)");
+    TSG_LAUNCH_PDL("sag_step(head bwd)", k_head_bwd, ctas, HEAD_THREADS, head_bwd_smem(H, H2, C), st, P, (const float*)w.z, d,
+                   (const float*)w.a1, (const float*)w.m, (const float*)w.a2, emb, demb, w.dz, w.part);
+    TSG_TRY(launch_partial_sum_final(w.part, w.packed, NG, nullptr, ctas, NG, st));
+    TSG_LAUNCH_PDL("sag_step(head grads)", k_head_unpack, (NG + 255) / 256, 256, 0, st, (const float*)w.packed, grads[12], grads[13],
+                   grads[14], grads[15], grads[16], grads[17], H * 2 * H, H, H2 * H, H2, C * H2, C);
   }
   return tsg_sag_encoder_bwd_compact(sh, label, level_ptr, params, w.dz, grads, arena, arena_bytes, stream);
 }
@@ -485,14 +492,12 @@ extern "C" int tsg_sag_triplet_step_compact(const tsg_sag_shape* sh, const tsg_s
   StepWs w;
   step_layout(sh, hd, LOSS_TRIPLET, workspace, &w);
   if (workspace_bytes < w.total) { set_error("sag_triplet_step: workspace too small (%zu < %zu)", workspace_bytes, w.total); return TSG_EWORKSPACE; }
-  cudaStream_t st = (cudaStream_t)stream;
   const int C = (int)hd->num_classes, G = (int)sh->num_graphs;
   const int64_t T = hd->num_triplets;
   float* emb = emb_out ? emb_out : w.emb;
   TSG_TRY(step_fwd(sh, hd, label, local_row, local_col, edge_ptr, level_ptr, params, dropout_mask, emb, w, arena, arena_bytes, stream));
   // triplet loss forward + backward (K9), d(loss) = 1
-  TSG_TRY(tsg_triplet_fwd(emb, triplets, T, G, C, hd->margin, hd->eps, w.dp, w.dn, loss, w.trip_ws, w.trip_bytes, stream));
-  k_store_one<<<1, 1, 0, st>>>(w.one, 1.0f);
+  TSG_TRY(triplet_fwd(emb, triplets, T, G, C, hd->margin, hd->eps, w.dp, w.dn, loss, w.one, w.trip_ws, w.trip_bytes, stream));
   TSG_TRY(tsg_triplet_bwd(emb, triplets, T, G, C, hd->margin, hd->eps, w.dp, w.dn, w.one, w.demb, w.trip_ws, w.trip_bytes, stream));
   return step_bwd(sh, hd, label, level_ptr, params, emb, w.demb, grads, w, arena, arena_bytes, stream);
 }
@@ -558,9 +563,10 @@ extern "C" int tsg_sag_nll_step_compact(const tsg_sag_shape* sh, const tsg_sag_h
   const int C = (int)hd->num_classes, G = (int)sh->num_graphs;
   float* emb = emb_out ? emb_out : w.emb;
   TSG_TRY(step_fwd(sh, hd, label, local_row, local_col, edge_ptr, level_ptr, params, dropout_mask, emb, w, arena, arena_bytes, stream));
-  k_nll_demb<<<grid_for((int64_t)G * C, 256, 8), 256, 0, st>>>(emb, y, G, C, w.demb, w.nll, step_status(sh, arena));
-  k_sum_fixed<<<1, SUM_THREADS, 0, st>>>(w.nll, nullptr, G, (float)G, loss, nullptr);
-  TSG_LAUNCH_CHECK("sag_nll_step(loss)");
+  TSG_LAUNCH_PDL("sag_nll_step(demb)", k_nll_demb, grid_for((int64_t)G * C, 256, 8), 256, 0, st, (const float*)emb, y, G, C, w.demb,
+                 w.nll, step_status(sh, arena));
+  TSG_LAUNCH_PDL("sag_nll_step(loss)", k_sum_fixed, 1, SUM_THREADS, 0, st, (const float*)w.nll, (const int*)nullptr, G, (float)G, loss,
+                 (int64_t*)nullptr);
   return step_bwd(sh, hd, label, level_ptr, params, emb, w.demb, grads, w, arena, arena_bytes, stream);
 }
 

@@ -146,7 +146,8 @@ extern "C" int tsg_linkpred_loss_fwd(const float* S, const int64_t* graph_ptr, c
   float* total = part + G;
   if (G == 0) { cudaMemsetAsync(loss, 0, 4, st); return TSG_OK; }
   k_linkpred<0><<<(int)G, LP_T, smem, st>>>(S, graph_ptr, rowptr, colidx, (int)K, eps, part, nullptr, 0.f, nullptr);
-  launch_partial_sum_final(part, total, 1, nullptr, (int)G, 1, st);
+  rc = launch_partial_sum_final(part, total, 1, nullptr, (int)G, 1, st);
+  if (rc) return rc;
   k_lp_finish<<<1, 1, 0, st>>>(total, (float)(1.0 / num_entries), loss);
   return check_launch("linkpred_loss_fwd");
 }

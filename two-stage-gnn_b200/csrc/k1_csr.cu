@@ -26,6 +26,8 @@ struct CsrArgs {
 };
 
 __global__ void k_csr_count(CsrArgs a, int* cnt_dst, int* cnt_src, int* loop_eid) {
+  pdl_wait();
+  pdl_launch_dependents();
   int64_t E = dev_count(a.E_cap, a.E_dev);
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < E;
        e += (int64_t)gridDim.x * blockDim.x) {
@@ -46,6 +48,8 @@ struct CountPlus {
 
 __global__ void k_csr_fill(CsrArgs a, const int* rowptr, int* fill_dst, int* tmp_dst,
                            const int* t_rowptr, int* fill_src, int* tmp_src) {
+  pdl_wait();
+  pdl_launch_dependents();
   int64_t E = dev_count(a.E_cap, a.E_dev);
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < E;
        e += (int64_t)gridDim.x * blockDim.x) {
@@ -66,6 +70,8 @@ __global__ void k_csr_place(CsrArgs a, const int* rowptr, const int* cnt_dst, co
                             int* colidx, int* eid,
                             const int* t_rowptr, const int* cnt_src, const int* tmp_src,
                             int* t_colidx, int* t_eid) {
+  pdl_wait();
+  pdl_launch_dependents();
   int64_t E = dev_count(a.E_cap, a.E_dev);
   int64_t stride = (int64_t)gridDim.x * blockDim.x;
   int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -102,6 +108,8 @@ __global__ void k_csr_place(CsrArgs a, const int* rowptr, const int* cnt_dst, co
 // dis[c] = 1/sqrt(sum of weights into c) ; sequential in CSR (= COO) order.
 __global__ void k_csr_degree(CsrArgs a, const int* rowptr, const int* eid_or_tmp, const int* loop_eid,
                              float* dis) {
+  pdl_wait();
+  pdl_launch_dependents();
   for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < a.N;
        c += (int64_t)gridDim.x * blockDim.x) {
     int s = rowptr[c], t = rowptr[c + 1] - 1;    // last slot is the loop
@@ -122,6 +130,8 @@ __global__ void k_csr_degree(CsrArgs a, const int* rowptr, const int* eid_or_tmp
 // one thread per CSR slot of one orientation; `rows` says which endpoint indexes the row.
 __global__ void k_csr_values(CsrArgs a, const int* rowptr, const int* colidx, const int* eid,
                              const int* loop_eid, const float* dis, float* val, int dst_major) {
+  pdl_wait();
+  pdl_launch_dependents();
   // thread per row, walking its slots: rows are short and this keeps row id for free.
   for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < a.N;
        r += (int64_t)gridDim.x * blockDim.x) {
@@ -206,15 +216,19 @@ extern "C" int tsg_csr_build(const int64_t* row, const int64_t* col, const float
 
   const int T = 256;
   int ge = grid_for(E, T), gn = grid_for(N, T);
-  if (E > 0) k_csr_count<<<ge, T, 0, st>>>(a, cnt_dst, both ? cnt_src : nullptr, loop_eid);
+  if (E > 0) TSG_LAUNCH_PDL("csr_build(count)", k_csr_count, ge, T, 0, st, a, cnt_dst, both ? cnt_src : nullptr, loop_eid);
   int rc = exclusive_scan(CountPlus{cnt_dst, gcn}, N, rowptr, scan_ws, st);
   if (rc) return rc;
   if (both) { rc = exclusive_scan(CountPlus{cnt_src, gcn}, N, t_rowptr, scan_ws, st); if (rc) return rc; }
-  if (E > 0) k_csr_fill<<<ge, T, 0, st>>>(a, rowptr, fill_dst, tmp_dst, both ? t_rowptr : nullptr, fill_src, tmp_src);
-  k_csr_place<<<grid_for(E > N ? E : N, T), T, 0, st>>>(a, rowptr, cnt_dst, tmp_dst, colidx, eid,
-                                                       both ? t_rowptr : nullptr, cnt_src, tmp_src, t_colidx, t_eid);
-  if (gcn) k_csr_degree<<<gn, T, 0, st>>>(a, rowptr, eid, loop_eid, dis);
-  k_csr_values<<<gn, T, 0, st>>>(a, rowptr, colidx, eid, loop_eid, dis, val, 1);
-  if (both) k_csr_values<<<gn, T, 0, st>>>(a, t_rowptr, t_colidx, t_eid, loop_eid, dis, t_val, 0);
-  return check_launch("csr_build");
+  const int* no_rows = nullptr;
+  if (E > 0) TSG_LAUNCH_PDL("csr_build(fill)", k_csr_fill, ge, T, 0, st, a, (const int*)rowptr, fill_dst, tmp_dst, both ? t_rowptr : no_rows,
+                            fill_src, tmp_src);
+  TSG_LAUNCH_PDL("csr_build(place)", k_csr_place, grid_for(E > N ? E : N, T), T, 0, st, a, (const int*)rowptr, (const int*)cnt_dst,
+                 (const int*)tmp_dst, colidx, eid, both ? t_rowptr : no_rows, (const int*)cnt_src, (const int*)tmp_src, t_colidx, t_eid);
+  if (gcn) TSG_LAUNCH_PDL("csr_build(degree)", k_csr_degree, gn, T, 0, st, a, (const int*)rowptr, (const int*)eid, (const int*)loop_eid, dis);
+  TSG_LAUNCH_PDL("csr_build(values)", k_csr_values, gn, T, 0, st, a, (const int*)rowptr, (const int*)colidx, (const int*)eid,
+                 (const int*)loop_eid, (const float*)dis, val, 1);
+  if (both) TSG_LAUNCH_PDL("csr_build(values)", k_csr_values, gn, T, 0, st, a, (const int*)t_rowptr, (const int*)t_colidx,
+                           (const int*)t_eid, (const int*)loop_eid, (const float*)dis, t_val, 0);
+  return TSG_OK;
 }

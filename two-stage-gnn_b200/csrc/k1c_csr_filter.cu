@@ -16,6 +16,8 @@
 namespace tsg {
 
 __global__ void k_inv_perm32(const int64_t* __restrict__ perm, int64_t k, int* __restrict__ inv) {
+  pdl_wait();
+  pdl_launch_dependents();
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < k; i += (int64_t)gridDim.x * blockDim.x)
     inv[perm[i]] = (int)i;
 }
@@ -25,6 +27,8 @@ __global__ void __launch_bounds__(256)
 k_csrf_count(const int* __restrict__ rowptr, const int* __restrict__ colidx, const int* __restrict__ t_rowptr,
              const int* __restrict__ t_colidx, const int64_t* __restrict__ perm, const int* __restrict__ inv,
              int k, int* __restrict__ cnt, int halves) {
+  pdl_wait();
+  pdl_launch_dependents();
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < halves * k; i += gridDim.x * blockDim.x) {
     const bool tr = i >= k;
     const int r = (int)perm[tr ? i - k : i];
@@ -45,6 +49,8 @@ k_csrf_write(const int* __restrict__ rowptr, const int* __restrict__ colidx, con
              int k, const int* __restrict__ cnt, const int* __restrict__ off,
              int* __restrict__ n_rowptr, int* __restrict__ n_colidx, float* __restrict__ n_val,
              int* __restrict__ nt_rowptr, int* __restrict__ nt_colidx, float* __restrict__ nt_val, int halves) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int half = off[k];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < halves * k; i += gridDim.x * blockDim.x) {
     const bool tr = i >= k;
@@ -78,8 +84,8 @@ extern "C" int tsg_inv_perm(const int64_t* perm, int64_t num_perm, int64_t num_n
   TSG_REQUIRE(num_perm >= 0 && num_nodes >= 0 && (num_nodes == 0 || inv_perm) && (num_perm == 0 || perm), "inv_perm: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
   if (num_nodes > 0) cudaMemsetAsync(inv_perm, 0xFF, (size_t)num_nodes * 4, st);
-  if (num_perm > 0) k_inv_perm32<<<grid_for(num_perm, 256), 256, 0, st>>>(perm, num_perm, inv_perm);
-  return check_launch("inv_perm");
+  if (num_perm > 0) TSG_LAUNCH_PDL("inv_perm", k_inv_perm32, grid_for(num_perm, 256), 256, 0, st, perm, num_perm, inv_perm);
+  return TSG_OK;
 }
 
 extern "C" size_t tsg_csr_filter_workspace_bytes(int64_t num_perm) {
@@ -106,10 +112,9 @@ extern "C" int tsg_csr_filter(const int32_t* rowptr, const int32_t* colidx, cons
   int* off = ws.take<int>(2 * num_perm + 2);
   int* scan_ws = ws.take<int>(scan_ws_ints(2 * num_perm + 1));
   const int grid = grid_for(halves * num_perm, 256);
-  k_csrf_count<<<grid, 256, 0, st>>>(rowptr, colidx, t_rowptr, t_colidx, perm, inv_perm, k, cnt, halves);
+  TSG_LAUNCH_PDL("csr_filter(count)", k_csrf_count, grid, 256, 0, st, rowptr, colidx, t_rowptr, t_colidx, perm, inv_perm, k, cnt, halves);
   int rc = exclusive_scan(CsrfCnt{cnt}, halves * num_perm, off, scan_ws, st);
   if (rc) return rc;
-  k_csrf_write<<<grid, 256, 0, st>>>(rowptr, colidx, t_rowptr, t_colidx, perm, inv_perm, k, cnt, off,
-                                     out_rowptr, out_colidx, out_val, out_t_rowptr, out_t_colidx, out_t_val, halves);
-  return check_launch("csr_filter");
+  return launch_pdl("csr_filter", k_csrf_write, grid, 256, 0, st, rowptr, colidx, t_rowptr, t_colidx, perm, inv_perm, k, (const int*)cnt,
+                    (const int*)off, out_rowptr, out_colidx, out_val, out_t_rowptr, out_t_colidx, out_t_val, halves);
 }

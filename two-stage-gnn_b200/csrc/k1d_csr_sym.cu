@@ -23,6 +23,8 @@ __global__ void __launch_bounds__(CSYM_THREADS)
 k_csr_sym(const int32_t* __restrict__ lrow, const int32_t* __restrict__ lcol, const int64_t* __restrict__ edge_ptr,
           const int64_t* __restrict__ node_ptr, int G, int nmax, int32_t* __restrict__ rowptr, int32_t* __restrict__ colidx,
           float* __restrict__ val, int* __restrict__ status) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) unsigned char sm[];
   int* rs = reinterpret_cast<int*>(sm);                       // [nmax + 2] first edge of every row
   float* dis = reinterpret_cast<float*>(sm + (size_t)(nmax + 2) * 4);
@@ -104,7 +106,6 @@ extern "C" int tsg_csr_build_graphs_sym_local(const int32_t* local_row, const in
     configured = 200 * 1024;
   }
   const int grid = (int)(G < (int64_t)TSG_NUM_SMS * 8 ? G : (int64_t)TSG_NUM_SMS * 8);
-  k_csr_sym<<<grid, CSYM_THREADS, smem, (cudaStream_t)stream>>>(local_row, local_col, edge_ptr, node_ptr, (int)G,
-                                                                  (int)max_graph_nodes, rowptr, colidx, val, status);
-  return check_launch("csr_build_graphs_sym");
+  return launch_pdl("csr_build_graphs_sym", k_csr_sym, grid, CSYM_THREADS, smem, (cudaStream_t)stream, local_row, local_col, edge_ptr,
+                    node_ptr, (int)G, (int)max_graph_nodes, rowptr, colidx, val, status);
 }

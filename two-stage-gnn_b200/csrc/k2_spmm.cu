@@ -29,6 +29,8 @@ k_spmm_vec4(const int* __restrict__ rowptr, const int* __restrict__ colidx,
             const float* __restrict__ val, const float4* __restrict__ H,
             const float4* __restrict__ bias, float4* __restrict__ Y,
             int num_rows, int F4, int relu) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int lane_in_row = threadIdx.x % LPR;
   // blocked assignment: CTA b owns rows [b*rpc, (b+1)*rpc) so the rows of one small graph (whose
   // neighbours are each other) are gathered through the same SM's L1
@@ -84,6 +86,8 @@ k_spmm_scalar(const int* __restrict__ rowptr, const int* __restrict__ colidx,
               const float* __restrict__ val, const float* __restrict__ H,
               const float* __restrict__ bias, float* __restrict__ Y,
               int num_rows, int F, int relu) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int lane_in_row = threadIdx.x % LPR;
   // blocked assignment: CTA b owns rows [b*rpc, (b+1)*rpc) so the rows of one small graph (whose
   // neighbours are each other) are gathered through the same SM's L1
@@ -281,6 +285,8 @@ k_spmm_g(const int* __restrict__ rowptr, const int* __restrict__ colidx,
          int num_rows, int F4, int relu, int hdist,
          const float4* __restrict__ dot_vec, float* __restrict__ dot_out,
          const int* __restrict__ row_label = nullptr, int num_labels = 0) {
+  pdl_wait();
+  pdl_launch_dependents();
   // (MODE & 2): H is a [num_labels, F] TABLE and neighbour c contributes H[row_label[c]] -- conv1 on one-hot
   // node-label features (x W = W[label]) without ever materialising x W: the gathers hit an L1-resident table.
   constexpr int RPI = THREADS / LPR;              // rows per CTA iteration
@@ -585,7 +591,7 @@ static int launch_spmm(const int* rowptr, const int* colidx, const float* val, c
     static const int ctas_per_sm_1024 = env_int("TSG_SPMM_CTAS", 2);
     if (legacy && row_label == nullptr) {
       int grid = grid_for(N, SPMM_THREADS / lpr, 32);
-#define TSG_GO(L) k_spmm_vec4<L, HAS_VAL><<<grid, SPMM_THREADS, 0, st>>>(rowptr, colidx, val, (const float4*)H, (const float4*)bias, (float4*)Y, (int)N, F4, relu)
+#define TSG_GO(L) TSG_LAUNCH_PDL("spmm", k_spmm_vec4<L, HAS_VAL>, grid, SPMM_THREADS, 0, st, rowptr, colidx, val, (const float4*)H, (const float4*)bias, (float4*)Y, (int)N, F4, relu)
       switch (lpr) {
         case 1: TSG_GO(1); break; case 2: TSG_GO(2); break; case 4: TSG_GO(4); break;
         case 8: TSG_GO(8); break; case 16: TSG_GO(16); break; default: TSG_GO(32); break;
@@ -606,7 +612,7 @@ static int launch_spmm(const int* rowptr, const int* colidx, const float* val, c
       const float4* dv = fuse_dot ? (const float4*)dot_vec : nullptr;
       if (dot_done) *dot_done = fuse_dot;
       const int mode = (dv ? 1 : 0) | (row_label ? 2 : 0);
-#define TSG_GM(L, FM, T, M) k_spmm_g<L, HAS_VAL, FM, T, M><<<g, T, 0, st>>>(rowptr, colidx, val, (const float4*)H, (const float4*)bias, (float4*)Y, (int)N, F4, relu, big ? hdist : 0, dv, dot_out, row_label, num_labels)
+#define TSG_GM(L, FM, T, M) TSG_LAUNCH_PDL("spmm", k_spmm_g<L, HAS_VAL, FM, T, M>, g, T, 0, st, rowptr, colidx, val, (const float4*)H, (const float4*)bias, (float4*)Y, (int)N, F4, relu, big ? hdist : 0, dv, dot_out, row_label, num_labels)
 #define TSG_G(L, FM, T) { if (mode == 0) TSG_GM(L, FM, T, 0); else if (mode == 1) TSG_GM(L, FM, T, 1); else if (mode == 2) TSG_GM(L, FM, T, 2); else TSG_GM(L, FM, T, 3); }
 #define TSG_GT(L, FM) if (big) TSG_G(L, FM, 1024) else TSG_G(L, FM, 256)
 #define TSG_GV(L) if (exact) { TSG_GT(L, false) } else { TSG_GT(L, true) }
@@ -623,7 +629,7 @@ static int launch_spmm(const int* rowptr, const int* colidx, const float* val, c
     int lpr = 1; while (lpr < F && lpr < 32) lpr <<= 1;
     int rows_per_block = SPMM_THREADS / lpr;
     int grid = grid_for(N, rows_per_block, 32);
-#define TSG_GO(L) k_spmm_scalar<L, HAS_VAL><<<grid, SPMM_THREADS, 0, st>>>(rowptr, colidx, val, H, bias, Y, (int)N, (int)F, relu)
+#define TSG_GO(L) TSG_LAUNCH_PDL("spmm", k_spmm_scalar<L, HAS_VAL>, grid, SPMM_THREADS, 0, st, rowptr, colidx, val, H, bias, Y, (int)N, (int)F, relu)
     switch (lpr) {
       case 1: TSG_GO(1); break; case 2: TSG_GO(2); break; case 4: TSG_GO(4); break;
       case 8: TSG_GO(8); break; case 16: TSG_GO(16); break; default: TSG_GO(32); break;
@@ -745,6 +751,8 @@ k_sag_conv_bwd_v4(const float4* __restrict__ dxo, const int* __restrict__ inv, c
                   const float4* __restrict__ Y, const float* __restrict__ dsw, const float4* __restrict__ ws4,
                   float4* __restrict__ dYm, float* __restrict__ part, int64_t N, int F4, int64_t rows_per_block,
                   float* __restrict__ dbias, float* __restrict__ dws, unsigned* ticket) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ float4 sm4[];                       // [2][CS_THREADS]
   int64_t r0 = (int64_t)blockIdx.x * rows_per_block;
   int64_t r1 = r0 + rows_per_block; if (r1 > N) r1 = N;
@@ -935,7 +943,7 @@ extern "C" int tsg_relu_bwd_colsum_rank1(const float* dY, const float* Y, const 
   else
     k_relu_bwd_colsum<<<nb, CS_THREADS, CS_THREADS * sizeof(float), st>>>(dY, Y, dYm, part, N, (int)F, rpb, row_scale, col_vec,
                                                                         dbias, ticket);
-  if (!ticket) launch_partial_sum_final(part, dbias, (int)F, nullptr, nb, (int)F, st);
+  if (!ticket) { int rc = launch_partial_sum_final(part, dbias, (int)F, nullptr, nb, (int)F, st); if (rc) return rc; }
   return check_launch("relu_bwd_colsum");
 }
 
@@ -955,12 +963,12 @@ extern "C" int tsg_sag_conv_bwd_fused(const float* dxo, const int32_t* inv, cons
   int64_t rpb = (N + nb - 1) / nb; if (rpb < 1) rpb = 1;
   unsigned* ticket = fused_tail_ok(nb, 2 * F) ? ticket_next() : nullptr;
   static const int cbr = env_int("TSG_CONV_BWD_ROWS", 2);      // measured at the level-0 shape: 1: 99 us, 2: 79, 4: 83, 8: 99
-#define TSG_CB(R) k_sag_conv_bwd_v4<R><<<nb, CS_THREADS, 2 * CS_THREADS * sizeof(float4), st>>>(                         \
+#define TSG_CB(R) TSG_LAUNCH_PDL("sag_conv_bwd_fused", k_sag_conv_bwd_v4<R>, nb, CS_THREADS, 2 * CS_THREADS * sizeof(float4), st, \
       (const float4*)dxo, inv, score, (const float4*)h, dsw, (const float4*)ws_vec, (float4*)dhm, part, N, (int)(F / 4), rpb, \
       dbias, dws, ticket)
   if (cbr == 1) TSG_CB(1); else if (cbr == 4) TSG_CB(4); else if (cbr == 8) TSG_CB(8); else TSG_CB(2);
 #undef TSG_CB
-  if (!ticket) launch_partial_sum_final(part, dbias, (int)F, dws, nb, (int)(2 * F), st);
+  if (!ticket) { int rc = launch_partial_sum_final(part, dbias, (int)F, dws, nb, (int)(2 * F), st); if (rc) return rc; }
   return check_launch("sag_conv_bwd_fused");
 }
 

@@ -146,6 +146,8 @@ __global__ void __launch_bounds__(LIN_THREADS)
 k_linear_fwd(const float* __restrict__ X, const float* __restrict__ W, const float* __restrict__ bias,
              float* __restrict__ Y, int N, int K, int M, int ldw, int ldy, int w_transposed, int flags, int ldx,
              int kmode) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float smem[];
   constexpr int RS = LIN_THREADS / CG;
   constexpr int R = RS * LIN_RPT;
@@ -232,6 +234,8 @@ template <int CG>
 __global__ void __launch_bounds__(LIN_THREADS)
 k_linear_fwd_dense(const float* __restrict__ X, const float* __restrict__ W, const float* __restrict__ bias,
                    float* __restrict__ Y, int N, int K, int M, int ldw, int ldy, int w_transposed, int flags) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float smem[];
   constexpr int RS = LIN_THREADS / CG;
   constexpr int R = RS * LIND_RPT;
@@ -476,6 +480,8 @@ template <int NK, int U>
 __global__ void __launch_bounds__(256)
 k_linear_bwd_weight(const float* __restrict__ X, const float* __restrict__ dY, float* __restrict__ part,
                     int N, int K, int M, int m0, int ldx) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float smem[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
   float* acc = smem + (size_t)w * K * 32;                   // [K][32] private to this warp
@@ -553,6 +559,8 @@ constexpr int LBWD_ROWS = 128;
 __global__ void __launch_bounds__(256)
 k_linear_bwd_weight_dense(const float* __restrict__ X, const float* __restrict__ dY, float* __restrict__ part,
                           int N, int K, int M) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float smem[];
   const int KB = K >> 2, MB = M >> 2, NB = KB * MB;
   const int groups = 256 / NB;                       // >= 1
@@ -625,6 +633,8 @@ template <int LPR>
 __global__ void __launch_bounds__(256)
 k_linear_fwd_small(const float* __restrict__ X, const float* __restrict__ W, const float* __restrict__ bias,
                    float* __restrict__ Y, int N, int K, int M, int w_transposed) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ float Ws[4][512];                   // [m][k], K <= 512
   for (int i = threadIdx.x; i < M * K; i += 256) {
     int m = i / K, k = i - m * K;
@@ -666,6 +676,8 @@ template <int LPR>
 __global__ void __launch_bounds__(256)
 k_linear_bwd_weight_small(const float* __restrict__ X, const float* __restrict__ dY, float* __restrict__ part,
                           int N, int K, int M, float* __restrict__ dW, unsigned* ticket) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) float smem[];            // [groups][K*M] for the in-CTA combine
   const int l = threadIdx.x % LPR, grp = threadIdx.x / LPR;
   const int groups = 256 / LPR;
@@ -751,7 +763,7 @@ extern "C" int tsg_linear_fwd(const float* X, const float* W, const float* bias,
   if (M <= 4 && flags == 0 && (K & 3) == 0 && K <= 128 && (((uintptr_t)X) & 15) == 0) {   // GEMV-shaped
     int lpr = 1; while (lpr * 4 < K) lpr <<= 1;
     int grid = grid_for(N, 256 / lpr, 16);
-#define TSG_GOS(L) k_linear_fwd_small<L><<<grid, 256, 0, st>>>(X, W, bias, Y, (int)N, (int)K, (int)M, w_transposed)
+#define TSG_GOS(L) TSG_LAUNCH_PDL("linear_fwd(small)", k_linear_fwd_small<L>, grid, 256, 0, st, X, W, bias, Y, (int)N, (int)K, (int)M, w_transposed)
     switch (lpr) {
       case 1: TSG_GOS(1); break; case 2: TSG_GOS(2); break; case 4: TSG_GOS(4); break;
       case 8: TSG_GOS(8); break; case 16: TSG_GOS(16); break; default: TSG_GOS(32); break;
@@ -776,7 +788,8 @@ extern "C" int tsg_linear_fwd(const float* X, const float* W, const float* bias,
       int grid_d = tiles_d < TSG_NUM_SMS * 4 ? tiles_d : TSG_NUM_SMS * 4;
 #define TSG_GOD(C)                                                                                  \
       rc = set_smem(k_linear_fwd_dense<C>, smem_d, "linear_fwd(dense)"); if (rc) return rc;           \
-      k_linear_fwd_dense<C><<<grid_d, LIN_THREADS, smem_d, st>>>(X, Wc, bc, Yc, (int)N, (int)K, (int)mc, ldw, (int)M, w_transposed, flags)
+      TSG_LAUNCH_PDL("linear_fwd(dense)", k_linear_fwd_dense<C>, grid_d, LIN_THREADS, smem_d, st, X, Wc, bc, Yc, (int)N, (int)K, (int)mc, ldw, \
+                     (int)M, w_transposed, flags)
       switch (cg) {
         case 1: TSG_GOD(1); break; case 2: TSG_GOD(2); break; case 4: TSG_GOD(4); break;
         case 8: TSG_GOD(8); break; case 16: TSG_GOD(16); break; default: TSG_GOD(32); break;
@@ -798,8 +811,8 @@ extern "C" int tsg_linear_fwd(const float* X, const float* W, const float* bias,
       int grid = tiles < TSG_NUM_SMS * 4 ? tiles : TSG_NUM_SMS * 4;
 #define TSG_GO(C)                                                                                  \
       rc = set_smem(k_linear_fwd<C>, smem, "linear_fwd"); if (rc) return rc;                        \
-      k_linear_fwd<C><<<grid, LIN_THREADS, smem, st>>>(X + k0, Wb, bc, Yc, (int)N, (int)kc, (int)mc, ldw, (int)M,      \
-                                                       w_transposed, flags, (int)K, kmode)
+      TSG_LAUNCH_PDL("linear_fwd", k_linear_fwd<C>, grid, LIN_THREADS, smem, st, X + k0, Wb, bc, Yc, (int)N, (int)kc, (int)mc, \
+                     ldw, (int)M, w_transposed, flags, (int)K, kmode)
       switch (cgb) {
         case 1: TSG_GO(1); break; case 2: TSG_GO(2); break; case 4: TSG_GO(4); break;
         case 8: TSG_GO(8); break; case 16: TSG_GO(16); break; default: TSG_GO(32); break;
@@ -867,13 +880,13 @@ extern "C" int tsg_linear_bwd_weight(const float* X, const float* dY, float* dW,
       unsigned* ticket = fused_tail_ok(grid, K * M) ? ticket_next() : nullptr;
 #define TSG_GOS(L)                                                                                          \
       { int rc = set_smem(k_linear_bwd_weight_small<L>, smem_s, "linear_bwd_weight(small)"); if (rc) return rc; \
-        k_linear_bwd_weight_small<L><<<grid, 256, smem_s, st>>>(X, dY, part, (int)N, (int)K, (int)M, dW, ticket); }
+        TSG_LAUNCH_PDL("linear_bwd_weight(small)", k_linear_bwd_weight_small<L>, grid, 256, smem_s, st, X, dY, part, (int)N, (int)K, (int)M, dW, ticket); }
       switch (lpr) {
         case 1: TSG_GOS(1) break; case 2: TSG_GOS(2) break; case 4: TSG_GOS(4) break;
         case 8: TSG_GOS(8) break; case 16: TSG_GOS(16) break; default: TSG_GOS(32) break;
       }
 #undef TSG_GOS
-      if (!ticket) launch_partial_sum_final(part, dW, (int)(K * M), nullptr, grid, (int)(K * M), st);
+      if (!ticket) { int rc = launch_partial_sum_final(part, dW, (int)(K * M), nullptr, grid, (int)(K * M), st); if (rc) return rc; }
       return check_launch("linear_bwd_weight(small)");
     }
   }
@@ -885,8 +898,8 @@ extern "C" int tsg_linear_bwd_weight(const float* X, const float* dY, float* dW,
     if (red > smem_d) smem_d = red;
     if (smem_d <= 200 * 1024) {
       int rc = set_smem(k_linear_bwd_weight_dense, smem_d, "linear_bwd_weight(dense)"); if (rc) return rc;
-      k_linear_bwd_weight_dense<<<LBW_GRID, 256, smem_d, st>>>(X, dY, part, (int)N, (int)K, (int)M);
-      launch_partial_sum_final(part, dW, (int)(K * M), nullptr, LBW_GRID, (int)(K * M), st);
+      TSG_LAUNCH_PDL("linear_bwd_weight(dense)", k_linear_bwd_weight_dense, LBW_GRID, 256, smem_d, st, X, dY, part, (int)N, (int)K, (int)M);
+      rc = launch_partial_sum_final(part, dW, (int)(K * M), nullptr, LBW_GRID, (int)(K * M), st); if (rc) return rc;
       return check_launch("linear_bwd_weight(dense)");
     }
   }
@@ -902,7 +915,8 @@ extern "C" int tsg_linear_bwd_weight(const float* X, const float* dY, float* dW,
     for (int m0 = 0; m0 < M; m0 += 32) {
 #define TSG_GO(NK_, U_)                                                                                    \
       { int rc = set_smem(k_linear_bwd_weight<NK_, U_>, smem, "linear_bwd_weight"); if (rc) return rc;       \
-        k_linear_bwd_weight<NK_, U_><<<grid, nwarps * 32, smem, st>>>(X + k0, dY, part, (int)N, (int)kc, (int)M, m0, (int)K); }
+        TSG_LAUNCH_PDL("linear_bwd_weight", k_linear_bwd_weight<NK_, U_>, grid, nwarps * 32, smem, st, X + k0, dY, part, (int)N, (int)kc, \
+                       (int)M, m0, (int)K); }
       switch (nk) {
         case 1: TSG_GO(1, 8); break; case 2: TSG_GO(2, 8); break; case 3: TSG_GO(3, 4); break;
         case 4: TSG_GO(4, 4); break; case 5: TSG_GO(5, 2); break; case 6: TSG_GO(6, 2); break;
@@ -910,7 +924,8 @@ extern "C" int tsg_linear_bwd_weight(const float* X, const float* dY, float* dW,
       }
 #undef TSG_GO
     }
-    launch_partial_sum_final(part, dW + k0 * M, (int)(kc * M), nullptr, grid, (int)(kc * M), st);
+    int rc = launch_partial_sum_final(part, dW + k0 * M, (int)(kc * M), nullptr, grid, (int)(kc * M), st);
+    if (rc) return rc;
   }
   return check_launch("linear_bwd_weight");
 }

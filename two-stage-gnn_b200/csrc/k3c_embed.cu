@@ -24,6 +24,8 @@ template <bool VEC4>
 __global__ void __launch_bounds__(EMB_THREADS)
 k_embed_fwd(const float* __restrict__ W, const int* __restrict__ label, float* __restrict__ out,
             int64_t N, int K, int M) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   if (VEC4) {
     const int m4 = M >> 2;
@@ -72,6 +74,8 @@ template <int EMB_UNROLL, bool PIPE>
 __global__ void __launch_bounds__(512)
 k_embed_bwd_weight(const int* __restrict__ label, const float* __restrict__ dY, float* __restrict__ part,
                    int64_t N, int K, int M, int64_t rows_per_cta) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ float tab[];
   const int nw = blockDim.x >> 5, w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int KM = K * M;
@@ -142,9 +146,8 @@ extern "C" int tsg_embed_fwd(const float* W, const int32_t* label, float* out, i
   const bool v4 = (M % 4 == 0) && (((uintptr_t)W | (uintptr_t)out) % 16 == 0);
   const int64_t total = v4 ? N * (M / 4) : N * M;
   const int grid = grid_for((total + EMB_FWD_ILP - 1) / EMB_FWD_ILP, EMB_THREADS, 8);
-  if (v4) k_embed_fwd<true><<<grid, EMB_THREADS, 0, st>>>(W, label, out, N, (int)K, (int)M);
-  else k_embed_fwd<false><<<grid, EMB_THREADS, 0, st>>>(W, label, out, N, (int)K, (int)M);
-  return check_launch("embed_fwd");
+  if (v4) return launch_pdl("embed_fwd", k_embed_fwd<true>, grid, EMB_THREADS, 0, st, W, label, out, N, (int)K, (int)M);
+  return launch_pdl("embed_fwd", k_embed_fwd<false>, grid, EMB_THREADS, 0, st, W, label, out, N, (int)K, (int)M);
 }
 
 /* 0 when the [K, M] table does not fit one warp's share of shared memory (use the dense K3 product instead) */
@@ -169,11 +172,14 @@ extern "C" int tsg_embed_bwd_weight(const int32_t* label, const float* dY, float
   static const int variant = [] { const char* e = getenv("TSG_EMB_VARIANT"); return e ? atoi(e) : 0; }();
   auto launch = [&](auto kern) {
     if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    kern<<<EMB_BWD_GRID, nw * 32, smem, st>>>(label, dY, part, N, (int)K, (int)M, rows_per_cta);
+    return launch_pdl("embed_bwd_weight", kern, EMB_BWD_GRID, nw * 32, smem, st, label, dY, part, N, (int)K, (int)M, rows_per_cta);
   };
-  if (variant == 1) launch(k_embed_bwd_weight<8, true>);          // A/B variants (TSG_EMB_VARIANT), measured in
-  else if (variant == 2) launch(k_embed_bwd_weight<16, false>);   // profiles/r01c_compact_input.md
-  else launch(k_embed_bwd_weight<16, true>);
-  launch_partial_sum_final(part, dW, (int)(K * M), nullptr, EMB_BWD_GRID, (int)(K * M), st);
+  int rc;
+  if (variant == 1) rc = launch(k_embed_bwd_weight<8, true>);          // A/B variants (TSG_EMB_VARIANT), measured in
+  else if (variant == 2) rc = launch(k_embed_bwd_weight<16, false>);   // profiles/r01c_compact_input.md
+  else rc = launch(k_embed_bwd_weight<16, true>);
+  if (rc) return rc;
+  rc = launch_partial_sum_final(part, dW, (int)(K * M), nullptr, EMB_BWD_GRID, (int)(K * M), st);
+  if (rc) return rc;
   return check_launch("embed_bwd_weight");
 }

@@ -40,6 +40,8 @@ __global__ void __launch_bounds__(TOPK_THREADS)
 k_topk_rank(const float* __restrict__ score, const int64_t* __restrict__ gptr,
             const int64_t* __restrict__ kptr, int64_t* __restrict__ perm, unsigned long long* __restrict__ gkeys,
             int skip_upto) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ __align__(16) unsigned long long skeys[TOPK_SMEM_KEYS];
   const int g = blockIdx.x;
   const int64_t base = gptr[g];
@@ -78,6 +80,8 @@ constexpr int TOPK_SORT_THREADS = 256;
 __global__ void __launch_bounds__(TOPK_SORT_THREADS)
 k_topk_sort(const float* __restrict__ score, const int64_t* __restrict__ gptr, const int64_t* __restrict__ kptr,
             int64_t* __restrict__ perm, int max_pad, int min_n) {
+  pdl_wait();
+  pdl_launch_dependents();
   extern __shared__ __align__(16) unsigned long long sk[];
   {
     const int g = blockIdx.x;
@@ -225,6 +229,8 @@ constexpr int TOPK_WARP_KEYS = 128;
 __global__ void __launch_bounds__(TOPK_RUN_THREADS)
 k_topk_runs(const float* __restrict__ score, const int64_t* __restrict__ gptr, const int64_t* __restrict__ kptr,
             int64_t* __restrict__ perm, int G, int cta_blocks) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ __align__(16) unsigned long long runs[TOPK_RUN_THREADS * 4];
   constexpr int NW = TOPK_RUN_THREADS / 32;
   if ((int)blockIdx.x >= cta_blocks) {
@@ -435,6 +441,8 @@ __global__ void __launch_bounds__(GSB_THREADS)
 k_gate_score_bwd(const float4* __restrict__ dxo, const float4* __restrict__ x, const float* __restrict__ score,
                  const int64_t* __restrict__ perm, float* __restrict__ dscore, float* __restrict__ part,
                  int64_t K, int F4, float* __restrict__ dbs, unsigned* ticket) {
+  pdl_wait();
+  pdl_launch_dependents();
   constexpr int GROUPS = GSB_THREADS / LPR;
   __shared__ float s_sum[GSB_THREADS / 32];
   const int l = threadIdx.x % LPR, grp = threadIdx.x / LPR;
@@ -531,14 +539,14 @@ extern "C" int tsg_topk_bounded(const float* score, const int64_t* gptr, const i
     const int cta_blocks = (int)(G < (int64_t)TSG_NUM_SMS * 8 ? G : (int64_t)TSG_NUM_SMS * 8);
     const int64_t groups = (G + TOPK_RUN_THREADS / 32 - 1) / (TOPK_RUN_THREADS / 32);
     const int warp_blocks = (int)(groups < (int64_t)TSG_NUM_SMS * 4 ? groups : (int64_t)TSG_NUM_SMS * 4);
-    k_topk_runs<<<cta_blocks + warp_blocks, TOPK_RUN_THREADS, 0, (cudaStream_t)stream>>>(score, gptr, kptr, perm, (int)G, cta_blocks);
+    TSG_LAUNCH_PDL("topk(runs)", k_topk_runs, cta_blocks + warp_blocks, TOPK_RUN_THREADS, 0, (cudaStream_t)stream, score, gptr, kptr, perm, (int)G, cta_blocks);
   }
   // the caller's bound on the largest graph decides which of the three size ranges can be populated at all
   if (!no_sort && max_graph_nodes > runs_upto)
-    k_topk_sort<<<(int)G, TOPK_SORT_THREADS, (size_t)TOPK_SMEM_KEYS * 8, (cudaStream_t)stream>>>(score, gptr, kptr, perm, max_pad, runs_upto);
+    TSG_LAUNCH_PDL("topk(sort)", k_topk_sort, (int)G, TOPK_SORT_THREADS, (size_t)TOPK_SMEM_KEYS * 8, (cudaStream_t)stream, score, gptr, kptr, perm, max_pad, runs_upto);
   // graphs larger than the sort's shared-memory budget (and everything when the sort is disabled)
   if (max_graph_nodes > max_pad)
-    k_topk_rank<<<(int)G, TOPK_THREADS, 0, (cudaStream_t)stream>>>(score, gptr, kptr, perm, gkeys, max_pad);
+    TSG_LAUNCH_PDL("topk(rank)", k_topk_rank, (int)G, TOPK_THREADS, 0, (cudaStream_t)stream, score, gptr, kptr, perm, gkeys, max_pad);
   return check_launch("topk");
 }
 
@@ -638,7 +646,7 @@ extern "C" int tsg_gate_score_bwd(const float* dxo, const float* x, const float*
   int lp = 1; while (lp < F4 && lp < 32) lp <<= 1;
   int grid = (int)((num_perm + (GSB_THREADS / lp) - 1) / (GSB_THREADS / lp));
   if (grid > GSB_GRID) grid = GSB_GRID;
-#define TSG_GS(L) k_gate_score_bwd<L><<<grid, GSB_THREADS, 0, st>>>((const float4*)dxo, (const float4*)x, score, perm, dscore, \
+#define TSG_GS(L) TSG_LAUNCH_PDL("gate_score_bwd", k_gate_score_bwd<L>, grid, GSB_THREADS, 0, st, (const float4*)dxo, (const float4*)x, score, perm, dscore, \
                                                                     (float*)workspace, num_perm, F4, dbias_score, ticket)
   switch (lp) {
     case 1: TSG_GS(1); break; case 2: TSG_GS(2); break; case 4: TSG_GS(4); break;

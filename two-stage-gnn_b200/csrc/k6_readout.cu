@@ -22,6 +22,8 @@ template <int VEC, int LPR>
 __global__ void __launch_bounds__(RO_THREADS)
 k_readout_fwd(const float* __restrict__ x, const int64_t* __restrict__ gptr, int G, int F, int mode,
               float* __restrict__ out, int64_t out_stride, int* __restrict__ argmax) {
+  pdl_wait();
+  pdl_launch_dependents();
   constexpr int RPW = 32 / LPR;
   const int lane = threadIdx.x & 31;
   const int sub = lane / LPR, l = lane % LPR;
@@ -123,6 +125,8 @@ __global__ void __launch_bounds__(RO_THREADS)
 k_gate_readout_fwd(const float4* __restrict__ x, const float* __restrict__ score, const int64_t* __restrict__ perm,
                    const int64_t* __restrict__ gptr, int G, int F4, float4* __restrict__ xo,
                    float* __restrict__ out, int64_t out_stride, int* __restrict__ argmax) {
+  pdl_wait();
+  pdl_launch_dependents();
   constexpr int RPW = 32 / LPR;
   const int lane = threadIdx.x & 31;
   const int sub = lane / LPR, l = lane % LPR;
@@ -237,6 +241,8 @@ template <int LPR>
 __global__ void __launch_bounds__(GL_THREADS)
 k_gate_linear(const float4* __restrict__ x, const float* __restrict__ score, const int64_t* __restrict__ perm, int64_t K,
               float4* __restrict__ xo, const float* __restrict__ Wn, float4* __restrict__ xw) {
+  pdl_wait();
+  pdl_launch_dependents();
   constexpr int F4 = LPR, F = 4 * LPR;
   constexpr int RPW = 32 / LPR;
   constexpr int WROWS = RPW * GL_WU;                  // rows per warp: 16 (F = 32), 8 (F = 64)
@@ -292,6 +298,8 @@ template <int VEC, int LPR>
 __global__ void __launch_bounds__(RO_BWD_THREADS)
 k_readout_bwd(const float* __restrict__ dout, int64_t dstride, const int* __restrict__ argmax,
               const int64_t* __restrict__ gptr, int G, int F, int mode, float* __restrict__ dx) {
+  pdl_wait();
+  pdl_launch_dependents();
   constexpr int RPW = 32 / LPR;
   const int lane = threadIdx.x & 31;
   const int sub = lane / LPR, l = lane % LPR;
@@ -348,7 +356,7 @@ using namespace tsg;
 template <int VEC>
 static int launch_fwd(int lpr, int grid, cudaStream_t st, const float* x, const int64_t* gptr, int G,
                       int F, int mode, float* out, int64_t os, int* am) {
-#define TSG_GO(L) k_readout_fwd<VEC, L><<<grid, RO_THREADS, 0, st>>>(x, gptr, G, F, mode, out, os, am)
+#define TSG_GO(L) TSG_LAUNCH_PDL("readout_fwd", k_readout_fwd<VEC, L>, grid, RO_THREADS, 0, st, x, gptr, G, F, mode, out, os, am)
   switch (lpr) {
     case 1: TSG_GO(1); break; case 2: TSG_GO(2); break; case 4: TSG_GO(4); break;
     case 8: TSG_GO(8); break; case 16: TSG_GO(16); break; default: TSG_GO(32); break;
@@ -360,7 +368,7 @@ static int launch_fwd(int lpr, int grid, cudaStream_t st, const float* x, const 
 template <int VEC>
 static int launch_bwd(int lpr, int grid, cudaStream_t st, const float* dout, int64_t ds, const int* am,
                       const int64_t* gptr, int G, int F, int mode, float* dx) {
-#define TSG_GO(L) k_readout_bwd<VEC, L><<<grid, RO_BWD_THREADS, 0, st>>>(dout, ds, am, gptr, G, F, mode, dx)
+#define TSG_GO(L) TSG_LAUNCH_PDL("readout_bwd", k_readout_bwd<VEC, L>, grid, RO_BWD_THREADS, 0, st, dout, ds, am, gptr, G, F, mode, dx)
   switch (lpr) {
     case 1: TSG_GO(1); break; case 2: TSG_GO(2); break; case 4: TSG_GO(4); break;
     case 8: TSG_GO(8); break; case 16: TSG_GO(16); break; default: TSG_GO(32); break;
@@ -410,7 +418,7 @@ extern "C" int tsg_gate_readout_fwd(const float* x, const float* score, const in
   cudaStream_t st = (cudaStream_t)stream;
   const int grid = grid_for(G, RO_THREADS / 32);
   const int F4 = (int)(F / 4);
-#define TSG_GR(L) k_gate_readout_fwd<L><<<grid, RO_THREADS, 0, st>>>((const float4*)x, score, perm, gptr, (int)G, F4, (float4*)xo, out, out_stride, argmax)
+#define TSG_GR(L) TSG_LAUNCH_PDL("gate_readout_fwd", k_gate_readout_fwd<L>, grid, RO_THREADS, 0, st, (const float4*)x, score, perm, gptr, (int)G, F4, (float4*)xo, out, out_stride, argmax)
   switch (pick_lpr(F4)) {
     case 1: TSG_GR(1); break; case 2: TSG_GR(2); break; case 4: TSG_GR(4); break;
     case 8: TSG_GR(8); break; case 16: TSG_GR(16); break; default: TSG_GR(32); break;
@@ -444,10 +452,10 @@ extern "C" int tsg_gate_readout_linear_fwd(const float* x, const float* score, c
     const int64_t grid = (num_rows_out + rows_per_cta - 1) / rows_per_cta;
     TSG_REQUIRE(grid < (int64_t)0x7fffffff, "gate_readout_linear_fwd: too many rows");
     const size_t smem = ((size_t)F * F + (size_t)(GL_THREADS / 32) * wrows * (F + 4)) * sizeof(float);
-    if (F == 32) k_gate_linear<8><<<(int)grid, GL_THREADS, smem, st>>>((const float4*)x, score, perm, num_rows_out, (float4*)xo, w_next, (float4*)xw_next);
-    else k_gate_linear<16><<<(int)grid, GL_THREADS, smem, st>>>((const float4*)x, score, perm, num_rows_out, (float4*)xo, w_next, (float4*)xw_next);
-    int rc = check_launch("gate_readout_linear_fwd");
-    if (rc) return rc;
+    if (F == 32) TSG_LAUNCH_PDL("gate_readout_linear_fwd", k_gate_linear<8>, (int)grid, GL_THREADS, smem, st, (const float4*)x, score, perm,
+                                num_rows_out, (float4*)xo, w_next, (float4*)xw_next);
+    else TSG_LAUNCH_PDL("gate_readout_linear_fwd", k_gate_linear<16>, (int)grid, GL_THREADS, smem, st, (const float4*)x, score, perm,
+                        num_rows_out, (float4*)xo, w_next, (float4*)xw_next);
   }
   return tsg_readout_fwd(xo, gptr, G, F, TSG_READOUT_MAX | TSG_READOUT_MEAN, out, out_stride, argmax, stream);
 }

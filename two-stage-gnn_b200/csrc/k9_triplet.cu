@@ -17,6 +17,8 @@ __global__ void __launch_bounds__(256)
 k_triplet_fwd(const float* __restrict__ emb, const int64_t* __restrict__ trip, int64_t T, int D,
               float margin, float eps, float* __restrict__ dpos, float* __restrict__ dneg,
               float* __restrict__ hinge) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -44,8 +46,11 @@ k_triplet_fwd(const float* __restrict__ emb, const int64_t* __restrict__ trip, i
   }
 }
 
-// deterministic mean of T values with one block
-__global__ void __launch_bounds__(1024) k_mean_1block(const float* __restrict__ v, int64_t T, float* __restrict__ out) {
+// deterministic mean of T values with one block; *seed (if given) receives 1.0, the d(loss) the step's backward starts from
+__global__ void __launch_bounds__(1024)
+k_mean_1block(const float* __restrict__ v, int64_t T, float* __restrict__ out, float* __restrict__ seed) {
+  pdl_wait();
+  pdl_launch_dependents();
   __shared__ float sm[1024];
   float s = 0.f;
   for (int64_t i = threadIdx.x; i < T; i += 1024) s += v[i];
@@ -55,10 +60,15 @@ __global__ void __launch_bounds__(1024) k_mean_1block(const float* __restrict__ 
     if (threadIdx.x < o) sm[threadIdx.x] += sm[threadIdx.x + o];
     __syncthreads();
   }
-  if (threadIdx.x == 0) *out = T > 0 ? sm[0] / (float)T : 0.f;
+  if (threadIdx.x == 0) {
+    *out = T > 0 ? sm[0] / (float)T : 0.f;
+    if (seed) *seed = 1.0f;
+  }
 }
 
 __global__ void k_iota64(int64_t* p, int64_t n) {
+  pdl_wait();
+  pdl_launch_dependents();
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
        i += (int64_t)gridDim.x * blockDim.x) p[i] = i;
 }
@@ -68,6 +78,8 @@ k_triplet_bwd(const float* __restrict__ emb, const int64_t* __restrict__ trip, i
               int D, float margin, float eps, const float* __restrict__ dpos,
               const float* __restrict__ dneg, const float* __restrict__ dloss,
               const int* __restrict__ rowptr, const int* __restrict__ slots, float* __restrict__ demb) {
+  pdl_wait();
+  pdl_launch_dependents();
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -127,18 +139,23 @@ extern "C" size_t tsg_triplet_workspace_bytes(int64_t T, int64_t M, int64_t D) {
   return b + 1024;
 }
 
-extern "C" int tsg_triplet_fwd(const float* emb, const int64_t* trip, int64_t T, int64_t M, int64_t D,
-                               float margin, float eps, float* dpos, float* dneg, float* loss,
-                               void* workspace, size_t workspace_bytes, void* stream) {
+int tsg::triplet_fwd(const float* emb, const int64_t* trip, int64_t T, int64_t M, int64_t D, float margin, float eps,
+                     float* dpos, float* dneg, float* loss, float* dloss_seed, void* workspace, size_t workspace_bytes,
+                     void* stream) {
   TSG_REQUIRE(T >= 0 && M >= 0 && D > 0, "triplet_fwd: bad shape");
   TSG_REQUIRE(loss && (T == 0 || (emb && trip && dpos && dneg)), "triplet_fwd: null pointer");
   if (workspace_bytes < tsg_triplet_workspace_bytes(T, M, D)) { set_error("triplet_fwd: workspace too small"); return TSG_EWORKSPACE; }
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
   float* hinge = ws.take<float>(T + 1);
-  if (T > 0) k_triplet_fwd<<<grid_for(T, 8), 256, 0, st>>>(emb, trip, T, (int)D, margin, eps, dpos, dneg, hinge);
-  k_mean_1block<<<1, 1024, 0, st>>>(hinge, T, loss);
-  return check_launch("triplet_fwd");
+  if (T > 0) TSG_LAUNCH_PDL("triplet_fwd", k_triplet_fwd, grid_for(T, 8), 256, 0, st, emb, trip, T, (int)D, margin, eps, dpos, dneg, hinge);
+  return launch_pdl("triplet_fwd(mean)", k_mean_1block, 1, 1024, 0, st, (const float*)hinge, T, loss, dloss_seed);
+}
+
+extern "C" int tsg_triplet_fwd(const float* emb, const int64_t* trip, int64_t T, int64_t M, int64_t D,
+                               float margin, float eps, float* dpos, float* dneg, float* loss,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+  return triplet_fwd(emb, trip, T, M, D, margin, eps, dpos, dneg, loss, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int tsg_triplet_bwd(const float* emb, const int64_t* trip, int64_t T, int64_t M, int64_t D,
@@ -159,13 +176,13 @@ extern "C" int tsg_triplet_bwd(const float* emb, const int64_t* trip, int64_t T,
   size_t csr_ws_bytes = tsg_csr_build_workspace_bytes(3 * T, M);
   char* csr_ws = ws.take<char>(csr_ws_bytes);
   if (!ws.ok()) { set_error("triplet_bwd: workspace carve failed"); return TSG_EWORKSPACE; }
-  if (T > 0) k_iota64<<<grid_for(3 * T, 256), 256, 0, st>>>(iota, 3 * T);
+  if (T > 0) TSG_LAUNCH_PDL("triplet_bwd(iota)", k_iota64, grid_for(3 * T, 256), 256, 0, st, iota, 3 * T);
   // inverted index: "edge" slot -> embedding row, grouped by embedding row in slot order
   int rc = tsg_csr_build(iota, trip, nullptr, 3 * T, nullptr, M, TSG_CSR_RAW, rowptr, slots, val, nullptr,
                          nullptr, nullptr, nullptr, nullptr, csr_ws, csr_ws_bytes, stream);
   if (rc) return rc;
-  k_triplet_bwd<<<grid_for(M, 8), 256, 0, st>>>(emb, trip, T, M, (int)D, margin, eps, dpos, dneg, dloss, rowptr, slots, demb);
-  return check_launch("triplet_bwd");
+  return launch_pdl("triplet_bwd", k_triplet_bwd, grid_for(M, 8), 256, 0, st, emb, trip, T, M, (int)D, margin, eps, dpos, dneg, dloss,
+                    (const int*)rowptr, (const int*)slots, demb);
 }
 
 extern "C" int tsg_pairdist_matrix(const float* emb, int64_t M, int64_t D, float eps, float* dist, void* stream) {

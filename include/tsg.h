@@ -274,6 +274,23 @@ size_t tsg_linear_bwd_weight_workspace_bytes(int64_t in_feat, int64_t out_feat);
 int tsg_linear_bwd_weight(const float* X, const float* dY, float* dW /*nullable*/,
                           float* db /*nullable*/, int64_t num_rows, int64_t in_feat, int64_t out_feat,
                           void* workspace, size_t workspace_bytes, void* stream);
+/* SAGPool level boundary of the encoder backward (levels 2 and 1) in one pass over the rows:
+ *   dxg = readout_bwd(dz) + dxw . W^T and dW = x^T . dxw,
+ * with dxw [N,H] (= A_hat^T dhm of conv_l), x [N,H] (conv_l's input), W [H,H] (conv_l's weight, read as
+ * tsg_linear_fwd(..., w_transposed=1) reads it), dz [G, >= 2H] (row stride dz_stride; [max || mean] gradient of the
+ * readout below) with argmax [G,H] and graph_ptr [G+1] of those N rows.  Bit-identical to tsg_linear_fwd(dxw, W,
+ * NULL, dxg, N, H, H, 1, 0) -> tsg_readout_bwd(dz, dz_stride, argmax, graph_ptr, G, N, H, MAX|MEAN|ACCUM, dxg) and
+ * tsg_linear_bwd_weight(x, dxw, dW, NULL, N, H, H):
+ *   dX[r,m]  = (sum_k dxw[r,k] W[m,k], one fmaf per term, k ascending from 0.f) + 0.f
+ *   dxg[r,m] = (dz[g,H+m] / (float)max(n_g,1) + (argmax[g,m] == r ? dz[g,m] : 0.f)) + dX[r,m]   (g: graph of row r;
+ *              a row outside graph_ptr's graphs gets dX[r,m])
+ *   dW       = tsg_linear_bwd_weight's dense partition: 2 x 148 CTAs of ceil(N / 296) rows, 128-row tiles from each
+ *              CTA's first row, row i of a tile to group i mod (256 / (H/4)^2), groups then CTAs summed in index order.
+ * hidden % 4 == 0 and 8 <= hidden <= 64; dxw, x, dxg, dz, argmax 16-byte aligned; dz_stride % 4 == 0;
+ * workspace >= tsg_linear_bwd_weight_workspace_bytes(hidden, hidden).  Two kernels (the pass + the partials' fold). */
+int tsg_sag_boundary_bwd(const float* dxw, const float* x, const float* W, const float* dz, int64_t dz_stride,
+                         const int32_t* argmax, const int64_t* graph_ptr, int64_t num_graphs, int64_t num_rows,
+                         int64_t hidden, float* dxg, float* dW, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Dense wire-format adapters (dense directories)

@@ -331,6 +331,15 @@ static int sag_bwd(const tsg_sag_shape* sh, const SagInput& in, const int64_t* l
   if (arena_bytes < a.total) { set_error("sag_encoder_bwd: arena too small (%zu < %zu)", arena_bytes, a.total); return TSG_EWORKSPACE; }
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t G = sh->num_graphs, H = sh->hidden;
+  // level l > 0's boundary in one pass (tsg_sag_boundary_bwd): conv_l's input and weight gradients and level l-1's
+  // readout gradient, in the widths and alignments where the dense K3 kernels it reproduces would run
+  static const bool no_dense = getenv("TSG_LIN_NODENSE") != nullptr;
+  auto boundary = [&](int l) {
+    if (l == 0) return false;
+    const uintptr_t al = (uintptr_t)a.dxw | (uintptr_t)a.dxg | (uintptr_t)a.lv[l - 1].xg | (uintptr_t)a.lv[l - 1].argmax |
+                         (uintptr_t)dz;
+    return H % 4 == 0 && H >= 8 && H <= 64 && (al & 15) == 0 && !no_dense && !sag_unfused_env();
+  };
   for (int l = 2; l >= 0; --l) {
     LevelBuf& b = a.lv[l];
     const int64_t n = sh->n[l], k = sh->n[l + 1], fin = l == 0 ? sh->in_feat : H;
@@ -339,9 +348,11 @@ static int sag_bwd(const tsg_sag_shape* sh, const SagInput& in, const int64_t* l
     const float* xin = l == 0 ? in.x : a.lv[l - 1].xg;
     const int64_t* ptr_n = level_ptr + (size_t)(l + 1) * (G + 1);
     // d(x_{l+1}) = readout backward (+ the next level's input gradient)
-    //   (the next level's linear backward already wrote its dX into a.dxg: accumulate in place)
-    TSG_TRY(tsg_readout_bwd(dz, 2 * H, b.argmax, ptr_n, G, k, H,
-                            TSG_READOUT_MAX | TSG_READOUT_MEAN | (l < 2 ? TSG_READOUT_ACCUM : 0), a.dxg, stream));
+    //   (the next level's linear backward already wrote its dX into a.dxg: accumulate in place; its boundary pass
+    //   already added this readout term)
+    if (l == 2 || !boundary(l + 1))
+      TSG_TRY(tsg_readout_bwd(dz, 2 * H, b.argmax, ptr_n, G, k, H,
+                              TSG_READOUT_MAX | TSG_READOUT_MEAN | (l < 2 ? TSG_READOUT_ACCUM : 0), a.dxg, stream));
     // fused level backward (k_sag_conv_bwd_v4): dh is never materialised and h is read once for mask, dbias and dws
     const bool fused = H % 4 == 0 && H <= 512 && (((uintptr_t)ws) & 15) == 0 && !sag_unfused_env();
     // score layer: score = A_hat (h ws) + bs; dscore from the gate, its sum = dbs
@@ -361,9 +372,14 @@ static int sag_bwd(const tsg_sag_shape* sh, const SagInput& in, const int64_t* l
       TSG_TRY(tsg_relu_bwd_colsum_rank1(a.dh, b.h, a.dsw, ws, a.dhm, dbias, n, H, a.scratch, a.scratch_bytes, stream));
     }
     TSG_TRY(tsg_spmm(b.t_rowptr, b.t_colidx, b.t_val, a.dhm, nullptr, a.dxw, n, H, 0, stream));
-    if (l > 0) TSG_TRY(tsg_linear_fwd(a.dxw, W, nullptr, a.dxg, n, H, fin, 1, 0, stream));   // d(x_l), k_{l-1} = n rows
-    if (l == 0 && in.label) TSG_TRY(tsg_embed_bwd_weight(in.label, a.dxw, dW, n, fin, H, a.scratch, a.scratch_bytes, stream));
-    else TSG_TRY(tsg_linear_bwd_weight(xin, a.dxw, dW, nullptr, n, fin, H, a.scratch, a.scratch_bytes, stream));
+    if (boundary(l)) {                 // d(x_l) + level l-1's readout gradient, and dW_l; k_{l-1} = n rows
+      TSG_TRY(tsg_sag_boundary_bwd(a.dxw, xin, W, dz, 2 * H, a.lv[l - 1].argmax, level_ptr + (size_t)l * (G + 1), G, n, H,
+                                   a.dxg, dW, a.scratch, a.scratch_bytes, stream));
+    } else {
+      if (l > 0) TSG_TRY(tsg_linear_fwd(a.dxw, W, nullptr, a.dxg, n, H, fin, 1, 0, stream));   // d(x_l), k_{l-1} = n rows
+      if (l == 0 && in.label) TSG_TRY(tsg_embed_bwd_weight(in.label, a.dxw, dW, n, fin, H, a.scratch, a.scratch_bytes, stream));
+      else TSG_TRY(tsg_linear_bwd_weight(xin, a.dxw, dW, nullptr, n, fin, H, a.scratch, a.scratch_bytes, stream));
+    }
   }
   return check_launch("sag_encoder_bwd");
 }

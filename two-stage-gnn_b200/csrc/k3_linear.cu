@@ -624,6 +624,195 @@ k_linear_bwd_weight_dense(const float* __restrict__ X, const float* __restrict__
 }
 
 // ------------------------------------------------------------------------------------------
+// SAGPool level boundary of the encoder backward (K10 sag_bwd, levels 2 and 1): from dxw = A_hat^T dhm [N, H],
+//   dxg = readout_bwd_{l-1}(dz) + dxw . W^T     (k_linear_fwd_dense, then k_readout_bwd MAX|MEAN|ACCUM)
+//   part = per-CTA partials of x^T . dxw        (k_linear_bwd_weight_dense)
+// in one pass: each LBWD_ROWS tile of dxw and x is staged once, dxg is written once.  Warps 0-7 accumulate dW over
+// k_linear_bwd_weight_dense's exact partition (LBW_GRID CTAs, rows_per_cta, tiles from r_begin, row i of a tile to
+// group i mod groups); warps 8-15 compute dX for the same tile with k_linear_fwd_dense's per-output chain (acc = 0,
+// fmaf over k ascending, then + 0.f) and add the readout term as k_readout_bwd does: (gs + (am == r ? gm : 0)) + dX.
+// Rows are staged at pitch H + 4 so the dX warps' float4 reads of four different rows hit different banks.
+// ------------------------------------------------------------------------------------------
+constexpr int SBB_THREADS = 512;
+
+// largest g in [-1, G] with gptr[g] <= r (gptr[-1] taken as -inf): the graph of row r when 0 <= g < G
+__device__ __forceinline__ int graph_search(const int64_t* __restrict__ gptr, int G, int64_t r) {
+  int lo = -1, hi = G;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(gptr + mid) <= r) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// shared memory of k_sag_boundary_bwd<H>: W, two double-buffered row tiles, the tile's graph table, the dW accumulators
+__host__ __device__ constexpr size_t sbb_smem_bytes(int H) {
+  return ((size_t)H * H + 4 * LBWD_ROWS * (H + 4)) * sizeof(float) + 2 * LBWD_ROWS * sizeof(int) + 4 * 256 * sizeof(float4);
+}
+
+// two CTAs per SM up to H = 32; from H = 36 the 64 registers that allows spill, and from H = 44 two CTAs' shared
+// memory does not fit an SM anyway
+template <int H>
+__global__ void __launch_bounds__(SBB_THREADS, H <= 32 ? 2 : 1)
+k_sag_boundary_bwd(const float* __restrict__ dxw, const float* __restrict__ X, const float* __restrict__ W,
+                   const float* __restrict__ dz, int64_t dz_stride, const int* __restrict__ argmax,
+                   const int64_t* __restrict__ gptr, int G, int N, float* __restrict__ dxg, float* __restrict__ part) {
+  pdl_wait();
+  pdl_launch_dependents();
+  constexpr int P = H + 4, CG = H / 4, NB = CG * CG, GROUPS = 256 / NB;
+  extern __shared__ __align__(16) float smem[];
+  float* Ws = smem;                                   // [H][H], Ws[k][m] = W[m][k]
+  float* Xs = Ws + H * H;                             // 2 x [ROWS][P]
+  float* Ys = Xs + 2 * LBWD_ROWS * P;                 // 2 x [ROWS][P] (dxw)
+  int* rg = reinterpret_cast<int*>(Ys + 2 * LBWD_ROWS * P);    // [ROWS] graph of the tile's row (-1: none)
+  float* rn = reinterpret_cast<float*>(rg + LBWD_ROWS);        // [ROWS] (float)max(n_g, 1)
+  float4* accs = reinterpret_cast<float4*>(rn + LBWD_ROWS);    // [4][256] dW accumulators
+  const int tid = threadIdx.x;
+  const int rows_per_cta = (N + gridDim.x - 1) / gridDim.x;
+  const int r_begin = blockIdx.x * rows_per_cta;
+  const int r_end = min(N, r_begin + rows_per_cta);
+  auto stage = [&](int buf, int r0) {
+    const int rows = max(0, min(LBWD_ROWS, r_end - r0));
+    float* xd = Xs + buf * LBWD_ROWS * P; float* yd = Ys + buf * LBWD_ROWS * P;
+    for (int i = tid; i < rows * CG; i += SBB_THREADS) {
+      const int r = i / CG, c = (i - r * CG) * 4;
+      cp_async16(xd + r * P + c, X + (size_t)(r0 + r) * H + c);
+      cp_async16(yd + r * P + c, dxw + (size_t)(r0 + r) * H + c);
+    }
+    cp_async_commit();
+  };
+  int buf = 0;
+  if (r_begin < r_end) stage(0, r_begin);
+  for (int i = tid; i < H * H; i += SBB_THREADS) {
+    const int k = i / H, m = i - k * H;
+    Ws[i] = W[(size_t)m * H + k];
+  }
+  // threads 256 + t look up the graph of row t of every tile, walking forward from the previous tile's row
+  const int lt = tid - 256;
+  const bool looker = lt >= 0 && lt < LBWD_ROWS;
+  int gw = (looker && r_begin + lt < r_end) ? graph_search(gptr, G, r_begin + lt) : -1;
+  // dW: thread tid < 256 owns the 4x4 block (kb, mb) of row group grp; its accumulators stay in shared memory
+  // between tiles, so they are not live in registers while the same warps' code path for dX runs
+  const int blk = tid % NB, grp = tid / NB;
+  const int kb = blk / CG, mb = blk - kb * CG;
+  const bool dw_thread = tid < 256 && grp < GROUPS;
+  if (dw_thread)
+#pragma unroll
+    for (int a = 0; a < 4; ++a) accs[a * 256 + tid] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int r0 = r_begin; r0 < r_end; r0 += LBWD_ROWS) {
+    const int rows = min(LBWD_ROWS, r_end - r0);
+    if (looker) {
+      int g = -1; float nf = 1.f;
+      if (lt < rows) {
+        const int64_t r = r0 + lt;
+        while (gw < G && __ldg(gptr + gw + 1) <= r) ++gw;
+        if (gw >= 0 && gw < G) {
+          const int n = (int)(__ldg(gptr + gw + 1) - __ldg(gptr + gw));
+          g = gw; nf = (float)(n > 0 ? n : 1);
+        }
+      }
+      rg[lt] = g; rn[lt] = nf;
+    }
+    if (r0 + LBWD_ROWS < r_end) { stage(buf ^ 1, r0 + LBWD_ROWS); cp_async_wait<1>(); } else { cp_async_wait<0>(); }
+    __syncthreads();
+    const float* xt = Xs + buf * LBWD_ROWS * P;
+    const float* yt = Ys + buf * LBWD_ROWS * P;
+    if (tid < 256) {
+      if (dw_thread) {
+        float acc[4][4];
+#pragma unroll
+        for (int a = 0; a < 4; ++a) {
+          const float4 v = accs[a * 256 + tid];
+          acc[a][0] = v.x; acc[a][1] = v.y; acc[a][2] = v.z; acc[a][3] = v.w;
+        }
+        const float* xb = xt + kb * 4;
+        const float* yb = yt + mb * 4;
+        for (int r = grp; r < rows; r += GROUPS) {
+          const float4 a = *reinterpret_cast<const float4*>(xb + r * P);
+          const float4 b = *reinterpret_cast<const float4*>(yb + r * P);
+          acc[0][0] = fmaf(a.x, b.x, acc[0][0]); acc[0][1] = fmaf(a.x, b.y, acc[0][1]); acc[0][2] = fmaf(a.x, b.z, acc[0][2]); acc[0][3] = fmaf(a.x, b.w, acc[0][3]);
+          acc[1][0] = fmaf(a.y, b.x, acc[1][0]); acc[1][1] = fmaf(a.y, b.y, acc[1][1]); acc[1][2] = fmaf(a.y, b.z, acc[1][2]); acc[1][3] = fmaf(a.y, b.w, acc[1][3]);
+          acc[2][0] = fmaf(a.z, b.x, acc[2][0]); acc[2][1] = fmaf(a.z, b.y, acc[2][1]); acc[2][2] = fmaf(a.z, b.z, acc[2][2]); acc[2][3] = fmaf(a.z, b.w, acc[2][3]);
+          acc[3][0] = fmaf(a.w, b.x, acc[3][0]); acc[3][1] = fmaf(a.w, b.y, acc[3][1]); acc[3][2] = fmaf(a.w, b.z, acc[3][2]); acc[3][3] = fmaf(a.w, b.w, acc[3][3]);
+        }
+#pragma unroll
+        for (int a = 0; a < 4; ++a) accs[a * 256 + tid] = make_float4(acc[a][0], acc[a][1], acc[a][2], acc[a][3]);
+      }
+    } else {
+      // unit u: columns 4 cg .. 4 cg + 3 of rows q, q + 32, q + 64, q + 96
+      for (int u = tid - 256; u < 32 * CG; u += SBB_THREADS - 256) {
+        const int cg = u % CG, q = u / CG;
+        float d[4][4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+#pragma unroll
+          for (int c = 0; c < 4; ++c) d[j][c] = 0.f;
+#pragma unroll 1
+        for (int k = 0; k < H; k += 4) {
+          float4 w[4];
+#pragma unroll
+          for (int s = 0; s < 4; ++s) w[s] = *reinterpret_cast<const float4*>(Ws + (k + s) * H + cg * 4);
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const float4 a = *reinterpret_cast<const float4*>(yt + (q + 32 * j) * P + k);
+            d[j][0] = fmaf(a.x, w[0].x, d[j][0]); d[j][1] = fmaf(a.x, w[0].y, d[j][1]);
+            d[j][2] = fmaf(a.x, w[0].z, d[j][2]); d[j][3] = fmaf(a.x, w[0].w, d[j][3]);
+            d[j][0] = fmaf(a.y, w[1].x, d[j][0]); d[j][1] = fmaf(a.y, w[1].y, d[j][1]);
+            d[j][2] = fmaf(a.y, w[1].z, d[j][2]); d[j][3] = fmaf(a.y, w[1].w, d[j][3]);
+            d[j][0] = fmaf(a.z, w[2].x, d[j][0]); d[j][1] = fmaf(a.z, w[2].y, d[j][1]);
+            d[j][2] = fmaf(a.z, w[2].z, d[j][2]); d[j][3] = fmaf(a.z, w[2].w, d[j][3]);
+            d[j][0] = fmaf(a.w, w[3].x, d[j][0]); d[j][1] = fmaf(a.w, w[3].y, d[j][1]);
+            d[j][2] = fmaf(a.w, w[3].z, d[j][2]); d[j][3] = fmaf(a.w, w[3].w, d[j][3]);
+          }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const int r = q + 32 * j;
+          if (r >= rows) continue;
+          float o[4];
+#pragma unroll
+          for (int c = 0; c < 4; ++c) o[c] = d[j][c] + 0.f;     // the bias-less add of k_linear_fwd_dense (-0 -> +0)
+          const int g = rg[r];
+          if (g >= 0) {
+            const float* dzg = dz + (int64_t)g * dz_stride + cg * 4;
+            const float4 gm = __ldg(reinterpret_cast<const float4*>(dzg));
+            const float4 gd = __ldg(reinterpret_cast<const float4*>(dzg + H));
+            const int4 am = __ldg(reinterpret_cast<const int4*>(argmax + (int64_t)g * H + cg * 4));
+            const float nf = rn[r];
+            const int row = r0 + r;
+            o[0] = (gd.x / nf + (am.x == row ? gm.x : 0.f)) + o[0];
+            o[1] = (gd.y / nf + (am.y == row ? gm.y : 0.f)) + o[1];
+            o[2] = (gd.z / nf + (am.z == row ? gm.z : 0.f)) + o[2];
+            o[3] = (gd.w / nf + (am.w == row ? gm.w : 0.f)) + o[3];
+          }
+          *reinterpret_cast<float4*>(dxg + (size_t)(r0 + r) * H + cg * 4) = make_float4(o[0], o[1], o[2], o[3]);
+        }
+      }
+    }
+    __syncthreads();
+    buf ^= 1;
+  }
+  // combine the row groups in index order through shared memory (reuse the staging buffers)
+  float* red = Xs;                                    // [GROUPS][H * H]
+  if (dw_thread) {
+#pragma unroll
+    for (int a = 0; a < 4; ++a) {
+      const float4 v = accs[a * 256 + tid];
+      const float vals[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int b = 0; b < 4; ++b) red[grp * H * H + (kb * 4 + a) * H + mb * 4 + b] = vals[b];
+    }
+  }
+  __syncthreads();
+  float* mypart = part + (size_t)blockIdx.x * H * H;
+  for (int i = tid; i < H * H; i += SBB_THREADS) {
+    float t = red[i];
+    for (int g2 = 1; g2 < GROUPS; ++g2) t += red[g2 * H * H + i];
+    mypart[i] = t;
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // Narrow outputs (M <= 4: SAGPool's score layer is F -> 1): GEMV-shaped, pure streaming of X.
 //   fwd : LPR = K/4 lanes read one row as float4s, M dot products, width-LPR shuffle reduction.
 //   dW  : the same lanes keep acc[4][M] for their 4 feature rows over the CTA's row range; row groups
@@ -928,6 +1117,36 @@ extern "C" int tsg_linear_bwd_weight(const float* X, const float* dY, float* dW,
     if (rc) return rc;
   }
   return check_launch("linear_bwd_weight");
+}
+
+extern "C" int tsg_sag_boundary_bwd(const float* dxw, const float* x, const float* W, const float* dz, int64_t dz_stride,
+                                    const int32_t* argmax, const int64_t* graph_ptr, int64_t G, int64_t N, int64_t H,
+                                    float* dxg, float* dW, void* workspace, size_t workspace_bytes, void* stream) {
+  TSG_REQUIRE(H % 4 == 0 && H >= 8 && H <= 64, "sag_boundary_bwd: hidden %lld is not a multiple of 4 in [8, 64]", (long long)H);
+  TSG_REQUIRE(N >= 0 && G >= 0 && N < (int64_t)0x7fffffff && G < (int64_t)0x7fffffff, "sag_boundary_bwd: bad shape");
+  TSG_REQUIRE(dz_stride >= 2 * H && dz_stride % 4 == 0, "sag_boundary_bwd: dz stride %lld must be >= 2 * hidden and a multiple of 4",
+              (long long)dz_stride);
+  TSG_REQUIRE(W && dW && graph_ptr && (N == 0 || (dxw && x && dxg)) && (G == 0 || (dz && argmax)), "sag_boundary_bwd: null pointer");
+  TSG_REQUIRE(((((uintptr_t)dxw) | ((uintptr_t)x) | ((uintptr_t)dxg) | ((uintptr_t)dz) | ((uintptr_t)argmax)) & 15) == 0,
+              "sag_boundary_bwd: dxw, x, dxg, dz and argmax must be 16-byte aligned");
+  if (workspace_bytes < ws_bytes((size_t)LBW_GRID * H * H, 4)) { set_error("sag_boundary_bwd: workspace too small"); return TSG_EWORKSPACE; }
+  cudaStream_t st = (cudaStream_t)stream;
+  float* part = (float*)workspace;
+  const size_t smem = sbb_smem_bytes((int)H);
+  int rc;
+#define TSG_GO(H_)                                                                                                        \
+  case H_:                                                                                                                \
+    rc = set_smem(k_sag_boundary_bwd<H_>, smem, "sag_boundary_bwd"); if (rc) return rc;                                  \
+    TSG_LAUNCH_PDL("sag_boundary_bwd", k_sag_boundary_bwd<H_>, LBW_GRID, SBB_THREADS, smem, st, dxw, x, W, dz, dz_stride, \
+                   argmax, graph_ptr, (int)G, (int)N, dxg, part);                                                         \
+    break;
+  switch (H) {
+    TSG_GO(8) TSG_GO(12) TSG_GO(16) TSG_GO(20) TSG_GO(24) TSG_GO(28) TSG_GO(32) TSG_GO(36)
+    TSG_GO(40) TSG_GO(44) TSG_GO(48) TSG_GO(52) TSG_GO(56) TSG_GO(60) TSG_GO(64)
+  }
+#undef TSG_GO
+  rc = launch_partial_sum_final(part, dW, (int)(H * H), nullptr, LBW_GRID, (int)(H * H), st); if (rc) return rc;
+  return check_launch("sag_boundary_bwd");
 }
 
 

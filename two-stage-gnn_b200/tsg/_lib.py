@@ -47,6 +47,7 @@ _PROTOTYPES = {
     "tsg_softmax_bwd": (I, [P, P, P, I64, I64, P]),
     "tsg_linear_bwd_weight_workspace_bytes": (SZ, [I64, I64]),
     "tsg_linear_bwd_weight": (I, [P, P, P, P, I64, I64, I64, P, SZ, P]),
+    "tsg_sag_boundary_bwd": (I, [P, P, P, P, I64, P, P, I64, I64, I64, P, P, P, SZ, P]),
     "tsg_dense_to_coo_workspace_bytes": (SZ, [I64, I64]),
     "tsg_dense_to_coo": (I, [P, I64, I64, I64, P, P, P, P, P, P, P, I64, P, P, SZ, P]),
     "tsg_nodebn_fwd": (I, [P, P, P, P, I64, I64, I64, P]),
@@ -150,8 +151,8 @@ KERNELS_PER_CALL = {
     "tsg_pack_batch": 1, "tsg_csr_build": 12, "tsg_edge_ptr": 1, "tsg_csr_build_graphs": 5, "tsg_csr_build_graphs_local": 5, "tsg_embed_fwd": 1, "tsg_embed_bwd_weight": 2, "tsg_spmm": 1, "tsg_spmm_tiled": 1, "tsg_relu_bwd_colsum": 1, "tsg_topk_sizes": 3, "tsg_topk": 2,
     "tsg_batch_to_ptr": 1, "tsg_filter_adj": 7, "tsg_gate_gather_fwd": 1, "tsg_gate_gather_bwd": 1,
     "tsg_readout_fwd": 1, "tsg_readout_bwd": 1, "tsg_triplet_fwd": 2, "tsg_triplet_bwd": 9,
-    "tsg_pairdist_matrix": 1, "tsg_linear_fwd": 1, "tsg_dense_epilogue_bwd": 1, "tsg_linear_bwd_weight": 2,
-    "tsg_eigpool_build": 1, "tsg_coarsen_edges": 6, "tsg_inv_perm": 1, "tsg_csr_filter": 5, "tsg_sag_encoder_fwd": 38, "tsg_sag_encoder_bwd": 26, "tsg_sag_encoder_fwd_compact": 36, "tsg_sag_encoder_embed_compact": 3, "tsg_sag_triplet_step_compact": 76, "tsg_sag_step_fwd_compact": 37, "tsg_sag_step_bwd_compact": 29, "tsg_sag_nll_step_compact": 68, "tsg_sag_classify_compact": 6, "tsg_linkpred_loss_fwd": 3, "tsg_linkpred_loss_bwd": 1, "tsg_spmm_label_dot": 1, "tsg_gate_readout_fwd": 1, "tsg_gate_readout_linear_fwd": 2, "tsg_sag_encoder_bwd_compact": 26, "tsg_relu_bwd_colsum_rank1": 1, "tsg_sag_conv_bwd_fused": 1, "tsg_gate_score_bwd": 1, "tsg_spmm_dot": 1, "tsg_pack_batch_compact": 1, "tsg_pack_dense_batch": 1, "tsg_pack_eigen_batch": 1, "tsg_seg_contract": 1, "tsg_seg_linear": 1, "tsg_seg_linear_tc": 1, "tsg_linear_tc": 2, "tsg_gat_fwd": 2, "tsg_gat_bwd": 2, "tsg_dense_to_coo": 6, "tsg_nodebn_fwd": 1, "tsg_nodebn_bwd": 1,
+    "tsg_pairdist_matrix": 1, "tsg_linear_fwd": 1, "tsg_dense_epilogue_bwd": 1, "tsg_linear_bwd_weight": 2, "tsg_sag_boundary_bwd": 2,
+    "tsg_eigpool_build": 1, "tsg_coarsen_edges": 6, "tsg_inv_perm": 1, "tsg_csr_filter": 5, "tsg_sag_encoder_fwd": 38, "tsg_sag_encoder_bwd": 22, "tsg_sag_encoder_fwd_compact": 36, "tsg_sag_encoder_embed_compact": 3, "tsg_sag_triplet_step_compact": 72, "tsg_sag_step_fwd_compact": 37, "tsg_sag_step_bwd_compact": 25, "tsg_sag_nll_step_compact": 64, "tsg_sag_classify_compact": 6, "tsg_linkpred_loss_fwd": 3, "tsg_linkpred_loss_bwd": 1, "tsg_spmm_label_dot": 1, "tsg_gate_readout_fwd": 1, "tsg_gate_readout_linear_fwd": 2, "tsg_sag_encoder_bwd_compact": 22, "tsg_relu_bwd_colsum_rank1": 1, "tsg_sag_conv_bwd_fused": 1, "tsg_gate_score_bwd": 1, "tsg_spmm_dot": 1, "tsg_pack_batch_compact": 1, "tsg_pack_dense_batch": 1, "tsg_pack_eigen_batch": 1, "tsg_seg_contract": 1, "tsg_seg_linear": 1, "tsg_seg_linear_tc": 1, "tsg_linear_tc": 2, "tsg_gat_fwd": 2, "tsg_gat_bwd": 2, "tsg_dense_to_coo": 6, "tsg_nodebn_fwd": 1, "tsg_nodebn_bwd": 1,
 }
 launch_calls = 0        # libtsg entry points called since import
 kernel_launches = 0     # kernels enqueued by them

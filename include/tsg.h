@@ -533,6 +533,52 @@ int tsg_linkpred_loss_bwd(const float* S, const int64_t* graph_ptr, const int32_
                           float* dS, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * K16  prediction head + cross-entropy of the dense encoders' supervised settings (original and 2stg+)
+ *   replaces the chain of nn.Linear / ReLU layers over the graph readouts r [G, in_dim] and F.cross_entropy of
+ *   Code/sage+gat+diffpool/train.py:85-152 (and the stage-2 loop of train_triplet_pre_train.py:249-256).
+ *   Layer l maps in_l (in_dim for l = 0, else out_dim[l-1]) to out_dim[l] with weight [out_l, in_l] (nn.Linear layout)
+ *   and an optional bias; bit l of relu_mask puts a ReLU after it.  Every unit is ONE fmaf chain over the input index
+ *   ascending from 0.f, then + bias (the chain of tsg_linear_fwd(..., w_transposed = 1, flags = 0)'s row kernels), so a
+ *   row's logits do not depend on the other rows of the batch or on num_rows.  num_layers = 0: the logits are r.
+ *   C = the last width.  softmax_first: the loss is the cross-entropy of softmax(logits) (the reference's 2stg+ stage 2).
+ *   Limits: 0 <= num_layers <= 8, every width in [1, 256]; TSG_EINVAL otherwise (and 0 from the workspace queries,
+ *   which are pure host code).  A label outside [0, C) is read clamped and ORs TSG_SAG_LABEL_RANGE into *status
+ *   (nullable: not reported).  No floating-point atomics: every sum has a fixed order.
+ *   tsg_pred_ce_fwd: *loss = mean over the rows of logsumexp(q) - q_y (q = logits, or their softmax), summed in a fixed
+ *     order; logits_out (nullable) [G, C]; saves the activations in the workspace for tsg_pred_ce_bwd (same workspace,
+ *     same arguments).
+ *   tsg_pred_ce_bwd: from *dloss (nullable => 1): dr [G, in_dim] (nullable), dweight[l] [out_l, in_l] and dbias[l]
+ *     [out_l] (nullable per layer) WRITTEN, not accumulated; the parameter gradients are K3's fixed-order reductions
+ *     (tsg_linear_bwd_weight, tsg_relu_bwd_colsum) over the per-row deltas.
+ *   tsg_pred_classify: the eval-mode forward: pred int64 [G] = first-index argmax of the logits (out.max(dim=1)[1]);
+ *     logits_out (nullable); with labels y, *correct (int64) = #(pred == y) and *ce_sum = the fixed-order sum of the
+ *     per-row loss (softmax_first included); both nullable.
+ * ------------------------------------------------------------------------------------------ */
+#define TSG_PRED_MAX_LAYERS 8
+#define TSG_PRED_MAX_WIDTH 256
+typedef struct tsg_pred_head {
+  int64_t num_layers;
+  int64_t in_dim;
+  int64_t out_dim[TSG_PRED_MAX_LAYERS];
+  int64_t relu_mask;
+  int64_t softmax_first;
+  const float* weight[TSG_PRED_MAX_LAYERS];
+  const float* bias[TSG_PRED_MAX_LAYERS];      /* nullable */
+} tsg_pred_head;
+size_t tsg_pred_ce_workspace_bytes(const tsg_pred_head* head, int64_t num_rows);
+int tsg_pred_ce_fwd(const tsg_pred_head* head, const float* r, const int64_t* y, int64_t num_rows, float* loss,
+                    float* logits_out /*nullable*/, int32_t* status /*nullable*/, void* workspace, size_t workspace_bytes,
+                    void* stream);
+int tsg_pred_ce_bwd(const tsg_pred_head* head, const float* r, const int64_t* y, int64_t num_rows,
+                    const float* dloss /*nullable*/, float* dr /*nullable*/, float* const* dweight,
+                    float* const* dbias, void* workspace, size_t workspace_bytes, void* stream);
+size_t tsg_pred_classify_workspace_bytes(const tsg_pred_head* head, int64_t num_rows);
+int tsg_pred_classify(const tsg_pred_head* head, const float* r, const int64_t* y /*nullable*/, int64_t num_rows,
+                      int64_t* pred, float* logits_out /*nullable*/, int64_t* correct /*nullable*/,
+                      float* ce_sum /*nullable*/, int32_t* status /*nullable*/, void* workspace, size_t workspace_bytes,
+                      void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * H1  TU-format dataset loader -> packed corpus arrays (SURVEY 8f n3).  HOST pointers throughout.
  *   replaces `read_graphfile` (Code/sage+gat+diffpool/load_data.py:12-126, Code/eigengcn/load_data.py) in
  *   TSG_TU_NETWORKX mode (node set / order / labels exactly as the networkx graphs the reference builds) and

@@ -304,6 +304,41 @@ static inline bool fused_tail_ok(int64_t nb, int64_t total) {
   return !off && nb * total <= 2048;
 }
 
+// A graph label read for a C-class head: outside [0, C) it is clamped for the read and sets TSG_SAG_LABEL_RANGE in `bad`
+// (the caller ORs that into its status word).
+__device__ __forceinline__ int clamp_label(int64_t y, int C, int& bad) {
+  if (y < 0 || y >= C) { bad = TSG_SAG_LABEL_RANGE; return y < 0 ? 0 : C - 1; }
+  return (int)y;
+}
+
+// Fixed-order totals over n rows on one CTA: thread t adds rows t, t + 1024, ... in order, then a fixed tree.
+// sum_out = (sum v) / div; count_out = sum hit (int64).  Either output may be NULL.  (The losses and evaluation totals of
+// K14 and K16.)
+constexpr int SUM_THREADS = 1024;
+static __global__ void __launch_bounds__(SUM_THREADS)
+k_sum_fixed(const float* __restrict__ v, const int* __restrict__ hit, int n, float div, float* sum_out, int64_t* count_out) {
+  pdl_wait();
+  pdl_launch_dependents();
+  __shared__ float sv[SUM_THREADS];
+  __shared__ long long sc[SUM_THREADS];
+  float s = 0.f;
+  long long c = 0;
+  for (int i = threadIdx.x; i < n; i += SUM_THREADS) {
+    if (sum_out) s += v[i];
+    if (count_out) c += hit[i];
+  }
+  sv[threadIdx.x] = s; sc[threadIdx.x] = c;
+  __syncthreads();
+  for (int o = SUM_THREADS / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) { sv[threadIdx.x] += sv[threadIdx.x + o]; sc[threadIdx.x] += sc[threadIdx.x + o]; }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    if (sum_out) *sum_out = sv[0] / div;
+    if (count_out) *count_out = sc[0];
+  }
+}
+
 unsigned* ticket_next();      // api.cu: a zeroed device counter from a per-device pool (nullptr if the pool cannot be made)
 
 // k9_triplet.cu: tsg_triplet_fwd that also stores 1.0 to *dloss_seed (if given) from its last kernel

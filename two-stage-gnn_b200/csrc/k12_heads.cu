@@ -25,11 +25,6 @@ namespace tsg {
 constexpr int KNN_MAXK = 32;
 constexpr int KNN_MAXC = 1024;
 
-__device__ __forceinline__ int clamp_label(int64_t y, int C, int& bad) {
-  if (y < 0 || y >= C) { bad = TSG_SAG_LABEL_RANGE; return y < 0 ? 0 : C - 1; }
-  return (int)y;
-}
-
 // Per-CTA integer tallies, the first KNN_TALLIES words of the dynamic shared memory: [0] correct count, [1] status
 // bits.  Flushed once per CTA: one 64-bit integer atomic for the count (no floating-point atomics), one OR.
 constexpr int KNN_TALLIES = 2;

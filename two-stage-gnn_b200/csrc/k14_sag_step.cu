@@ -298,33 +298,6 @@ __global__ void k_classify_rows(const float* __restrict__ emb, const int64_t* __
   }
 }
 
-// Fixed-order totals over n rows on one CTA: thread t adds rows t, t + 1024, ... in order, then a fixed tree.
-// sum_out = (sum v) / div; count_out = sum hit (int64).  Either output may be NULL.
-constexpr int SUM_THREADS = 1024;
-__global__ void __launch_bounds__(SUM_THREADS)
-k_sum_fixed(const float* __restrict__ v, const int* __restrict__ hit, int n, float div, float* sum_out, int64_t* count_out) {
-  pdl_wait();
-  pdl_launch_dependents();
-  __shared__ float sv[SUM_THREADS];
-  __shared__ long long sc[SUM_THREADS];
-  float s = 0.f;
-  long long c = 0;
-  for (int i = threadIdx.x; i < n; i += SUM_THREADS) {
-    if (sum_out) s += v[i];
-    if (count_out) c += hit[i];
-  }
-  sv[threadIdx.x] = s; sc[threadIdx.x] = c;
-  __syncthreads();
-  for (int o = SUM_THREADS / 2; o > 0; o >>= 1) {
-    if (threadIdx.x < o) { sv[threadIdx.x] += sv[threadIdx.x + o]; sc[threadIdx.x] += sc[threadIdx.x + o]; }
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) {
-    if (sum_out) *sum_out = sv[0] / div;
-    if (count_out) *count_out = sc[0];
-  }
-}
-
 static int head_ctas(int G) {
   // one batch of HEAD_WARPS graphs per CTA up to two CTAs per SM (ncu, first cut: 110 CTAs of 4 batches = 12 % warps
   // active, 55 us for 3,504 graphs -- the kernel is latency bound, so it wants every SM busy)

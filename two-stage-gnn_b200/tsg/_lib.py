@@ -80,6 +80,11 @@ _PROTOTYPES = {
     "tsg_linkpred_workspace_bytes": (SZ, [I64]),
     "tsg_linkpred_loss_fwd": (I, [P, P, P, P, I64, I64, ctypes.c_double, F32, P, P, SZ, P]),
     "tsg_linkpred_loss_bwd": (I, [P, P, P, P, I64, I64, ctypes.c_double, F32, P, P, P]),
+    "tsg_pred_ce_workspace_bytes": (SZ, [P, I64]),
+    "tsg_pred_ce_fwd": (I, [P, P, P, I64, P, P, P, P, SZ, P]),
+    "tsg_pred_ce_bwd": (I, [P, P, P, I64, P, P, P, P, P, SZ, P]),
+    "tsg_pred_classify_workspace_bytes": (SZ, [P, I64]),
+    "tsg_pred_classify": (I, [P, P, P, I64, P, P, P, P, P, P, SZ, P]),
     "tsg_knn_predict": (I, [P, P, P, I64, I64, I64, I, I, P, P]),
     "tsg_knn_classify": (I, [P, P, P, P, I64, I64, I64, I, I, P, P, P, P]),
     "tsg_mlp1_predict": (I, [P, P, I64, I64, I64, I64, I64, P, F32, P, P, P, P, P]),
@@ -127,6 +132,12 @@ class SagHead(ctypes.Structure):
     _fields_ = [("num_classes", c_int64), ("num_triplets", c_int64), ("margin", c_float), ("eps", c_float),
                 ("dropout_p", c_float), ("seed", ctypes.c_uint64)]
 
+class PredHead(ctypes.Structure):
+    """tsg_pred_head (include/tsg.h)."""
+    _fields_ = [("num_layers", c_int64), ("in_dim", c_int64), ("out_dim", c_int64 * 8), ("relu_mask", c_int64),
+                ("softmax_first", c_int64), ("weight", c_void_p * 8), ("bias", c_void_p * 8)]
+
+
 
 EXPORTS = tuple(_PROTOTYPES)
 
@@ -153,6 +164,7 @@ KERNELS_PER_CALL = {
     "tsg_readout_fwd": 1, "tsg_readout_bwd": 1, "tsg_triplet_fwd": 2, "tsg_triplet_bwd": 9,
     "tsg_pairdist_matrix": 1, "tsg_linear_fwd": 1, "tsg_dense_epilogue_bwd": 1, "tsg_linear_bwd_weight": 2, "tsg_sag_boundary_bwd": 2,
     "tsg_eigpool_build": 1, "tsg_coarsen_edges": 6, "tsg_inv_perm": 1, "tsg_csr_filter": 5, "tsg_sag_encoder_fwd": 38, "tsg_sag_encoder_bwd": 22, "tsg_sag_encoder_fwd_compact": 36, "tsg_sag_encoder_embed_compact": 3, "tsg_sag_triplet_step_compact": 72, "tsg_sag_step_fwd_compact": 37, "tsg_sag_step_bwd_compact": 25, "tsg_sag_nll_step_compact": 64, "tsg_sag_classify_compact": 6, "tsg_linkpred_loss_fwd": 3, "tsg_linkpred_loss_bwd": 1, "tsg_spmm_label_dot": 1, "tsg_gate_readout_fwd": 1, "tsg_gate_readout_linear_fwd": 2, "tsg_sag_encoder_bwd_compact": 22, "tsg_relu_bwd_colsum_rank1": 1, "tsg_sag_conv_bwd_fused": 1, "tsg_gate_score_bwd": 1, "tsg_spmm_dot": 1, "tsg_pack_batch_compact": 1, "tsg_pack_dense_batch": 1, "tsg_pack_eigen_batch": 1, "tsg_seg_contract": 1, "tsg_seg_linear": 1, "tsg_seg_linear_tc": 1, "tsg_linear_tc": 2, "tsg_gat_fwd": 2, "tsg_gat_bwd": 2, "tsg_dense_to_coo": 6, "tsg_nodebn_fwd": 1, "tsg_nodebn_bwd": 1,
+    "tsg_pred_ce_fwd": 2, "tsg_pred_ce_bwd": 1, "tsg_pred_classify": 2,
 }
 launch_calls = 0        # libtsg entry points called since import
 kernel_launches = 0     # kernels enqueued by them

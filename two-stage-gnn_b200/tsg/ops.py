@@ -7,6 +7,7 @@ There is no CPU path: CPU tensors raise.
 """
 from __future__ import annotations
 
+import ctypes
 import os
 from dataclasses import dataclass
 from typing import Optional, Tuple
@@ -702,3 +703,103 @@ def linkpred_loss(s: torch.Tensor, graph_ptr: torch.Tensor, csr_raw: CSR, num_en
     """K15: SoftPoolingGcnEncoder.loss's link-prediction term (Code/sage+gat+diffpool/encoders.py:416-440) on packed
     assignment rows s [sum n, K] and the RAW CSR of the 0/1 adjacency; num_entries = sum_g n_g^2 (host)."""
     return _LinkPredLoss.apply(s, graph_ptr, csr_raw, num_entries, eps)
+
+
+# --------------------------------------------------------------------------------------------
+# K16 prediction head + cross-entropy
+# --------------------------------------------------------------------------------------------
+PRED_MAX_LAYERS, PRED_MAX_WIDTH = 8, 256
+
+
+def check_pred_head(in_dim: int, out_dims) -> None:
+    """Raise ValueError unless a head over rows of width `in_dim` with layers of widths `out_dims` fits K16 (at most 8
+    layers, every width in [1, 256]): there is no other path for such a head."""
+    widths = [int(in_dim)] + [int(w) for w in out_dims]
+    if len(widths) - 1 > PRED_MAX_LAYERS or min(widths) < 1 or max(widths) > PRED_MAX_WIDTH:
+        raise ValueError(f"tsg: the prediction head ({len(widths) - 1} layers, widths {widths}) is beyond K16's limits: at "
+                         f"most {PRED_MAX_LAYERS} Linear layers, every width in [1, {PRED_MAX_WIDTH}]")
+
+
+def pred_head_desc(in_dim: int, layers, softmax_first: bool) -> "_lib.PredHead":
+    """The tsg_pred_head of a chain of `layers` [(weight [out, in], bias [out] or None, relu_after), ...] over rows of
+    width `in_dim` (check_pred_head first)."""
+    check_pred_head(in_dim, [int(w.size(0)) for w, _, _ in layers])
+    h = _lib.PredHead()
+    h.num_layers, h.in_dim, h.softmax_first = len(layers), int(in_dim), int(bool(softmax_first))
+    mask, inp = 0, int(in_dim)
+    for l, (w, b, relu) in enumerate(layers):
+        if w.dim() != 2 or w.size(1) != inp:
+            raise ValueError(f"tsg: prediction-head layer {l} takes {tuple(w.shape)} weights after a width of {inp}")
+        h.out_dim[l], h.weight[l], h.bias[l] = int(w.size(0)), ptr(w), ptr(b)
+        mask |= (1 << l) if relu else 0
+        inp = int(w.size(0))
+    h.relu_mask = mask
+    return h
+
+
+class _PredCE(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, r, y, softmax_first, relus, *params):
+        from . import nn as tnn
+        r = r.contiguous()
+        layers = [(params[2 * l].contiguous(), None if params[2 * l + 1] is None else params[2 * l + 1].contiguous(), relus[l])
+                  for l in range(len(relus))]
+        desc = pred_head_desc(r.size(1), layers, softmax_first)
+        G = r.size(0)
+        wsb = lib.tsg_pred_ce_workspace_bytes(ctypes.byref(desc), G)
+        ws = workspace(wsb, r.device)
+        loss = torch.empty((), dtype=torch.float32, device=r.device)
+        call("tsg_pred_ce_fwd", ctypes.byref(desc), ptr(r), ptr(y), G, ptr(loss), None, ptr(tnn._status_word(r.device)),
+             ptr(ws), wsb, stream_ptr())
+        ctx.desc, ctx.ws, ctx.wsb, ctx.layers = desc, ws, wsb, layers      # the layers keep desc's pointers alive
+        ctx.save_for_backward(r, y)
+        return loss
+
+    @staticmethod
+    def backward(ctx, dloss):
+        r, y = ctx.saved_tensors
+        L = len(ctx.layers)
+        dr = torch.empty_like(r) if ctx.needs_input_grad[0] else None
+        dws = [torch.empty_like(w) for w, _, _ in ctx.layers]
+        dbs = [None if b is None else torch.empty_like(b) for _, b, _ in ctx.layers]
+        arr = ctypes.c_void_p * max(L, 1)
+        call("tsg_pred_ce_bwd", ctypes.byref(ctx.desc), ptr(r), ptr(y), r.size(0), ptr(dloss.contiguous().view(1)), ptr(dr),
+             arr(*[ptr(t) for t in dws]), arr(*[ptr(t) for t in dbs]), ptr(ctx.ws), ctx.wsb, stream_ptr())
+        grads = []
+        for dw, db in zip(dws, dbs):
+            grads += [dw, db]
+        return (dr, None, None, None, *grads)
+
+
+def pred_ce(r: torch.Tensor, layers, y: torch.Tensor, softmax_first: bool = False) -> torch.Tensor:
+    """K16: mean cross-entropy of the head `layers` [(weight [out, in], bias or None, relu_after), ...] over the readout
+    rows r [G, D0] against int64 labels y [G] (softmax_first: of softmax(logits), the reference's 2stg+ stage 2).  An
+    autograd Function: backward reaches r (and the encoder below it) and every weight and bias.  A label outside
+    [0, C) sets status bit 8 (tsg.nn.check_fused_status raises)."""
+    flat = []
+    for w, b, _ in layers:
+        flat += [w, b]
+    return _PredCE.apply(r, y.contiguous(), bool(softmax_first), tuple(bool(x) for _, _, x in layers), *flat)
+
+
+def pred_classify(r: torch.Tensor, layers, y: Optional[torch.Tensor] = None, softmax_first: bool = False,
+                  want_logits: bool = False):
+    """K16's eval-mode forward: -> (pred int64 [G] (first-index argmax of the logits), logits [G, C] or None,
+    correct int64 [1] or None, ce_sum float32 [1] or None); the last two need the labels y and are fixed-order totals
+    (ce_sum includes the softmax_first loss)."""
+    from . import nn as tnn
+    r = r.contiguous()
+    with torch.no_grad():
+        layers = [(w.detach().contiguous(), None if b is None else b.detach().contiguous(), relu) for w, b, relu in layers]
+        desc = pred_head_desc(r.size(1), layers, softmax_first)
+        G, dev = r.size(0), r.device
+        C = layers[-1][0].size(0) if layers else r.size(1)
+        pred = torch.empty(G, dtype=torch.int64, device=dev)
+        logits = torch.empty(G, C, dtype=torch.float32, device=dev) if want_logits else None
+        correct = torch.empty(1, dtype=torch.int64, device=dev) if y is not None else None
+        ce_sum = torch.empty(1, dtype=torch.float32, device=dev) if y is not None else None
+        wsb = lib.tsg_pred_classify_workspace_bytes(ctypes.byref(desc), G)
+        ws = workspace(wsb, dev)
+        call("tsg_pred_classify", ctypes.byref(desc), ptr(r), ptr(None if y is None else y.contiguous()), G, ptr(pred),
+             ptr(logits), ptr(correct), ptr(ce_sum), ptr(tnn._status_word(dev)), ptr(ws), wsb, stream_ptr())
+    return pred, logits, correct, ce_sum

@@ -646,7 +646,117 @@ class ClassifierTrainer:
         return float(acc[0] / n), float(acc[1] / n)
 
 
-class DenseTripletTrainer:
+class _DenseEncoderTrainer:
+    """What the trainers of the dense encoders share: the model / feature-table checks, the batch assembled on the GPU
+    from an HBM-resident corpus (DeviceCorpus.pack_dense, after the host-side `_check`) and the forward up to the graph
+    readout.  Subclasses call `_bind` first."""
+
+    def _bind(self, model: torch.nn.Module, table: torch.Tensor, max_nodes: int) -> list:
+        """Check the model and the table and keep them: -> the model's parameters."""
+        from . import dense, diffpool, gat
+        if isinstance(model, gat.PackedGatEncoder):
+            self.kind, in_dim = "gat", model.conv_first.heads()[0].input_dim
+        elif isinstance(model, diffpool.PackedSoftPoolEncoder):
+            self.kind, in_dim = "diffpool", model.conv_first.input_dim
+            if int(model.max_num_nodes) != int(max_nodes):
+                raise ValueError(f"tsg: the DiffPool model was built for max_num_nodes = {model.max_num_nodes}, the trainer "
+                                 f"pads to max_nodes = {max_nodes}")
+        elif isinstance(model, dense.PackedGcnEncoder):
+            self.kind, in_dim = "base", model.conv_first.input_dim
+        else:
+            raise TypeError(f"tsg: {type(self).__name__} takes a PackedGcnEncoder, PackedGatEncoder or PackedSoftPoolEncoder")
+        if int(max_nodes) < 1:
+            raise ValueError("tsg: max_nodes must be at least 1")
+        if table.dim() != 2 or table.size(0) < int(max_nodes):
+            raise ValueError(f"tsg: the feature table must be [max_nodes = {max_nodes}, F], not {tuple(table.shape)}")
+        if table.size(1) != in_dim:
+            raise ValueError(f"tsg: the feature table has {table.size(1)} columns, the model takes {in_dim}")
+        params = list(model.parameters())
+        dev = params[0].device if params else table.device
+        self.model, self.max_nodes = model, int(max_nodes)
+        self.table = table.to(device=dev, dtype=torch.float32).contiguous()
+        self.want_eid = self.kind == "gat"                 # GAT's backward walks both orientations by edge id
+        return params
+
+    def _forward(self, batch):
+        if self.kind == "gat":
+            return self.model(batch.x, batch.csr, batch.graph_ptr, batch.max_nodes)
+        return self.model(batch.x, batch.csr, batch.graph_ptr, batch.has_pad)
+
+    def _readout(self, batch):
+        """The model's forward up to its graph readout (the input of its heads)."""
+        if self.kind == "gat":
+            return self.model.readout(batch.x, batch.csr, batch.graph_ptr, batch.max_nodes)
+        return self.model.readout(batch.x, batch.csr, batch.graph_ptr, batch.has_pad)
+
+    def pack(self, corpus, ids_host):
+        """ids -> tsg.feeder.DenseBatch for this trainer's model (eids for GAT), assembled on the GPU."""
+        return corpus.pack_dense(ids_host, self.table, self.max_nodes, want_eid=self.want_eid)
+
+    def _check(self, corpus, ids_host) -> np.ndarray:
+        """The host-side checks of a pack (no device work): -> the ids as int64 numpy."""
+        return corpus.check_dense(ids_host, self.table, self.max_nodes)
+
+    def _pack_checked(self, corpus, ids: np.ndarray):
+        """`pack` for ids that passed `_check`: one staged upload, one launch."""
+        return corpus.pack_dense_staged(*corpus._stage(ids), self.table, self.max_nodes, self.want_eid)
+
+    def _batch(self, corpus, ids: np.ndarray):
+        """`_pack_checked` and the graphs' labels (int64 [B], gathered on the device from corpus.y by the staged ids)."""
+        meta, B, nptr, eptr = corpus._stage(ids)
+        batch = corpus.pack_dense_staged(meta, B, nptr, eptr, self.table, self.max_nodes, self.want_eid)
+        return batch, corpus.y.index_select(0, meta[:B])
+
+
+class _WaveEncoderTrainer(_DenseEncoderTrainer):
+    """`_DenseEncoderTrainer` for the EigenGCN encoder (tsg.dense.PackedWaveEncoder = Code/eigengcn's
+    WavePoolingGcnEncoder with one pooling level) against a corpus whose EigenPooling operands are attached
+    (DeviceCorpus.attach_eigen): every batch is assembled on the GPU by DeviceCorpus.pack_eigen in one launch.
+    Refused on the host: a model with more than one pooling level (the operands describe one), operands with fewer
+    pooling matrices than the model uses, and a corpus whose node-label count differs from the model's input_dim."""
+
+    def _bind(self, model: torch.nn.Module, table, max_nodes: int) -> list:
+        from . import dense
+        if not isinstance(model, dense.PackedWaveEncoder):
+            raise TypeError(f"tsg: {type(self).__name__} takes a PackedWaveEncoder")
+        if len(model.pool_sizes) != 1:
+            raise ValueError(f"tsg: the model has {len(model.pool_sizes)} pooling levels; the EigenPooling operands "
+                             "describe one")
+        if int(max_nodes) < 1:
+            raise ValueError("tsg: max_nodes must be at least 1")
+        self.kind, self.table, self.want_eid = "wave", None, False
+        self.model, self.max_nodes = model, int(max_nodes)
+        return list(model.parameters())
+
+    def _check(self, corpus, ids_host) -> np.ndarray:
+        m = self.model
+        if corpus.feat != m.conv_first.input_dim:
+            raise ValueError(f"tsg: the corpus has {corpus.feat} node labels, the model takes input_dim = "
+                             f"{m.conv_first.input_dim}")
+        ids, _, _ = corpus.check_eigen(ids_host, self.max_nodes, m.num_pool_matrix, m.num_pool_final_matrix)
+        return ids
+
+    def _pack_checked(self, corpus, ids: np.ndarray):
+        return corpus.pack_eigen_checked(ids, self.max_nodes, self.model.num_pool_matrix,
+                                         self.model.num_pool_final_matrix)
+
+    def _batch(self, corpus, ids: np.ndarray):
+        return self._pack_checked(corpus, ids), corpus.y.index_select(0, corpus._upload([ids]))
+
+    def pack(self, corpus, ids_host):
+        """ids -> tsg.feeder.EigenBatch for this trainer's model, assembled on the GPU."""
+        return self._pack_checked(corpus, self._check(corpus, ids_host))
+
+    def _forward(self, batch):
+        args, kw = batch.readout_args()
+        return self.model(*args, **kw)
+
+    def _readout(self, batch):
+        args, kw = batch.readout_args()
+        return self.model.readout(*args, **kw)
+
+
+class DenseTripletTrainer(_DenseEncoderTrainer):
     """2stg stage-1 training and scoring of the dense encoders of Code/sage+gat+diffpool against an HBM-resident corpus
     (tsg.feeder.DeviceCorpus): tsg.dense.PackedGcnEncoder ("base" / GraphSAGE), tsg.gat.PackedGatEncoder and
     tsg.diffpool.PackedSoftPoolEncoder.  Every batch is assembled on the GPU by DeviceCorpus.pack_dense: node features are
@@ -664,42 +774,9 @@ class DenseTripletTrainer:
 
     def __init__(self, model: torch.nn.Module, table: torch.Tensor, max_nodes: int = 1000, lr: float = 1e-3,
                  margin: float = 1.5, clip_norm: Optional[float] = 2.0, group=None):
-        from . import dense, diffpool, gat
-        if isinstance(model, gat.PackedGatEncoder):
-            self.kind, in_dim = "gat", model.conv_first.heads()[0].input_dim
-        elif isinstance(model, diffpool.PackedSoftPoolEncoder):
-            self.kind, in_dim = "diffpool", model.conv_first.input_dim
-            if int(model.max_num_nodes) != int(max_nodes):
-                raise ValueError(f"tsg: the DiffPool model was built for max_num_nodes = {model.max_num_nodes}, the trainer "
-                                 f"pads to max_nodes = {max_nodes}")
-        elif isinstance(model, dense.PackedGcnEncoder):
-            self.kind, in_dim = "base", model.conv_first.input_dim
-        else:
-            raise TypeError("tsg: DenseTripletTrainer takes a PackedGcnEncoder, PackedGatEncoder or PackedSoftPoolEncoder")
-        if int(max_nodes) < 1:
-            raise ValueError("tsg: max_nodes must be at least 1")
-        if table.dim() != 2 or table.size(0) < int(max_nodes):
-            raise ValueError(f"tsg: the feature table must be [max_nodes = {max_nodes}, F], not {tuple(table.shape)}")
-        if table.size(1) != in_dim:
-            raise ValueError(f"tsg: the feature table has {table.size(1)} columns, the model takes {in_dim}")
-        params = list(model.parameters())
-        dev = params[0].device if params else table.device
-        self.model, self.margin, self.group = model, margin, group
-        self.max_nodes, self.clip_norm = int(max_nodes), clip_norm
-        self.table = table.to(device=dev, dtype=torch.float32).contiguous()
-        self.want_eid = self.kind == "gat"                 # GAT's backward walks both orientations by edge id
+        params = self._bind(model, table, max_nodes)
+        self.margin, self.group, self.clip_norm = margin, group, clip_norm
         self.opt = torch.optim.Adam(params, lr=lr)          # train_triplet.py:216
-
-    def _forward(self, batch):
-        if self.kind == "gat":
-            return self.model(batch.x, batch.csr, batch.graph_ptr, batch.max_nodes)
-        return self.model(batch.x, batch.csr, batch.graph_ptr, batch.has_pad)
-
-    def _readout(self, batch):
-        """The model's forward up to its graph readout (the input of the head that makes element [1])."""
-        if self.kind == "gat":
-            return self.model.readout(batch.x, batch.csr, batch.graph_ptr, batch.max_nodes)
-        return self.model.readout(batch.x, batch.csr, batch.graph_ptr, batch.has_pad)
 
     def _head(self, r):
         """Element [1] of the model's forward from its readout `r` (encoders.py:207-217, encoders_GAT.py:191-198)."""
@@ -709,18 +786,6 @@ class DenseTripletTrainer:
         if m.final_dim not in ("pretrain", "output_dim"):
             return m.pred_model(m.pre_pred_model(r))
         return m.map_model(r)
-
-    def pack(self, corpus, ids_host):
-        """ids -> tsg.feeder.DenseBatch for this trainer's model (eids for GAT), assembled on the GPU."""
-        return corpus.pack_dense(ids_host, self.table, self.max_nodes, want_eid=self.want_eid)
-
-    def _check(self, corpus, ids_host) -> np.ndarray:
-        """The host-side checks of a pack (no device work): -> the ids as int64 numpy."""
-        return corpus.check_dense(ids_host, self.table, self.max_nodes)
-
-    def _pack_checked(self, corpus, ids: np.ndarray):
-        """`pack` for ids that passed `_check`: one staged upload, one launch."""
-        return corpus.pack_dense_staged(*corpus._stage(ids), self.table, self.max_nodes, self.want_eid)
 
     def _embedding(self, batch) -> torch.Tensor:
         """The embedding the triplet loss sees (element [1] of the model's output)."""
@@ -806,58 +871,196 @@ class DenseTripletTrainer:
                                 self.group)
 
 
-class WaveTripletTrainer(DenseTripletTrainer):
-    """2stg stage-1 training and scoring of the EigenGCN encoder (tsg.dense.PackedWaveEncoder = Code/eigengcn's
-    WavePoolingGcnEncoder with one pooling level) against an HBM-resident corpus whose EigenPooling operands are
-    attached (DeviceCorpus.attach_eigen).  Every batch is assembled on the GPU by DeviceCorpus.pack_eigen in one launch:
-    one-hot node labels, the RAW adjacency, P_j^T, the coarsened adjacency and the final pooling, with the per-level
-    padded-row flags of `max_nodes`.  The embedding is the model's output, the one bench config 5 feeds the triplet
-    loss; DenseTripletTrainer's step / run_from_ids / embed / evaluate contract applies (embed: readouts in packed
-    batches, pred_model once over all rows).  Defaults: Adam 1e-3, margin 1.5, no clip (bench config 5's step).
-    Refused on the host: a model with more than one pooling level (the operands describe one), operands with fewer
-    pooling matrices than the model uses, and a corpus whose node-label count differs from the model's input_dim."""
+class WaveTripletTrainer(_WaveEncoderTrainer, DenseTripletTrainer):
+    """2stg stage-1 training and scoring of the EigenGCN encoder (see _WaveEncoderTrainer for the batches and what is
+    refused on the host).  The embedding is the model's output, the one bench config 5 feeds the triplet loss;
+    DenseTripletTrainer's step / run_from_ids / embed / evaluate contract applies (embed: readouts in packed batches,
+    pred_model once over all rows).  Defaults: Adam 1e-3, margin 1.5, no clip (bench config 5's step)."""
 
     def __init__(self, model: torch.nn.Module, max_nodes: int = 1000, lr: float = 1e-3, margin: float = 1.5,
                  clip_norm: Optional[float] = None, group=None):
-        from . import dense
-        if not isinstance(model, dense.PackedWaveEncoder):
-            raise TypeError("tsg: WaveTripletTrainer takes a PackedWaveEncoder")
-        if len(model.pool_sizes) != 1:
-            raise ValueError(f"tsg: the model has {len(model.pool_sizes)} pooling levels; the EigenPooling operands "
-                             "describe one")
-        if int(max_nodes) < 1:
-            raise ValueError("tsg: max_nodes must be at least 1")
-        self.kind, self.table, self.want_eid = "wave", None, False
-        self.model, self.margin, self.group = model, margin, group
-        self.max_nodes, self.clip_norm = int(max_nodes), clip_norm
-        self.opt = torch.optim.Adam(list(model.parameters()), lr=lr)
-
-    def _check(self, corpus, ids_host) -> np.ndarray:
-        m = self.model
-        if corpus.feat != m.conv_first.input_dim:
-            raise ValueError(f"tsg: the corpus has {corpus.feat} node labels, the model takes input_dim = "
-                             f"{m.conv_first.input_dim}")
-        ids, _, _ = corpus.check_eigen(ids_host, self.max_nodes, m.num_pool_matrix, m.num_pool_final_matrix)
-        return ids
-
-    def _pack_checked(self, corpus, ids: np.ndarray):
-        return corpus.pack_eigen_checked(ids, self.max_nodes, self.model.num_pool_matrix,
-                                         self.model.num_pool_final_matrix)
-
-    def pack(self, corpus, ids_host):
-        """ids -> tsg.feeder.EigenBatch for this trainer's model, assembled on the GPU."""
-        return self._pack_checked(corpus, self._check(corpus, ids_host))
-
-    def _forward(self, batch):
-        args, kw = batch.readout_args()
-        return self.model(*args, **kw)
+        params = self._bind(model, None, max_nodes)
+        self.margin, self.group, self.clip_norm = margin, group, clip_norm
+        self.opt = torch.optim.Adam(params, lr=lr)
 
     def _embedding(self, batch) -> torch.Tensor:
         return self._forward(batch)
 
-    def _readout(self, batch):
-        args, kw = batch.readout_args()
-        return self.model.readout(*args, **kw)
-
     def _head(self, r):
         return self.model.pred_model(r)
+
+
+def _linear_chain(*mods) -> list:
+    """nn.Linear / nn.ReLU / nn.Sequential modules in call order -> K16's layers [(weight, bias, relu_after), ...]."""
+    out = []
+    for m in mods:
+        for c in (m if isinstance(m, torch.nn.Sequential) else [m]):
+            if isinstance(c, torch.nn.Linear):
+                out.append([c.weight, c.bias, False])
+            elif isinstance(c, torch.nn.ReLU) and out:
+                out[-1][2] = True
+            else:
+                raise ValueError(f"tsg: the prediction head holds a {type(c).__name__}; K16 runs Linear and ReLU layers")
+    return [tuple(x) for x in out]
+
+
+class DenseClassifierTrainer(_DenseEncoderTrainer):
+    """Supervised training and evaluation of the dense encoders (tsg.dense.PackedGcnEncoder "base", tsg.gat.PackedGatEncoder,
+    tsg.diffpool.PackedSoftPoolEncoder) against an HBM-resident corpus with graph labels, batches assembled as for
+    DenseTripletTrainer.  The head over the readout and the cross-entropy are K16 (tsg.ops.pred_ce); the encoder's
+    backward continues from the readout gradient.  The logits per setting (Code/sage+gat+diffpool, SURVEY A.2):
+
+      setting="original" (train.py:85-152; the model's final_dim must not be "output_dim" or "pretrain"):
+        base / DiffPool: pred_model(pre_pred_model(readout)); GAT: pred_model(readout); plain cross-entropy.
+      setting="2stg+" (stage 2 of train_triplet_pre_train.py:249-256, after stage 1 with DenseTripletTrainer):
+        base / DiffPool (final_dim="pretrain"): map2_model(map_model(readout)), 2 classes; GAT (any final_dim): the raw
+        readout, embedding_dim classes, no head parameters.  The reference applies softmax to these logits before
+        F.cross_entropy; so does this trainer.
+
+    The step is the reference's: the loss (plus the DiffPool link-prediction term with linkpred=True, original only),
+    backward, clip_grad_norm(clip_norm) (None: no clip), Adam(lr) -- or `optimizer`, e.g. the stage-1 trainer's `opt`,
+    whose state then carries on.  Under a process group one all-reduce of [G_r * grads, G_r * loss, G_r] per step makes
+    the loss and gradient those of the global batch, before the clip.
+
+    Refused on the host (ValueError): a final_dim that does not fit the setting, linkpred on anything but DiffPool
+    original, a head beyond K16's limits (at most 8 layers, widths <= 256), and a corpus label outside the class count."""
+
+    def __init__(self, model: torch.nn.Module, table: torch.Tensor, max_nodes: int = 1000, setting: str = "original",
+                 lr: float = 1e-3, clip_norm: Optional[float] = 2.0, linkpred: bool = False, optimizer=None, group=None):
+        params = self._bind(model, table, max_nodes)
+        self._setup(setting, linkpred)
+        self.clip_norm, self.group = clip_norm, group
+        self.opt = optimizer if optimizer is not None else torch.optim.Adam(params, lr=lr)     # train.py: Adam 1e-3
+
+    def _setup(self, setting: str, linkpred: bool) -> None:
+        """The head modules, softmax_first and the class count of (model, setting), checked against K16's limits."""
+        if setting not in ("original", "2stg+"):
+            raise ValueError(f"tsg: setting must be 'original' or '2stg+', not {setting!r}")
+        m, kind = self.model, self.kind
+        fd = getattr(m, "final_dim", None)
+        note = ""
+        if kind == "wave":                          # EigenGCN: pred_model in both settings, no softmax (SURVEY 3c, a13)
+            mods, softmax_first = (m.pred_model,), False
+        elif setting == "original":
+            if fd in ("output_dim", "pretrain"):
+                raise ValueError(f"tsg: the original setting classifies with pred_model: the model's final_dim must not be "
+                                 f"'output_dim' or 'pretrain' (it is {fd!r})")
+            mods = (m.pred_model,) if kind == "gat" else (m.pre_pred_model, m.pred_model)
+            softmax_first = False
+        elif kind == "gat":
+            mods, softmax_first = (), True
+            note = f"2stg+ takes the GAT readout's embedding_dim = {m.map_model.in_features} columns as the logits"
+        else:
+            if fd != "pretrain":
+                raise ValueError(f"tsg: 2stg+ classifies with map2_model(map_model(readout)): the model's final_dim must be "
+                                 f"'pretrain' (it is {fd!r})")
+            mods, softmax_first = (m.map_model, m.map2_model), True
+            note = "2stg+ takes map2_model's 2 outputs as the logits"
+        if linkpred and not (kind == "diffpool" and setting == "original"):
+            raise ValueError("tsg: linkpred adds DiffPool's link-prediction loss: it needs a PackedSoftPoolEncoder in the "
+                             "original setting")
+        self.setting, self.linkpred, self.softmax_first = setting, bool(linkpred), softmax_first
+        self._head_mods, self._label_note = mods, note
+        layers = self._layers()
+        in_dim = layers[0][0].size(1) if layers else m.map_model.in_features
+        ops.check_pred_head(in_dim, [w.size(0) for w, _, _ in layers])
+        self.num_classes = int(layers[-1][0].size(0)) if layers else int(in_dim)
+
+    def _layers(self) -> list:
+        return _linear_chain(*self._head_mods)
+
+    def _check_labels(self, corpus) -> None:
+        try:
+            corpus.check_labels(self.num_classes)
+        except ValueError as e:
+            if not self._label_note or corpus.y is None:
+                raise
+            raise ValueError(f"{e}: {self._label_note}") from None
+
+    def step(self, batch, y: torch.Tensor) -> torch.Tensor:
+        """One training step on a packed batch (DenseBatch, or EigenBatch for WaveClassifierTrainer) with its labels y
+        (int64 [G], on the device).  Returns the loss (the global batch's mean under a process group)."""
+        self.model.train()
+        if self.linkpred:
+            b = batch
+            r, aux = self.model.readout(b.x, b.csr, b.graph_ptr, b.has_pad, return_aux=True)
+        else:
+            r = self._readout(batch)
+        loss = ops.pred_ce(r, self._layers(), y, self.softmax_first)
+        if self.linkpred:                                                  # encoders.py:409-441
+            loss = loss + self.model.link_loss(aux["s"], batch.csr, batch.graph_ptr, np.diff(batch.node_ptr_host))
+        self.opt.zero_grad(set_to_none=True)
+        loss.backward()
+        params = list(self.model.parameters())
+        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
+        if world > 1:
+            loss = all_reduce_grads_and_loss(params, loss, int(y.shape[0]), self.group)
+        if self.clip_norm is not None:
+            torch.nn.utils.clip_grad_norm_(params, self.clip_norm)
+        self.opt.step()
+        return loss.detach()
+
+    def run_from_ids(self, corpus, id_batches) -> list:
+        """Training loop against an HBM-resident corpus with labels: per step the host provides only the graph ids (int64
+        numpy [B]); the batch is assembled on the GPU, its labels gathered there from corpus.y, and the loss is read
+        back into pinned memory without stalling the enqueue thread.  Labels are checked against the class count on
+        the host once; the status word once, at the end.  Returns the per-step losses."""
+        self._check_labels(corpus)
+        host_losses = []
+        for ids_host in id_batches:
+            loss = self.step(*self._batch(corpus, self._check(corpus, ids_host)))
+            h = torch.empty((), dtype=torch.float32, pin_memory=True)
+            h.copy_(loss, non_blocking=True)
+            host_losses.append(h)
+        torch.cuda.current_stream(corpus.device).synchronize()
+        _check_status()
+        return [float(h) for h in host_losses]
+
+    def evaluate(self, corpus, ids, batch_graphs: int = 4096):
+        """(accuracy, mean cross-entropy) over the graphs `ids` in eval mode, the caller's mode restored: readouts in
+        packed batches of `batch_graphs`, then K16's classify over all rows at once (tsg_pred_classify: pred = the
+        first-index argmax of the logits, the loss as in training, softmax_first included), so the totals do not depend
+        on `batch_graphs`.  One device-to-host read of [correct, loss sum, status]; under a process group every rank
+        passes its own ids and [correct, loss sum, count] is all-reduced."""
+        from . import nn as tnn
+        if batch_graphs < 1:
+            raise ValueError("tsg: batch_graphs must be at least 1")
+        ids = self._check(corpus, ids)
+        self._check_labels(corpus)
+        dev = corpus.device
+        status = tnn._status_word(dev)
+        was_training = self.model.training
+        self.model.eval()
+        try:
+            with torch.no_grad():
+                parts = [self._readout(self._pack_checked(corpus, ids[s:s + batch_graphs]))
+                         for s in range(0, ids.shape[0], batch_graphs)]
+                r = parts[0] if len(parts) == 1 else torch.cat(parts)
+                y = corpus.y.index_select(0, corpus._upload([ids]))
+                _, _, correct, ce_sum = ops.pred_classify(r, self._layers(), y, self.softmax_first)
+        finally:
+            self.model.train(was_training)
+        host = torch.cat([correct.double(), ce_sum.double(), status.double()]).cpu().numpy()
+        tnn.check_fused_status({status.device.index: int(host[2])})
+        acc = np.array([host[0], host[1], float(ids.shape[0])], dtype=np.float64)
+        if dist.is_initialized() and dist.get_world_size(self.group) > 1:
+            red = torch.from_numpy(acc).to(dev)
+            dist.all_reduce(red, op=dist.ReduceOp.SUM, group=self.group)
+            acc = red.cpu().numpy()
+        n = max(acc[2], 1.0)
+        return float(acc[0] / n), float(acc[1] / n)
+
+
+class WaveClassifierTrainer(_WaveEncoderTrainer, DenseClassifierTrainer):
+    """DenseClassifierTrainer for the EigenGCN encoder (tsg.dense.PackedWaveEncoder, batches as for WaveTripletTrainer).
+    The logits are pred_model(readout) in both settings, with plain cross-entropy: in 2stg+ the reference swaps in a
+    map_model that the forward never reaches (SURVEY 3c, row a13), and SURVEY records no softmax before its loss.  The
+    reference's stage 2 steps the stage-1 optimiser: pass WaveTripletTrainer's `opt` as `optimizer` for that.  Defaults
+    as WaveTripletTrainer: Adam 1e-3, no clip."""
+
+    def __init__(self, model: torch.nn.Module, max_nodes: int = 1000, setting: str = "original", lr: float = 1e-3,
+                 clip_norm: Optional[float] = None, optimizer=None, group=None):
+        params = self._bind(model, None, max_nodes)
+        self._setup(setting, False)
+        self.clip_norm, self.group = clip_norm, group
+        self.opt = optimizer if optimizer is not None else torch.optim.Adam(params, lr=lr)

@@ -481,6 +481,63 @@ int tsg_coarsen_edges(const int64_t* row, const int64_t* col, const float* weigh
                       void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * K17  a resident corpus's EigenPooling operands (tsg.feeder.DeviceCorpus.build_eigen), in attach_eigen's layout
+ *   replaces the per-graph host loop of tsg.eigen_synth (make_operands = bfs_clusters + operands_from_clusters), i.e.
+ *   Code/eigengcn/coarsen_pooling_with_last_eigen_padding.py:121-182 with the clustering input of :125-126 (sklearn
+ *   SpectralClustering there) replaced by eigen_synth's BFS chunks or by labels the caller gives.
+ *   The corpus is coalesced and symmetric (as for K0d; graph-local int32 row / col, int64 node_ptr / edge_ptr [G+1]).
+ *   The entries work on a CHUNK of graphs first_graph .. first_graph + num_graphs - 1 holding num_nodes nodes and
+ *   num_edges edges (each below 2^31 together), graphs of at most max_nodes <= TSG_EIGEN_BUILD_MAX_NODES nodes
+ *   (3 max_nodes + 2 ints of shared memory per CTA).  In the chunk, graph g's nodes start at nb = node_ptr[g] -
+ *   node_ptr[first_graph], its edges at ob, and its cluster k has the chunk id nb + k (a graph has no more clusters
+ *   than nodes; rows nb + nc .. nb + n - 1 stay empty), so the chunk arrays are:
+ *     rowptr [num_nodes + 1] / colidx [num_edges]: the RAW adjacency CSR with chunk node ids (val = 1 implied);
+ *     cluster_g [num_nodes]: chunk cluster id of every node; member_ptr [num_nodes + 1] / member [num_nodes]: the
+ *     members of every chunk cluster row -- together exactly what tsg_eigpool_build takes (num_clusters = num_nodes).
+ *   status int32 [4], initialised by the caller to INT32_MAX: [0] = least graph whose edge list breaks the promise
+ *   (range, self loop, order or symmetry; its rows are left empty), [1] = least graph with a cluster of more than
+ *   TSG_EIG_MAX members, [2] = least graph with a label outside [0, n); [3] is free for tsg_eigpool_build's status.
+ *   tsg_eigen_bfs_clusters: eigen_synth.bfs_clusters -- the queue BFS from node 0 over ascending neighbour lists
+ *     (scipy breadth_first_order on the symmetric list), unreached nodes appended in ascending order, clusters =
+ *     chunks of pool_size (1 .. TSG_EIG_MAX) in that order.  Writes cluster_of [sum n] (corpus, graph-local ids),
+ *     num_clusters [G] (corpus, ceil(n / pool_size)) and the chunk arrays, members in BFS order.  Level-synchronous,
+ *     one CTA per graph: every node takes its first discoverer, and a level is ordered by (discoverer, node id).
+ *   tsg_eigen_group_clusters: the chunk arrays for the graph-local labels cluster_of (corpus, input), members in
+ *     ascending node order; num_clusters (nullable) [G] = max label + 1.
+ *   tsg_eigen_coarse: per graph, the entries of Omega^T A_ext Omega (coarsen...py:135-149): the (cl[row], cl[col])
+ *     pairs of the inter-cluster edges, merged, sorted row-major (np.nonzero's order), count = weight.  Counting pass
+ *     (coarse_row NULL): num_coarse [G] (corpus).  Writing pass: coarse_row / coarse_col (graph-local cluster ids) /
+ *     coarse_w at the corpus offsets coarse_ptr [G+1]; row_scratch [num_nodes].  Any member order works.
+ *   tsg_eigen_final: the final pooling (:150-182 with one cluster holding every coarse node): the first num_vectors
+ *     eigenvectors of D - A of the binary coarse adjacency of every graph with min_clusters < nc <= max_clusters (<=
+ *     TSG_EIGEN_FINAL_MAX) clusters, with K11's ordering, sign and repeat rules, to final_w [num_vectors, final_stride]
+ *     at the corpus offsets cluster_ptr [G+1]; other graphs are not written (another size class, or the caller
+ *     computes them).  One CTA per graph, fp64 cyclic Jacobi in 2 max_clusters (max_clusters + 1) doubles of shared
+ *     memory, so a launch per size class keeps small graphs many to an SM.
+ * ------------------------------------------------------------------------------------------ */
+#define TSG_EIGEN_BUILD_MAX_NODES 19370
+#define TSG_EIGEN_FINAL_MAX 112
+int tsg_eigen_bfs_clusters(const int64_t* corpus_node_ptr, const int64_t* corpus_edge_ptr, const int32_t* corpus_row,
+                           const int32_t* corpus_col, int64_t first_graph, int64_t num_graphs, int64_t num_nodes,
+                           int64_t num_edges, int64_t max_nodes, int64_t pool_size, int32_t* cluster_of,
+                           int32_t* num_clusters, int32_t* rowptr, int32_t* colidx, int32_t* cluster_g,
+                           int32_t* member_ptr, int32_t* member, int32_t* status, void* stream);
+int tsg_eigen_group_clusters(const int64_t* corpus_node_ptr, const int64_t* corpus_edge_ptr,
+                             const int32_t* corpus_row, const int32_t* corpus_col, int64_t first_graph,
+                             int64_t num_graphs, int64_t num_nodes, int64_t num_edges, int64_t max_nodes,
+                             const int32_t* cluster_of, int32_t* num_clusters /*nullable*/, int32_t* rowptr,
+                             int32_t* colidx, int32_t* cluster_g, int32_t* member_ptr, int32_t* member,
+                             int32_t* status, void* stream);
+int tsg_eigen_coarse(const int64_t* corpus_node_ptr, int64_t first_graph, int64_t num_graphs,
+                     const int32_t* num_clusters, const int32_t* rowptr, const int32_t* colidx,
+                     const int32_t* cluster_g, const int32_t* member_ptr, const int32_t* member,
+                     int32_t* row_scratch, int32_t* num_coarse, const int64_t* coarse_ptr, int32_t* coarse_row,
+                     int32_t* coarse_col, float* coarse_w, void* stream);
+int tsg_eigen_final(const int64_t* cluster_ptr, const int64_t* coarse_ptr, const int32_t* coarse_row,
+                    const int32_t* coarse_col, int64_t first_graph, int64_t num_graphs, int64_t min_clusters,
+                    int64_t max_clusters, int64_t num_vectors, float* final_w, int64_t final_stride, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * K12  stage-2 evaluation heads on graph embeddings (SURVEY 8f n4)
  *   tsg_knn_classify replaces KNeighborsClassifier(n_neighbors=k).fit(train).predict(query) of `evaluate`
  *     (Code/sage+gat+diffpool/train_triplet.py:80-85): Euclidean, uniform weights; distance ties -> lower

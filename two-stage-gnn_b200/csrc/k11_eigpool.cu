@@ -39,6 +39,7 @@ k_cluster_eig(const int* __restrict__ rowptr, const int* __restrict__ colidx, co
   if (c >= num_clusters) return;
   const int m0 = member_ptr[c], n = member_ptr[c + 1] - m0;
   if (n > EIG_MAX) { if (lane == 0) atomicExch(status, 1); return; }     // caller falls back to the host path
+  if (n == 0) return;                           // an empty cluster has no vector (its rank lookup would read sRank[-1])
   double (*A)[EIG_MAX + 1] = sA[w];
   double (*V)[EIG_MAX + 1] = sV[w];
   if (lane < n) sNode[w][lane] = member[m0 + lane];

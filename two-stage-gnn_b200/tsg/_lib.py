@@ -77,6 +77,10 @@ _PROTOTYPES = {
     "tsg_eigpool_build": (I, [P, P, P, P, P, P, I64, I64, I, P, P, P, P, P]),
     "tsg_coarsen_edges_workspace_bytes": (SZ, [I64]),
     "tsg_coarsen_edges": (I, [P, P, P, I64, P, P, P, P, P, P, SZ, P]),
+    "tsg_eigen_bfs_clusters": (I, [P, P, P, P, I64, I64, I64, I64, I64, I64, P, P, P, P, P, P, P, P, P]),
+    "tsg_eigen_group_clusters": (I, [P, P, P, P, I64, I64, I64, I64, I64, P, P, P, P, P, P, P, P, P]),
+    "tsg_eigen_coarse": (I, [P, I64, I64, P, P, P, P, P, P, P, P, P, P, P, P, P]),
+    "tsg_eigen_final": (I, [P, P, P, P, I64, I64, I64, I64, I64, P, I64, P]),
     "tsg_linkpred_workspace_bytes": (SZ, [I64]),
     "tsg_linkpred_loss_fwd": (I, [P, P, P, P, I64, I64, ctypes.c_double, F32, P, P, SZ, P]),
     "tsg_linkpred_loss_bwd": (I, [P, P, P, P, I64, I64, ctypes.c_double, F32, P, P, P]),
@@ -163,7 +167,7 @@ KERNELS_PER_CALL = {
     "tsg_batch_to_ptr": 1, "tsg_filter_adj": 7, "tsg_gate_gather_fwd": 1, "tsg_gate_gather_bwd": 1,
     "tsg_readout_fwd": 1, "tsg_readout_bwd": 1, "tsg_triplet_fwd": 2, "tsg_triplet_bwd": 9,
     "tsg_pairdist_matrix": 1, "tsg_linear_fwd": 1, "tsg_dense_epilogue_bwd": 1, "tsg_linear_bwd_weight": 2, "tsg_sag_boundary_bwd": 2,
-    "tsg_eigpool_build": 1, "tsg_coarsen_edges": 6, "tsg_inv_perm": 1, "tsg_csr_filter": 5, "tsg_sag_encoder_fwd": 38, "tsg_sag_encoder_bwd": 22, "tsg_sag_encoder_fwd_compact": 36, "tsg_sag_encoder_embed_compact": 3, "tsg_sag_triplet_step_compact": 72, "tsg_sag_step_fwd_compact": 37, "tsg_sag_step_bwd_compact": 25, "tsg_sag_nll_step_compact": 64, "tsg_sag_classify_compact": 6, "tsg_linkpred_loss_fwd": 3, "tsg_linkpred_loss_bwd": 1, "tsg_spmm_label_dot": 1, "tsg_gate_readout_fwd": 1, "tsg_gate_readout_linear_fwd": 2, "tsg_sag_encoder_bwd_compact": 22, "tsg_relu_bwd_colsum_rank1": 1, "tsg_sag_conv_bwd_fused": 1, "tsg_gate_score_bwd": 1, "tsg_spmm_dot": 1, "tsg_pack_batch_compact": 1, "tsg_pack_dense_batch": 1, "tsg_pack_eigen_batch": 1, "tsg_seg_contract": 1, "tsg_seg_linear": 1, "tsg_seg_linear_tc": 1, "tsg_linear_tc": 2, "tsg_gat_fwd": 2, "tsg_gat_bwd": 2, "tsg_dense_to_coo": 6, "tsg_nodebn_fwd": 1, "tsg_nodebn_bwd": 1,
+    "tsg_eigpool_build": 1, "tsg_coarsen_edges": 6, "tsg_eigen_bfs_clusters": 1, "tsg_eigen_group_clusters": 1, "tsg_eigen_coarse": 1, "tsg_eigen_final": 1, "tsg_inv_perm": 1, "tsg_csr_filter": 5, "tsg_sag_encoder_fwd": 38, "tsg_sag_encoder_bwd": 22, "tsg_sag_encoder_fwd_compact": 36, "tsg_sag_encoder_embed_compact": 3, "tsg_sag_triplet_step_compact": 72, "tsg_sag_step_fwd_compact": 37, "tsg_sag_step_bwd_compact": 25, "tsg_sag_nll_step_compact": 64, "tsg_sag_classify_compact": 6, "tsg_linkpred_loss_fwd": 3, "tsg_linkpred_loss_bwd": 1, "tsg_spmm_label_dot": 1, "tsg_gate_readout_fwd": 1, "tsg_gate_readout_linear_fwd": 2, "tsg_sag_encoder_bwd_compact": 22, "tsg_relu_bwd_colsum_rank1": 1, "tsg_sag_conv_bwd_fused": 1, "tsg_gate_score_bwd": 1, "tsg_spmm_dot": 1, "tsg_pack_batch_compact": 1, "tsg_pack_dense_batch": 1, "tsg_pack_eigen_batch": 1, "tsg_seg_contract": 1, "tsg_seg_linear": 1, "tsg_seg_linear_tc": 1, "tsg_linear_tc": 2, "tsg_gat_fwd": 2, "tsg_gat_bwd": 2, "tsg_dense_to_coo": 6, "tsg_nodebn_fwd": 1, "tsg_nodebn_bwd": 1,
     "tsg_pred_ce_fwd": 2, "tsg_pred_ce_bwd": 1, "tsg_pred_classify": 2,
 }
 launch_calls = 0        # libtsg entry points called since import

@@ -258,6 +258,164 @@ class DeviceCorpus:
                           pool_w=stack(pool_w, Nt), final_w=stack(final_w, NCt), J=len(pool_w), Jf=len(final_w),
                           nc=nc, ncoarse=np.diff(qptr))
 
+    def build_eigen(self, pool_size: int = 10, num_pool_matrix: int = 1, num_pool_final_matrix: int = 1,
+                    cluster_of=None, chunk_size: int = 1 << 24) -> int:
+        """Build this corpus's EigenPooling operands on the GPU (K17 + K11's per-cluster eigensolver) and leave them as
+        `attach_eigen` does.  Without `cluster_of`: the device form of eigen_synth.make_operands(corpus, pool_size,
+        num_pool_matrix, num_pool_final_matrix) -- BFS chunks of `pool_size` nodes, members in BFS order.  With
+        `cluster_of` (integer [sum n] graph-local ids, numpy or a tensor): the device form of operands_from_clusters,
+        members in ascending node order; clusters may have at most TSG_EIG_MAX = 32 members, ids lie in [0, n).
+        Works on `from_device` corpora (no host copy of the corpus); graphs are processed in chunks of about
+        `chunk_size` nodes + edges, so scratch memory does not grow with the corpus.  One device-to-host read of the
+        per-graph cluster and coarse-entry counts; the final pooling of graphs with more than TSG_EIGEN_FINAL_MAX = 112
+        clusters is computed on the host from their coarse lists (eigen_synth._eigvecs) and uploaded.  Returns the
+        number of such graphs.  Nothing collective: each rank builds its own shard.
+        Integer arrays equal the host operands exactly.  Eigenvectors of simple eigenvalues match the host's; where an
+        eigenvalue is repeated, the vector is another unit vector of the same eigenspace (sign and repeat rules kept),
+        so training from a device build follows a different trajectory than from host operands.
+        ValueError, before any device work, for a corpus that is not coalesced and symmetric (attach_eigen takes host
+        operands for those), a dense_x corpus, pool_size outside [1, 32], J < 1 or Jf < 0, a cluster_of of the wrong
+        length or with a negative id, and a graph of more than TSG_EIGEN_BUILD_MAX_NODES = 19,370 nodes; after the
+        device work (nothing attached) for a label >= its graph's node count, a cluster of more than 32 members and an
+        edge list that breaks the coalesced promise."""
+        from . import eigen_synth
+        max_nodes_cap, final_cap, i32_max = 19370, 112, 2 ** 31 - 1
+        G, Nt, Et = self.num_graphs, int(self.n.sum()), int(self.e.sum())
+        ps, J, Jf = int(pool_size), int(num_pool_matrix), int(num_pool_final_matrix)
+        if not self.coalesced:
+            raise ValueError("tsg: build_eigen needs a coalesced, symmetric corpus; build the operands on the host "
+                             "(eigen_synth) and attach_eigen them")
+        if self.x is not None:
+            raise ValueError("tsg: build_eigen is for one-hot node label corpora; this one carries per-node feature rows "
+                             "(dense_x)")
+        if not 1 <= ps <= 32:
+            raise ValueError(f"tsg: pool_size = {ps}, outside [1, 32]")
+        if J < 1 or Jf < 0:
+            raise ValueError(f"tsg: num_pool_matrix = {J} (>= 1) and num_pool_final_matrix = {Jf} (>= 0)")
+        if G and int(self.n.max()) > max_nodes_cap:
+            g = int(np.argmax(self.n))
+            raise ValueError(f"tsg: graph {g} has {int(self.n[g])} nodes, more than build_eigen's {max_nodes_cap}")
+        if Nt + Et > i32_max:
+            raise ValueError("tsg: the corpus exceeds 32-bit indexing")
+        dev = self.device
+        i32 = dict(dtype=torch.int32, device=dev)
+        f32 = dict(dtype=torch.float32, device=dev)
+        labels = None
+        if cluster_of is not None:
+            if isinstance(cluster_of, torch.Tensor):
+                if cluster_of.numel() != Nt:
+                    raise ValueError(f"tsg: cluster_of has {cluster_of.numel()} entries, the corpus has {Nt} nodes")
+                if cluster_of.is_floating_point() or cluster_of.is_complex() or cluster_of.dtype == torch.bool:
+                    raise ValueError("tsg: cluster_of must hold integer cluster ids")
+                if Nt and int(cluster_of.min()) < 0:
+                    raise ValueError("tsg: cluster ids must be non-negative")
+                labels = cluster_of.reshape(-1).clamp(max=i32_max).to(**i32, copy=True)
+            else:
+                host = np.asarray(cluster_of).reshape(-1)
+                if host.shape[0] != Nt:
+                    raise ValueError(f"tsg: cluster_of has {host.shape[0]} entries, the corpus has {Nt} nodes")
+                if host.size and not np.issubdtype(host.dtype, np.integer):
+                    raise ValueError("tsg: cluster_of must hold integer cluster ids")
+                if host.size and int(host.min()) < 0:
+                    raise ValueError("tsg: cluster ids must be non-negative")
+                labels = torch.from_numpy(np.clip(host, 0, i32_max).astype(np.int32)).to(dev)
+
+        nptr = np.zeros(G + 1, np.int64); np.cumsum(self.n, out=nptr[1:])
+        eptr = np.zeros(G + 1, np.int64); np.cumsum(self.e, out=eptr[1:])
+        w = self.n + self.e
+        cid = (np.cumsum(w) - w) // max(int(chunk_size), 1)
+        starts = np.concatenate([[0], np.flatnonzero(np.diff(cid)) + 1]) if G else np.zeros(0, np.int64)
+        chunks = [(int(a), int(b)) for a, b in zip(starts, np.append(starts[1:], G))]
+        cap_n = max([int(nptr[b] - nptr[a]) for a, b in chunks], default=0)
+        cap_e = max([int(eptr[b] - eptr[a]) for a, b in chunks], default=0)
+        rowptr, colidx = torch.empty(cap_n + 1, **i32), torch.empty(max(cap_e, 1), **i32)
+        cluster_g, member_ptr, member = torch.empty(max(cap_n, 1), **i32), torch.empty(cap_n + 1, **i32), \
+            torch.empty(max(cap_n, 1), **i32)
+        pool_val, pool_nodes = torch.empty(max(J * cap_n, 1), **f32), torch.empty(max(J * cap_n, 1), **f32)
+        row_off = torch.empty(max(cap_n, 1), **i32)
+        counts = torch.empty(2 * G + 4, **i32)          # clusters [G] | coarse entries [G] | status [4]
+        nc_d, nq_d, status = counts[:G], counts[G:2 * G], counts[2 * G:]
+        status.fill_(i32_max)
+        cl = labels if labels is not None else torch.empty(max(Nt, 1), **i32)
+        pool_w = torch.empty(J, Nt, **f32)
+        st = stream_ptr()
+        corpus = (ptr(self.node_ptr), ptr(self.edge_ptr), ptr(self.row), ptr(self.col))
+        chunk_bufs = (ptr(rowptr), ptr(colidx), ptr(cluster_g), ptr(member_ptr), ptr(member), ptr(status))
+
+        def group(g0, g1, nc_out):
+            Nc, Ec = int(nptr[g1] - nptr[g0]), int(eptr[g1] - eptr[g0])
+            call("tsg_eigen_group_clusters", *corpus, g0, g1 - g0, Nc, Ec, int(self.n[g0:g1].max()), ptr(cl), nc_out,
+                 *chunk_bufs, st)
+
+        def coarse(g0, g1, write):
+            out = (ptr(row_off), None, ptr(d_qptr), ptr(coarse_row), ptr(coarse_col), ptr(coarse_w)) if write else \
+                (None, ptr(nq_d), None, None, None, None)
+            call("tsg_eigen_coarse", ptr(self.node_ptr), g0, g1 - g0, ptr(nc_d), ptr(rowptr), ptr(colidx),
+                 ptr(cluster_g), ptr(member_ptr), ptr(member), *out, st)
+
+        # pass 1: clusters, per-cluster eigenvectors (K11), coarse-entry counts
+        for g0, g1 in chunks:
+            n0, n1 = int(nptr[g0]), int(nptr[g1])
+            Nc, Ec = n1 - n0, int(eptr[g1] - eptr[g0])
+            if labels is None:
+                call("tsg_eigen_bfs_clusters", *corpus, g0, g1 - g0, Nc, Ec, int(self.n[g0:g1].max()), ps, ptr(cl),
+                     ptr(nc_d), *chunk_bufs, st)
+            else:
+                group(g0, g1, ptr(nc_d))
+            if Nc:
+                call("tsg_eigpool_build", ptr(rowptr), ptr(colidx), None, ptr(cluster_g), ptr(member_ptr), ptr(member),
+                     Nc, Nc, J, ptr(pool_val), ptr(pool_nodes), None, ptr(status[3:]), st)
+                pool_w[:, n0:n1].copy_(pool_nodes[:J * Nc].view(J, Nc))
+            coarse(g0, g1, False)
+        host = counts.cpu().numpy()
+        bad = host[2 * G:2 * G + 3]
+        if bad[0] != i32_max:
+            raise ValueError(f"tsg: graph {int(bad[0])}'s edge list is not coalesced and symmetric")
+        if bad[2] != i32_max:
+            g = int(bad[2])
+            raise ValueError(f"tsg: graph {g} has a cluster id outside [0, {int(self.n[g])}) (at most one cluster per "
+                             "node)")
+        if bad[1] != i32_max:
+            raise ValueError(f"tsg: graph {int(bad[1])} has a cluster of more than 32 members")
+        nc, ncoarse = host[:G].astype(np.int64), host[G:2 * G].astype(np.int64)
+        cptr = np.zeros(G + 1, np.int64); np.cumsum(nc, out=cptr[1:])
+        qptr = np.zeros(G + 1, np.int64); np.cumsum(ncoarse, out=qptr[1:])
+        NCt, ECt = int(cptr[-1]), int(qptr[-1])
+        if NCt + ECt > i32_max:
+            raise ValueError("tsg: the operands exceed 32-bit indexing")
+        t64 = lambda a: torch.from_numpy(a).to(dev)
+        d_cptr, d_qptr = t64(cptr), t64(qptr)
+        coarse_row, coarse_col, coarse_w = torch.empty(ECt, **i32), torch.empty(ECt, **i32), torch.empty(ECt, **f32)
+        final_w = torch.empty(Jf, NCt, **f32) if Jf else torch.zeros(1, NCt, **f32)
+
+        # pass 2: the coarse lists at their corpus offsets, then the final pooling
+        for g0, g1 in chunks:
+            if ECt:
+                group(g0, g1, None)
+                coarse(g0, g1, True)
+            for lo, hi in ((0, 32), (32, 64), (64, final_cap)) if Jf else ():     # shared memory per size class
+                sel = nc[g0:g1][(nc[g0:g1] > lo) & (nc[g0:g1] <= hi)]
+                if sel.size:
+                    call("tsg_eigen_final", ptr(d_cptr), ptr(d_qptr), ptr(coarse_row), ptr(coarse_col), g0, g1 - g0,
+                         lo, int(sel.max()), Jf, ptr(final_w), NCt, st)
+        fallback = np.flatnonzero(nc > final_cap) if Jf else np.zeros(0, np.int64)
+        if fallback.size:
+            from .synth import _ragged_arange
+            idx = torch.from_numpy(_ragged_arange(qptr[fallback], ncoarse[fallback])).to(dev)
+            rows, cols = coarse_row[idx].cpu().numpy(), coarse_col[idx].cpu().numpy()
+            o = 0
+            for g in fallback.tolist():
+                k, m = int(nc[g]), int(ncoarse[g])
+                adj = np.zeros((k, k), np.float32)
+                adj[rows[o:o + m], cols[o:o + m]] = 1.0
+                o += m
+                ev = eigen_synth._eigvecs(adj, Jf)
+                final_w[:, int(cptr[g]):int(cptr[g + 1])] = torch.from_numpy(np.ascontiguousarray(ev.T, np.float32)).to(dev)
+        self.eigen = dict(cluster_ptr=d_cptr, coarse_ptr=d_qptr, cluster_of=cl[:Nt], coarse_row=coarse_row,
+                          coarse_col=coarse_col, coarse_w=coarse_w, pool_w=pool_w, final_w=final_w, J=J, Jf=Jf, nc=nc,
+                          ncoarse=ncoarse)
+        return int(fallback.size)
+
     def check_eigen(self, ids_host, max_nodes: int, num_pool_matrix=None, num_pool_final_matrix=None):
         """The host-side checks of `pack_eigen` (no device work): -> (ids int64 numpy, J, Jf).  ValueError when no
         operands are attached, for a corpus with per-node feature rows, an empty id list, an id outside the corpus, a
